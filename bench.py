@@ -66,7 +66,13 @@ def parse_args():
     ap.add_argument("--c5-sweeps", type=int, default=20)
     ap.add_argument("--budget-s", type=float, default=840.0,
                     help="wall-clock budget of the whole run: the stated job is shortened (fewer sweeps, said so) when it would not fit")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's reads) as DIR/*.npy, at most 60 MB, so that two builds "
+                         "can be compared output for output; see dump_outputs()")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def build_workload(args):
@@ -158,6 +164,39 @@ def field_layout_bytes(stats: dict) -> float:
     """The same unit in THIS kernel's layout (DESIGN.md section 4): 8 B local field + 2 bits per attempt, and an 8 B read +
     8 B write of one local field per neighbour update.  Reported next to the SURVEY figure, not used for `frac`."""
     return 8.25 * stats["attempts"] + 16.0 * stats["nbr_updates"]
+
+
+DUMP_ENERGY_BYTES = 16 << 20     # energies.npy + energy_reads.npy
+DUMP_STATE_BYTES = 44 << 20      # states.npy + state_reads.npy
+
+
+def dump_outputs(out_dir, states, energies, seed: int) -> None:
+    """Write what one step of the timed path hands its caller -- final states int8 [R][n] and energies fp64 [R], both on the
+    device -- as .npy files in float32 / float64, at most 60 MB in all:
+
+        energies.npy      fp64, every read's energy (a seeded sample of 1 M reads when R is larger)
+        energy_reads.npy  fp64, the read index of each entry of energies.npy
+        states.npy        fp32 (+-1), whole final states of a seeded sample of reads, as many as fit 44 MB with their indices
+        state_reads.npy   fp64, the read index of each row of states.npy
+
+    The sample depends on (R, n, seed) only, so two runs with the same arguments dump the same reads."""
+    import torch
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    R, n = states.shape
+    rng = np.random.default_rng(seed)
+
+    def sample(k):
+        return np.arange(R) if k >= R else np.sort(rng.choice(R, size=k, replace=False))
+
+    e_idx = sample(DUMP_ENERGY_BYTES // 16)
+    s_idx = sample(max(1, DUMP_STATE_BYTES // (4 * n + 8)))
+    e = energies[torch.from_numpy(e_idx).to(energies.device)].cpu().numpy()
+    s = states[torch.from_numpy(s_idx).to(states.device)].cpu().numpy()
+    np.save(out / "energies.npy", e.astype(np.float64))
+    np.save(out / "energy_reads.npy", e_idx.astype(np.float64))
+    np.save(out / "states.npy", s.astype(np.float32))
+    np.save(out / "state_reads.npy", s_idx.astype(np.float64))
 
 
 def run_cpu_sample(model, betas, spb, seed, reads, threads, states=None, seeds=None):
@@ -403,6 +442,8 @@ def main():
             step_resident(True)
         barrier()
         elapsed = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, states_dev, energies_dev, args.seed)
     wall_s = allmax(elapsed)
     attempts_per_step_per_gpu = n * len(betas) * spb * R
     # device time: the library brackets every call with CUDA events on the stream it launches on (qa_stats.ms_total);

@@ -41,6 +41,39 @@ def test_committed_bench_lines_carry_the_contract_keys(name, n_gpus):
         assert line["strong"]["reads"] == 100000 and line["strong"]["reads_per_rank"] == 50000
 
 
+def test_steps_must_be_positive(monkeypatch):
+    monkeypatch.setattr("sys.argv", ["bench.py", "--steps", "2", "--warmup", "0"])
+    assert bench.parse_args().steps == 2
+    monkeypatch.setattr("sys.argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse_args()
+
+
+@pytest.mark.parametrize("state_budget", [None, 3 * (4 * 50 + 8)])
+def test_dump_outputs_writes_float_arrays_of_a_fixed_sample(tmp_path, monkeypatch, state_budget):
+    import numpy as np
+    import torch
+    if state_budget is not None:      # force the sampled form: 3 rows of states, 7 energies
+        monkeypatch.setattr(bench, "DUMP_STATE_BYTES", state_budget)
+        monkeypatch.setattr(bench, "DUMP_ENERGY_BYTES", 7 * 16)
+    R, n = 20, 50
+    g = torch.Generator().manual_seed(0)
+    states = (torch.randint(0, 2, (R, n), dtype=torch.int8, generator=g) * 2 - 1)
+    energies = torch.randn(R, dtype=torch.float64, generator=g)
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, states, energies, seed=1234)
+    files = {p.name: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert set(files) == {"energies.npy", "energy_reads.npy", "states.npy", "state_reads.npy"}
+    assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+    e_idx, s_idx = files["energy_reads.npy"], files["state_reads.npy"]
+    assert len(e_idx) == (R if state_budget is None else 7) and len(s_idx) == (R if state_budget is None else 3)
+    assert np.array_equal(files["energies.npy"], energies.numpy()[e_idx.astype(int)])
+    assert np.array_equal(files["states.npy"], states.numpy()[s_idx.astype(int)].astype(np.float32))
+    for name, a in files.items():      # same arguments, same sample and bytes
+        assert np.array_equal(a, np.load(tmp_path / "b" / name))
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 << 20
+
+
 def test_algorithmic_bytes_follow_survey_8d():
     # 10 attempts, 3 accepted flips with 7 neighbour updates in total, 40 directed entries per read and sweep, 1 sweep of 2 reads,
     # rows shared by 2 reads: 8*10 + 9*3 + 17*7 + 12*40*(10/5)/2 with num_variables = 5

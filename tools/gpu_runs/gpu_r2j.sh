@@ -9,7 +9,7 @@ for v in base dn_lop3 dn_c3 dn_lop3_c3; do
   for reads in 37888 56832; do
     echo "== $v reads $reads" >> $o/r2j_ab_dense.log
     if [ $v = base ]; then timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep "reads $reads " >> $o/r2j_ab_dense.log
-    else QA_LIB_PATH=$PWD/gpurun_variants/$v.so timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep "reads $reads " >> $o/r2j_ab_dense.log; fi
+    else QA_LIB_PATH=$PWD/build/variants/$v.so timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep "reads $reads " >> $o/r2j_ab_dense.log; fi
   done
 done
 # dense kernel: plain run, then the full ncu set on one launch (small read count: the per-SM shape is the same, 8 warps per SM)

@@ -9,7 +9,7 @@ for v in base dn_lop3 dn_c3 dn_lop3_c3; do
   for reads in 37888 56832; do
     echo "== $v reads $reads" >> $o/r2k_ab_dense.log
     if [ $v = base ]; then timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep -E "reads $reads |Error|error" >> $o/r2k_ab_dense.log
-    else QA_LIB_PATH=$PWD/gpurun_variants/$v.so timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep -E "reads $reads |Error|error" >> $o/r2k_ab_dense.log; fi
+    else QA_LIB_PATH=$PWD/build/variants/$v.so timeout 300 python tools/probe_c5.py --reads $((reads/2)) --ref-reads 0 2>&1 | grep -E "reads $reads |Error|error" >> $o/r2k_ab_dense.log; fi
   done
 done
 timeout 420 ncu --replay-mode application --section SpeedOfLight --section WarpStateStats --section SchedulerStats --section Occupancy \
