@@ -118,6 +118,15 @@ int qa_model_from_ising(qa_ctx *ctx, int32_t n, const double *h, int64_t m, cons
  * (cut+balance, DQM cluster-size and CQM size penalties; SURVEY.md Appendix A). grp[v] = -1: none. */
 int qa_model_set_groups(qa_model *model, int32_t ngroups, const int32_t *grp, const int32_t *coef,
                         const double *lambda, const int64_t *kappa);
+/* Interval bounds for the groups of qa_model_set_groups (inequality constraints without slack variables).  With
+ * u_g = sum_{v: grp[v]==g} coef[v]*s_v + kappa[g] and d(u) = max(lo[g] - u, 0, u - hi[g]), group g contributes
+ *     lambda[g] * (double)(d*d) * 0.25
+ * and a flip that moves u to u' costs lambda[g] * ((double)(d(u')^2 - d(u)^2) * 0.25): integers exact, one rounding.
+ * lo = hi = 0 is the equality term above, bit for bit.  Bounds are clamped to the reachable range
+ * [kappa - sum|coef|, kappa + sum|coef|] (INT64_MIN / INT64_MAX: unbounded); lo > hi gives QA_ERR_ARG, a clamped
+ * distance d whose square reaches 2^53 QA_ERR_LIMIT.  lo = hi = NULL: equality groups again.  Call after
+ * qa_model_set_groups; a later qa_model_set_groups clears the bounds. */
+int qa_model_set_group_bounds(qa_model *model, const int64_t *lo, const int64_t *hi);
 /* Dense k-way form (BASELINE config 5; the all-pairs same-case term of DQM_clustering.py:36-37 on a dense affinity):
  * variable v = cell*K + case, J[(i,c),(j,c)] = W[i][j] for every case c, J[(i,c),(i,c')] = P.  Derives W (n/K x n/K) and P
  * from the model's adjacency on the device and verifies the structure.  Returns 1 when the model has it -- QA_MODE_THROUGHPUT
@@ -182,6 +191,9 @@ int qa_energy_argmin(qa_ctx *ctx, qa_model *model, int32_t num_reads, const int8
  *   qa_build_dqm_onehot    DQM_clustering.py:29-43   one-hot expansion (variable i*K + c), penalty*(sum_c x_ic - 1)^2,
  *                                                    cluster-size term as K groups; intended = 0: set_* semantics as written
  *   qa_build_cqm_penalty   CQM_clustering.py:30-48   objective + A*(one-hot)^2 + B*(N_j - min_size - slack_j)^2 as K groups
+ *   qa_build_cqm_interval  same constraint, no slack: objective + A*(one-hot)^2 + B*max(0, min_size - N_j)^2 as K interval
+ *                          groups (coef 1, kappa = n - 2*min_size, bounds [0, +inf)); h, couplers and offset are those of
+ *                          the first n*K variables of qa_build_cqm_penalty
  */
 int qa_build_cut_balance(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *eu, const int32_t *ev, const double *w,
                          double gamma_factor, double k, qa_model **out, double *offset_out, double *gamma_out);
@@ -195,6 +207,9 @@ int qa_build_dqm_onehot(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *
 int qa_build_cqm_penalty(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *eu, const int32_t *ev, const double *w,
                          int32_t num_clusters, int32_t min_size, double onehot_penalty, double size_penalty, qa_model **out,
                          double *offset_out);
+int qa_build_cqm_interval(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *eu, const int32_t *ev, const double *w,
+                          int32_t num_clusters, int32_t min_size, double onehot_penalty, double size_penalty, qa_model **out,
+                          double *offset_out);
 
 /* ---- SNN graph construction on the device (the step before the path: Seurat FindNeighbors as the reference's notebooks use
  * it, R/pbmc3k/Pbmc3k_general_data_preparation.Rmd:47-75, R/benchmarks/Benchmark.Rmd:150-166):
@@ -222,8 +237,8 @@ int qa_graph_split(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *eu, c
                    const int32_t *part, int32_t num_parts, qa_graph **out);
 /* parent node of every node of child `problem` (problem < 0: all children back to back); host or device destination */
 int qa_graph_get_nodes(const qa_graph *graph, int32_t problem, int32_t *node_ids_out);
-/* single-problem models (rank-1 groups included) -> one batched model for qa_sa_sample_model_batch; the inputs stay valid and
- * owned by the caller.  Batched models with groups run on the warp-per-read kernel. */
+/* single-problem models (rank-1 groups and their interval bounds included) -> one batched model for qa_sa_sample_model_batch;
+ * the inputs stay valid and owned by the caller.  Batched models with groups run on the warp-per-read kernel. */
 int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa_model **out);
 /* qa_sa_sample_ising_batch on a resident batched model.  betas_per_problem = 0: beta_schedules is one schedule [num_betas] for
  * every problem; 1: [num_problems][num_betas], problem p anneals with its own schedule (what separate sampler calls with

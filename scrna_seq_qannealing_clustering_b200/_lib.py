@@ -89,6 +89,7 @@ SIGNATURES = {
     "qa_ctx_last_kernel": (C.c_int, [_p]),
     "qa_model_from_ising": (C.c_int, [_p, _i32, _p, _i64, _p, _p, _p, C.POINTER(_p)]),
     "qa_model_set_groups": (C.c_int, [_p, _i32, _p, _p, _p, _p]),
+    "qa_model_set_group_bounds": (C.c_int, [_p, _p, _p]),
     "qa_model_enable_dense": (C.c_int, [_p, _i32]),
     "qa_model_num_variables": (C.c_int, [_p]),
     "qa_model_num_couplers": (_i64, [_p]),
@@ -103,6 +104,7 @@ SIGNATURES = {
     "qa_build_subsampling": (C.c_int, [_p, _i32, _i64, _p, _p, _p, C.c_double, C.c_double, C.POINTER(_p), C.POINTER(C.c_double)]),
     "qa_build_dqm_onehot": (C.c_int, [_p, _i32, _i64, _p, _p, _p, _i32, C.c_double, C.c_double, _i32, C.POINTER(_p), C.POINTER(C.c_double)]),
     "qa_build_cqm_penalty": (C.c_int, [_p, _i32, _i64, _p, _p, _p, _i32, _i32, C.c_double, C.c_double, C.POINTER(_p), C.POINTER(C.c_double)]),
+    "qa_build_cqm_interval": (C.c_int, [_p, _i32, _i64, _p, _p, _p, _i32, _i32, C.c_double, C.c_double, C.POINTER(_p), C.POINTER(C.c_double)]),
     "qa_energy_argmin": (C.c_int, [_p, _p, _i32, _p, _p, C.POINTER(C.c_double), C.POINTER(_i64), C.POINTER(QAStats)]),
     "qa_aggregate_reads": (C.c_int, [_p, _i32, _i32, _p, C.POINTER(_i32), _p, _p]),
     "qa_dev_alloc": (C.c_int, [_p, _i64, C.POINTER(_p)]),

@@ -209,13 +209,15 @@ def clustering_dqm(G, num_of_clusters, gamma, sampler=None, penalty=None, semant
         _close(model)
 
 
-def _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, subindex, device_build, sa_kwargs):
+def _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, subindex, device_build, sa_kwargs,
+         size_lowering="slack"):
     smp = _sampler(sampler)
     if _on_device(smp, device_build):
         model = smp.build_on_device("cqm", G, num_of_clusters=num_of_clusters, min_size=min_size, onehot_penalty=onehot_penalty,
-                                    size_penalty=size_penalty, subindex=subindex)
+                                    size_penalty=size_penalty, subindex=subindex, size_lowering=size_lowering)
     else:
-        model = models.cqm_model(G, num_of_clusters, min_size, onehot_penalty, size_penalty, subindex=subindex)
+        model = models.cqm_model(G, num_of_clusters, min_size, onehot_penalty, size_penalty, subindex=subindex,
+                                 size_lowering=size_lowering)
     try:
         with warnings.catch_warnings():
             warnings.simplefilter("ignore", UserWarning)
@@ -225,16 +227,19 @@ def _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, su
 
 
 def clustering_cqm(G, num_of_clusters, sampler=None, onehot_penalty=None, size_penalty=None, min_size=20, device_build=None,
-                   **sa_kwargs):
-    """k-way CQM clustering with one-hot and minimum-size constraints (CQM_clustering.py:25-55)."""
-    return _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, None, device_build, sa_kwargs)
+                   size_lowering="slack", **sa_kwargs):
+    """k-way CQM clustering with one-hot and minimum-size constraints (CQM_clustering.py:25-55).  ``size_lowering``:
+    'slack' (slack-bit equality penalty) or 'interval' (B * max(0, min_size - N_j)^2, no slack bits; models.cqm_model)."""
+    return _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, None, device_build, sa_kwargs,
+                size_lowering)
 
 
 def clustering_cqm_2(G, num_of_clusters, sampler=None, onehot_penalty=None, size_penalty=None, min_size=20, device_build=None,
-                     **sa_kwargs):
+                     size_lowering="slack", **sa_kwargs):
     """As ``clustering_cqm`` but variables are named by the node attribute ``subindex`` (CQM_clustering.py:57-91)."""
     sub = [G.nodes[i]["subindex"] for i in G.nodes]
-    return _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, sub, device_build, sa_kwargs)
+    return _cqm(G, num_of_clusters, sampler, onehot_penalty, size_penalty, min_size, sub, device_build, sa_kwargs,
+                size_lowering)
 
 
 def graph_subsampling(G, gamma, solver="hybrid", sampler=None, device_build=None, **sa_kwargs):

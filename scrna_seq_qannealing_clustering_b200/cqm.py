@@ -13,7 +13,7 @@ from typing import Dict, Hashable, List, Optional, Tuple
 import numpy as np
 
 from .bqm import BinaryQuadraticModel
-from .models import LoweredModel, lowered_from_bqm
+from .models import Groups, LoweredModel, lowered_from_bqm
 
 
 class QuadExpr:
@@ -179,7 +179,8 @@ class ConstrainedQuadraticModel:
                 ok &= np.abs(val) <= 1e-9
         return ok
 
-    def to_bqm(self, onehot_penalty: float, constraint_penalty: float) -> BinaryQuadraticModel:
+    def to_bqm(self, onehot_penalty: float, constraint_penalty: float, constraints: bool = True) -> BinaryQuadraticModel:
+        """Objective + one-hot penalties + (``constraints``) slack penalties of the linear constraints."""
         bqm = BinaryQuadraticModel({}, {}, self.objective.offset, "BINARY")
         for v in self.variables:
             bqm.add_variable(v, 0.0)
@@ -190,7 +191,7 @@ class ConstrainedQuadraticModel:
         for grp in self.discrete.values():
             bqm.add_linear_equality_constraint([(v, 1) for v in grp], onehot_penalty, -1)
         import warnings
-        for label, con in self.constraints.items():
+        for label, con in (self.constraints.items() if constraints else ()):
             terms = [(v, int(a) if float(a).is_integer() else a) for v, a in con.lhs.linear.items()]
             const = con.lhs.offset
             const = int(const) if float(const).is_integer() else const
@@ -215,10 +216,59 @@ class ConstrainedQuadraticModel:
             gain[v] = gain.get(v, 0.0) + abs(b)
         return max(gain.values(), default=0.0) + 1.0, 1.0
 
-    def to_lowered(self, onehot_penalty: Optional[float] = None, constraint_penalty: Optional[float] = None) -> LoweredModel:
+    def to_lowered(self, onehot_penalty: Optional[float] = None, constraint_penalty: Optional[float] = None,
+                   lowering: str = "slack") -> LoweredModel:
+        """Spin model of the CQM.  ``lowering="slack"``: every linear constraint becomes a slack penalty (dimod's
+        add_linear_inequality_constraint).  ``"interval"``: no slack variables; each constraint ``sum a_i x_i + c (sense) 0``
+        becomes one interval group (``models.Groups``) with coef a_i, kappa = sum a_i + 2c, lam = B and bounds [0, +inf) for
+        ``>=``, (-inf, 0] for ``<=``, [0, 0] for ``==``: the penalty B * violation^2.  It needs integer a_i and 2c, pairwise
+        disjoint constraint variables and at most QA_MAX_GROUPS constraints, and raises ValueError otherwise.  Discrete
+        (one-hot) constraints are couplers either way."""
+        if lowering not in ("slack", "interval"):
+            raise ValueError(f"lowering must be 'slack' or 'interval', not {lowering!r}")
         A0, B0 = self.default_penalties()
         A = A0 if onehot_penalty is None else float(onehot_penalty)
         B = B0 if constraint_penalty is None else float(constraint_penalty)
-        model = lowered_from_bqm(self.to_bqm(A, B))
-        model.meta.update({"kind": "cqm_generic", "cqm": self, "onehot_penalty": A, "size_penalty": B})
+        interval = lowering == "interval"
+        if interval:
+            groups_spec = self._interval_groups()
+        model = lowered_from_bqm(self.to_bqm(A, B, constraints=not interval))
+        if interval:
+            index = {v: i for i, v in enumerate(model.labels)}
+            n, G = model.num_variables, len(groups_spec)
+            grp = np.full(n, -1, dtype=np.int32)
+            coef = np.zeros(n, dtype=np.int32)
+            kappa, lo, hi = (np.zeros(G, dtype=np.int64) for _ in range(3))
+            for g, (terms, kap, lo_g, hi_g) in enumerate(groups_spec):
+                for v, a in terms:
+                    grp[index[v]], coef[index[v]] = g, a
+                kappa[g], lo[g], hi[g] = kap, lo_g, hi_g
+            model.groups = Groups(grp, coef, np.full(G, B), kappa, lo, hi)
+        model.meta.update({"kind": "cqm_generic", "cqm": self, "onehot_penalty": A, "size_penalty": B, "lowering": lowering})
         return model
+
+    def _interval_groups(self):
+        """[(terms [(label, int a)], kappa, lo, hi)] of the non-discrete constraints, or ValueError."""
+        from ._lib import QA_MAX_GROUPS
+        if len(self.constraints) > QA_MAX_GROUPS:
+            raise ValueError(f"{len(self.constraints)} constraints: the interval lowering takes at most {QA_MAX_GROUPS}")
+        owner: Dict[Hashable, Hashable] = {}
+        out = []
+        i64 = np.iinfo(np.int64)
+        for label, con in self.constraints.items():
+            terms = []
+            for v, a in con.lhs.linear.items():
+                if not float(a).is_integer():
+                    raise ValueError(f"constraint {label!r}: coefficient {a} of {v!r} is not an integer")
+                if v in owner:
+                    raise ValueError(f"variable {v!r} appears in constraints {owner[v]!r} and {label!r}: interval groups "
+                                     "must not overlap")
+                owner[v] = label
+                terms.append((v, int(a)))
+            c2 = 2 * con.lhs.offset
+            if not float(c2).is_integer():
+                raise ValueError(f"constraint {label!r}: twice its constant ({c2}) is not an integer")
+            kap = sum(a for _, a in terms) + int(c2)
+            lo, hi = {">=": (0, i64.max), "<=": (i64.min, 0), "==": (0, 0)}[con.sense]
+            out.append((terms, kap, lo, hi))
+        return out

@@ -83,7 +83,8 @@ __device__ __forceinline__ double ls_field_direct(const ProblemDesc &D, const ui
 
 // Runs the schedule from (bi, swi) on.  VARIANT 0 = push sweeps (bit-exact), 2 = one pass that only evaluates the local fields
 // from the spins and stores them (neal get_flip_energy order): the initialisation of the push variant.
-template <int VARIANT, bool GROUPS>
+// GROUPS: 0 none, 1 rank-1 groups, 2 rank-1 groups with interval bounds (kap_sh then holds {kappa, lo, hi} per group).
+template <int VARIANT, int GROUPS>
 __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, unsigned long long &s0,
                           unsigned long long &s1, LaneStats &st) {
     const ProblemDesc &D = c.D;
@@ -261,8 +262,13 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                         g = sg.gm[i];
                         if (g >= 0) {
                             a = sg.am[i];
-                            const long long t = (long long)a * ((long long)a - (up ? 1 : -1) * ((long long)Mcol[g * QA_LS_TPB] + c.kap_sh[g]));
-                            dE = dE + c.lam_sh[g] * (double)t;
+                            if (GROUPS == 2) {
+                                const long long *kb = c.kap_sh + 3 * g;
+                                dE = dE + interval_flip_cost(c.lam_sh[g], a, up, (long long)Mcol[g * QA_LS_TPB] + kb[0], kb[1], kb[2]);
+                            } else {
+                                const long long t = (long long)a * ((long long)a - (up ? 1 : -1) * ((long long)Mcol[g * QA_LS_TPB] + c.kap_sh[g]));
+                                dE = dE + c.lam_sh[g] * (double)t;
+                            }
                         }
                     }
                     const bool cand = active && !(dE >= thr);
@@ -342,7 +348,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
     return finished;
 }
 
-template <int VARIANT, bool GROUPS>
+template <int VARIANT, int GROUPS>
 __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned long long &s1, LaneStats &st, int *error_flag) {
     const ProblemDesc &D = c.D;
     const int n = D.n;
@@ -383,7 +389,7 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
     bool finished = false;
     if (!finished) {
         int ib = 0, is = 0;
-        ls_sweeps<2, false>(c, ib, is, false, s0, s1, st);  // local fields from the current spins
+        ls_sweeps<2, 0>(c, ib, is, false, s0, s1, st);  // local fields from the current spins
         ls_sweeps<0, GROUPS>(c, bi, swi, false, s0, s1, st);
     }
 
@@ -398,18 +404,19 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
     }
 }
 
-__host__ __device__ inline size_t ls_smem_bytes(int max_groups) {
+__host__ __device__ inline size_t ls_smem_bytes(int max_groups, bool interval = false) {
     size_t b = sizeof(double) * QA_LS_D * QA_LS_TPB;   // cur (push phases) / spin words (field evaluation phases)
     b += (sizeof(LsStage) + sizeof(LsStagePull)) * QA_LS_WPB;
-    b += (sizeof(double) + sizeof(long long)) * (size_t)max_groups;
+    b += (sizeof(double) + (interval ? 3 : 1) * sizeof(long long)) * (size_t)max_groups;
     b += sizeof(int) * (size_t)max_groups * QA_LS_TPB;
     return b;
 }
 
-template <int VARIANT, bool GROUPS>
+template <int VARIANT, int GROUPS>
 __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P) {
     extern __shared__ __align__(16) unsigned char ls_smem[];
     // layout: [cur: D x TPB doubles, aliased by the spin words] [LsStage x warps] [LsStagePull x warps] [lambda] [kappa] [M]
+    // (interval groups: [kappa] is {kappa, lo, hi} per group)
     unsigned char *sp = ls_smem;
     double *cur_all = reinterpret_cast<double *>(sp);
     sp += sizeof(double) * QA_LS_D * QA_LS_TPB;
@@ -421,7 +428,7 @@ __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P
     double *lam_sh = reinterpret_cast<double *>(sp);
     sp += sizeof(double) * P.max_groups;
     long long *kap_sh = reinterpret_cast<long long *>(sp);
-    sp += sizeof(long long) * P.max_groups;
+    sp += (GROUPS == 2 ? 3 : 1) * sizeof(long long) * P.max_groups;
     int *M_all = reinterpret_cast<int *>(sp);
     __shared__ unsigned long long next_tile[QA_LS_WPB];
     const int lane = threadIdx.x & 31;
@@ -432,7 +439,13 @@ __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P
         const ProblemDesc &D0 = P.descs[0];
         for (int g = threadIdx.x; g < D0.ngroups; g += blockDim.x) {
             lam_sh[g] = D0.lambda[g];
-            kap_sh[g] = D0.kappa[g];
+            if (GROUPS == 2) {
+                kap_sh[3 * g] = D0.kappa[g];
+                kap_sh[3 * g + 1] = D0.kappa[D0.ngroups + g];
+                kap_sh[3 * g + 2] = D0.kappa[2 * D0.ngroups + g];
+            } else {
+                kap_sh[g] = D0.kappa[g];
+            }
         }
     }
     __syncthreads();
@@ -560,9 +573,10 @@ int launch_lockstep(Launch &L) {
     // lockstep: one warp = 32 reads of one problem
     const int tpp = (reads_per_problem + 31) / 32;
     const int64_t total_tiles = (int64_t)P * tpp;
-    const size_t smem = ls_smem_bytes(std::max(M->ngroups, 1));
+    const size_t smem = ls_smem_bytes(std::max(M->ngroups, 1), groups && L.interval);
     const void *fn = nullptr;
-    fn = groups ? (const void *)k_anneal_lockstep<0, true> : (const void *)k_anneal_lockstep<0, false>;
+    fn = !groups ? (const void *)k_anneal_lockstep<0, 0>
+                 : (L.interval ? (const void *)k_anneal_lockstep<0, 2> : (const void *)k_anneal_lockstep<0, 1>);
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, QA_LS_TPB, smem, cudaOccupancyDefault));

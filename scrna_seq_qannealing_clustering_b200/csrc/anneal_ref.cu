@@ -16,7 +16,8 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // one read, reference order.  Restates neal simulated_annealing_run() for one `state`.
 // ------------------------------------------------------------------------------------------------
-template <bool GROUPS>
+// GROUPS: 0 none, 1 rank-1 groups, 2 rank-1 groups with interval bounds (read per problem, like lambda / kappa)
+template <int GROUPS>
 __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t r_local, double *__restrict__ f,
                             uint32_t *__restrict__ spw, unsigned long long &s0, unsigned long long &s1,
                             long long *Mw, WarpStats &st, int *error_flag) {
@@ -97,7 +98,7 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                 double fv = __ldcg(f + v);
                 uint32_t w = __shfl_sync(FULL_MASK, wg, k);
                 int g = -1;
-                long long a = 0, kap = 0;
+                long long a = 0, kap = 0, glo = 0, ghi = 0;
                 double lam = 0.0;
                 if (GROUPS) {
                     g = __ldg(D.grp + v);
@@ -105,6 +106,10 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                         a = __ldg(D.coef + v);
                         lam = __ldg(D.lambda + g);
                         kap = __ldg(D.kappa + g);
+                        if (GROUPS == 2) {
+                            glo = __ldg(D.kappa + D.ngroups + g);
+                            ghi = __ldg(D.kappa + 2 * D.ngroups + g);
+                        }
                     }
                 }
                 // neal's delta_energy[v] == -2*s_v*f[v] exactly; plus the lazily evaluated rank-1 cost
@@ -113,8 +118,12 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                     double d = up ? -2.0 * fv : 2.0 * fv;
                     if (GROUPS) {
                         if (g >= 0) {
-                            const long long t = a * (a - (up ? 1 : -1) * (Mw[g] + kap));
-                            d = d + lam * (double)t;
+                            if (GROUPS == 2) {
+                                d = d + interval_flip_cost(lam, a, up, Mw[g] + kap, glo, ghi);
+                            } else {
+                                const long long t = a * (a - (up ? 1 : -1) * (Mw[g] + kap));
+                                d = d + lam * (double)t;
+                            }
                         }
                     }
                     return d;
@@ -212,7 +221,7 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
     for (int c = lane; c < nch; c += 32) D.packedT[(int64_t)c * D.rpad + r_local] = __ldcg(spw + c);
 }
 
-template <bool GROUPS>
+template <int GROUPS>
 __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
     __shared__ long long Msh[GROUPS ? (QA_TPB_MAX / 32) * QA_MAX_GROUPS : 1];
     __shared__ unsigned long long next_read[QA_TPB_MAX / 32];
@@ -264,7 +273,7 @@ namespace qa {
 
 int ref_resident_reads(qa_ctx *ctx, int *out) {
     int bps = 0;
-    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<false>, QA_TPB_MAX, 0));
+    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<0>, QA_TPB_MAX, 0));
     *out = bps * ctx->num_sms * (QA_TPB_MAX / 32);
     return QA_OK;
 }
@@ -291,8 +300,9 @@ int launch_ref(Launch &L) {
     else if (total_reads < (int64_t)ctx->num_sms * wpb) wpb = (int)std::max<int64_t>(1, (total_reads + ctx->num_sms - 1) / ctx->num_sms);
     const int tpb = wpb * 32;
     int bps = 0;
-    if (groups) QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<true>, tpb, 0));
-    else QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<false>, tpb, 0));
+    if (groups && L.interval) QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<2>, tpb, 0));
+    else if (groups) QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<1>, tpb, 0));
+    else QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<0>, tpb, 0));
     if (bps < 1) return fail(QA_ERR_CUDA, "annealing kernel does not fit on an SM");
     int64_t grid = (int64_t)bps * ctx->num_sms;  // multiple of the SM count
     const int64_t need = (total_reads + wpb - 1) / wpb;
@@ -316,8 +326,9 @@ int launch_ref(Launch &L) {
         A.read_begin = done;
         A.read_end = std::min(total_reads, done + wave);
         QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));
-        if (groups) k_anneal_ref<true><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
-        else k_anneal_ref<false><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
+        if (groups && L.interval) k_anneal_ref<2><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
+        else if (groups) k_anneal_ref<1><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
+        else k_anneal_ref<0><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
         QA_CUDA(cudaGetLastError());
         ctx->launches++;
         if (st) st->anneal_launches++;

@@ -241,11 +241,12 @@ int launch_replay(Launch &L) {
     // replay: one CTA = `nw` consecutive 32-read tiles of one problem, coupling slabs shared through a TMA ring
     const int tpp = (reads_per_problem + 31) / 32;
     const int mg = std::max(M->ngroups, 1);
+    const bool ivl = groups && L.interval;
     int nw = ctx->replay_warps;
     if (nw < 1 || nw > RP_MAX_WARPS) {
         nw = 1;
         while (nw < RP_MAX_WARPS && nw < tpp) nw *= 2;
-        while (nw > 1 && rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots) > (size_t)(226 * 1024 / RP_MIN_CTAS - 1024)) nw /= 2;   // RP_MIN_CTAS CTAs per SM
+        while (nw > 1 && rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl) > (size_t)(226 * 1024 / RP_MIN_CTAS - 1024)) nw /= 2;   // RP_MIN_CTAS CTAs per SM
         // less than one full wave of 8-warp CTAs: 4-warp CTAs (3 per SM) balance the SMs better -- measured on config 3
         // (profiles/r2_probe_strong_scaling_read_counts.log): 50 000 reads 7.4e10 against 6.8e10 with 8 warps, 25 000 and 12 500
         // reads within 1 % of the best choice; 1- and 2-warp CTAs are residency-limited by the slab ring's shared memory
@@ -255,9 +256,11 @@ int launch_replay(Launch &L) {
     }
     const int64_t gpp = (tpp + nw - 1) / nw;
     const int64_t total_items = (int64_t)P * gpp;
-    size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots);
+    size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl);
     const void *fn = nullptr;
-    if (M->rp_slots == 32)
+    if (groups && L.interval)
+        fn = M->rp_slots == 32 ? (const void *)k_anneal_replay<3, 32> : (const void *)k_anneal_replay<3, 64>;
+    else if (M->rp_slots == 32)
         fn = !groups ? (const void *)k_anneal_replay<0, 32>
                      : (M->groups_i32 ? (const void *)k_anneal_replay<1, 32> : (const void *)k_anneal_replay<2, 32>);
     else
@@ -311,7 +314,7 @@ int launch_replay(Launch &L) {
             QA_CUDA(cudaStreamSynchronize(ctx->stream));
             if (fl[0] == QA_ERR_SMEM_BASE) {
                 ctx->rp_smem_base = (unsigned)fl[1];
-                smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots);
+                smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl);
                 QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
                 QA_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 2 * sizeof(int), ctx->stream));
                 QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));

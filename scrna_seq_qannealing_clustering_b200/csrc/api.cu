@@ -118,6 +118,7 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
     L.reads_per_problem = reads_per_problem;
     L.total_reads = total_reads;
     L.groups = groups;
+    L.interval = groups && M->gbounds;
     L.seed_mode = seed_mode;
     L.interrupt = interrupt;
     L.iuser = iuser;

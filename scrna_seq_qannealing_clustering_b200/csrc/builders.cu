@@ -386,13 +386,17 @@ static int build_kway(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, cons
     return rc;
 }
 
-int qa_build_cqm_penalty(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, const int32_t *ev, const double *w, int32_t K,
-                         int32_t min_size, double onehot_penalty, double size_penalty, qa_model **out, double *offset_out) {
+// objective + A*(one-hot)^2 + the K cluster-size groups.  slack: B*(N_j - min_size - slack_j)^2 with the binary slack bits
+// behind the n*K cell bits; interval: B*max(0, min_size - N_j)^2, no slack bits (u = 2 (N_j - min_size), bounds [0, +inf)).
+// The cell part (h, couplers, offset) is the same in both: slack bits only appear in the groups.
+static int build_cqm(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, const int32_t *ev, const double *w, int32_t K,
+                     int32_t min_size, double onehot_penalty, double size_penalty, bool interval, qa_model **out,
+                     double *offset_out) {
     if (!ctx || !out || !offset_out) return fail(QA_ERR_ARG, "null argument");
     if (K < 1 || K > QA_MAX_GROUPS) return fail(QA_ERR_LIMIT, "number of clusters must be in [1, QA_MAX_GROUPS]");
     *out = nullptr;
     QA_CUDA(cudaSetDevice(ctx->device));
-    const std::vector<int> coeffs = slack_coefficients_host((int64_t)n - min_size);
+    const std::vector<int> coeffs = interval ? std::vector<int>() : slack_coefficients_host((int64_t)n - min_size);
     const int nb = (int)coeffs.size();
     double off = 0.0;
     qa_model *M = nullptr;
@@ -409,10 +413,24 @@ int qa_build_cqm_penalty(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, c
     std::vector<double> lam(K, size_penalty);
     std::vector<int64_t> kap(K, (int64_t)n - csum - 2 * (int64_t)min_size);
     rc = qa_model_set_groups(M, K, grp.data(), coef.data(), lam.data(), kap.data());
+    if (!rc && interval) {
+        const std::vector<int64_t> lo(K, 0), hi(K, INT64_MAX);
+        rc = qa_model_set_group_bounds(M, lo.data(), hi.data());
+    }
     if (rc) { qa_model_destroy(M); return rc; }
     *offset_out = off + onehot_penalty * n;
     *out = M;
     return QA_OK;
+}
+
+int qa_build_cqm_penalty(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, const int32_t *ev, const double *w, int32_t K,
+                         int32_t min_size, double onehot_penalty, double size_penalty, qa_model **out, double *offset_out) {
+    return build_cqm(ctx, n, m, eu, ev, w, K, min_size, onehot_penalty, size_penalty, false, out, offset_out);
+}
+
+int qa_build_cqm_interval(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, const int32_t *ev, const double *w, int32_t K,
+                          int32_t min_size, double onehot_penalty, double size_penalty, qa_model **out, double *offset_out) {
+    return build_cqm(ctx, n, m, eu, ev, w, K, min_size, onehot_penalty, size_penalty, true, out, offset_out);
 }
 
 int qa_build_dqm_onehot(qa_ctx *ctx, int32_t n, int64_t m, const int32_t *eu, const int32_t *ev, const double *w, int32_t K,

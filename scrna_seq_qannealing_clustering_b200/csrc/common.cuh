@@ -68,7 +68,7 @@ struct ProblemDesc {
     const int32_t *grp;     // [nch*32] or null
     const int32_t *coef;    // [nch*32]
     const double *lambda;   // [ngroups]
-    const long long *kappa; // [ngroups]
+    const long long *kappa; // [ngroups]; interval groups (qa_model_set_group_bounds): [3][ngroups] = kappa, lo, hi
     int8_t *states;         // [reads][n]
     uint32_t *packedT;      // [nch][rpad] final spins, bit i of word (c, r) = spin of variable 32c+i (1: +1)
     double *energies;       // [reads]
@@ -188,6 +188,8 @@ struct qa_model {
     int32_t *grp = nullptr, *coef = nullptr;
     double *lambda = nullptr;
     long long *kappa = nullptr;
+    bool gbounds = false;  // the groups carry interval bounds: kappa[ngroups .. 3 ngroups) = lo, hi (clamped to the reachable range)
+    std::vector<int64_t> gumin, gumax;         // host: reachable range kappa -+ sum |a| of every group (single-problem models)
     qa::ProblemDesc *d_descs = nullptr;
     std::vector<qa::ProblemDesc> descs;  // host mirror (pointers are device pointers)
     // block word tables of the pull variant (built on first use)
@@ -261,6 +263,21 @@ inline int upload(qa_ctx *ctx, T **dst, const T *src, size_t count) {
     return QA_OK;
 }
 
+// Interval rank-1 group term (qa_model_set_group_bounds).  u = sum_g a_v s_v + kappa, d(u) = max(lo - u, 0, u - hi),
+// E = lambda * (double)(d*d) * 0.25.  Flipping a variable with spin s and coefficient a moves u to u - 2 a s; the change of the
+// term is an exact integer difference, scaled by 0.25 (exact) and rounded once by the product with lambda.  For lo = hi = 0,
+// d(u')^2 - d(u)^2 = 4 a (a - s u): bitwise the equality groups' lambda * (double)(a * (a - s u)).  The host keeps every
+// d^2 below 2^53.
+__host__ __device__ __forceinline__ long long interval_dist(long long u, long long lo, long long hi) {
+    return u < lo ? lo - u : (u > hi ? u - hi : 0ll);
+}
+__host__ __device__ __forceinline__ double interval_flip_cost(double lam, long long a, bool up, long long u, long long lo,
+                                                              long long hi) {
+    const long long d0 = interval_dist(u, lo, hi);
+    const long long d1 = interval_dist(up ? u - 2 * a : u + 2 * a, lo, hi);
+    return lam * ((double)(d1 * d1 - d0 * d0) * 0.25);
+}
+
 inline unsigned blocks_for(int64_t count, int tpb = 256) { return (unsigned)std::max<int64_t>(1, (count + tpb - 1) / tpb); }
 
 // device scratch of one build, freed on every path
@@ -292,6 +309,7 @@ struct Launch {
     int32_t reads_per_problem;
     int64_t total_reads;
     bool groups;
+    bool interval;         // the groups carry interval bounds
     int32_t seed_mode;
     qa_interrupt_fn interrupt;
     void *iuser;

@@ -13,6 +13,9 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // energies: neal get_state_energy(), one thread per read, reads on lanes (coalesced packedT loads)
 // ------------------------------------------------------------------------------------------------
+// INTERVAL: the groups carry interval bounds (every problem with groups has them): E_g = lambda * (double)(d*d) * 0.25 with
+// d = max(lo - u, 0, u - hi), u = M_g + kappa_g -- the equality term below is the case lo = hi = 0.
+template <bool INTERVAL>
 __global__ void __launch_bounds__(128) k_energy(const ProblemDesc *descs) {
     const ProblemDesc D = descs[blockIdx.y];
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
@@ -67,7 +70,7 @@ __global__ void __launch_bounds__(128) k_energy(const ProblemDesc *descs) {
         E += (bu ^ bv) ? -wt : wt;
     }
     for (int g = 0; g < D.ngroups; ++g) {
-        const long long t = M[g] + D.kappa[g];
+        const long long t = INTERVAL ? interval_dist(M[g] + D.kappa[g], D.kappa[D.ngroups + g], D.kappa[2 * D.ngroups + g]) : M[g] + D.kappa[g];
         E += D.lambda[g] * (double)(t * t) * 0.25;
     }
     D.energies[r] = E;
@@ -97,7 +100,8 @@ namespace qa {
 
 int launch_energy(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem) {
     dim3 g((unsigned)((reads_per_problem + 127) / 128), (unsigned)M->num_problems);
-    k_energy<<<g, 128, 0, ctx->stream>>>(M->d_descs);
+    if (M->gbounds) k_energy<true><<<g, 128, 0, ctx->stream>>>(M->d_descs);
+    else k_energy<false><<<g, 128, 0, ctx->stream>>>(M->d_descs);
     QA_CUDA(cudaGetLastError());
     ctx->launches++;
     return QA_OK;

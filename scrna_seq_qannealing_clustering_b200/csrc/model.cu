@@ -195,6 +195,9 @@ int qa_model_set_groups(qa_model *M, int32_t ngroups, const int32_t *grp, const 
     if (M->coef) { cudaFree(M->coef); M->coef = nullptr; }
     if (M->lambda) { cudaFree(M->lambda); M->lambda = nullptr; }
     if (M->kappa) { cudaFree(M->kappa); M->kappa = nullptr; }
+    M->gbounds = false;   // new groups are equality groups until bounds are set again
+    M->gumin.clear();
+    M->gumax.clear();
     M->ngroups = ngroups;
     if (ngroups > 0) M->dn_ok = false;   // the dense form carries no group terms
     if (M->rp_slabs) { cudaFree(M->rp_slabs); M->rp_slabs = nullptr; }   // the slabs carry the group metadata
@@ -237,12 +240,54 @@ int qa_model_set_groups(qa_model *M, int32_t ngroups, const int32_t *grp, const 
     QA_CUDA(cudaMalloc((void **)&M->grp, npad * sizeof(int32_t)));
     QA_CUDA(cudaMalloc((void **)&M->coef, npad * sizeof(int32_t)));
     QA_CUDA(cudaMalloc((void **)&M->lambda, ngroups * sizeof(double)));
-    QA_CUDA(cudaMalloc((void **)&M->kappa, ngroups * sizeof(long long)));
+    QA_CUDA(cudaMalloc((void **)&M->kappa, 3 * ngroups * sizeof(long long)));   // room for interval bounds behind kappa
     QA_CUDA(cudaMemcpy(M->grp, hg.data(), npad * sizeof(int32_t), cudaMemcpyHostToDevice));
     QA_CUDA(cudaMemcpy(M->coef, hc.data(), npad * sizeof(int32_t), cudaMemcpyHostToDevice));
     QA_CUDA(cudaMemcpy(M->lambda, lambda, ngroups * sizeof(double), cudaMemcpyDefault));
     QA_CUDA(cudaMemcpy(M->kappa, hk.data(), ngroups * sizeof(long long), cudaMemcpyHostToDevice));
     D.grp = M->grp; D.coef = M->coef; D.lambda = M->lambda; D.kappa = M->kappa;
+    M->gumin.resize(ngroups);
+    M->gumax.resize(ngroups);
+    for (int g = 0; g < ngroups; ++g) {   // span < 2^31 above: exact
+        M->gumin[g] = hk[g] - (int64_t)sumabs[g];
+        M->gumax[g] = hk[g] + (int64_t)sumabs[g];
+    }
+    return QA_OK;
+}
+
+int qa_model_set_group_bounds(qa_model *M, const int64_t *lo, const int64_t *hi) {
+    if (!M) return fail(QA_ERR_ARG, "null model");
+    if (M->num_problems != 1) return fail(QA_ERR_ARG, "group bounds need a single-problem model");
+    if ((lo == nullptr) != (hi == nullptr)) return fail(QA_ERR_ARG, "lo and hi must both be given or both be null");
+    qa_ctx *ctx = M->ctx;
+    QA_CUDA(cudaSetDevice(ctx->device));
+    const int G = M->ngroups;
+    if (lo && G == 0) return fail(QA_ERR_ARG, "no groups: call qa_model_set_groups first");
+    std::vector<long long> hl(G), hh(G);
+    if (lo) {
+        QA_CUDA(cudaMemcpy(hl.data(), lo, (size_t)G * sizeof(int64_t), cudaMemcpyDefault));
+        QA_CUDA(cudaMemcpy(hh.data(), hi, (size_t)G * sizeof(int64_t), cudaMemcpyDefault));
+        for (int g = 0; g < G; ++g) {
+            if (hl[g] > hh[g]) return fail(QA_ERR_ARG, "group bound lo > hi");
+            // u stays in [umin, umax]: a bound beyond that range never binds, so clamping it leaves d(u) unchanged there
+            hl[g] = std::max<long long>(hl[g], M->gumin[g]);
+            hh[g] = std::min<long long>(hh[g], M->gumax[g]);
+            const __int128 dmax = std::max<__int128>(std::max<__int128>((__int128)hl[g] - M->gumin[g], (__int128)M->gumax[g] - hh[g]), 0);
+            if (dmax * dmax >= ((__int128)1 << 53)) return fail(QA_ERR_LIMIT, "group bounds too far from the reachable range for exact integer evaluation");
+        }
+    }
+    if (M->rp_slabs) { cudaFree(M->rp_slabs); M->rp_slabs = nullptr; }
+    if (M->rp_off) { cudaFree(M->rp_off); M->rp_off = nullptr; }
+    M->rp_built = false;
+    M->rp_ok = false;
+    ProblemDesc &D = M->descs[0];
+    D.rp_slabs = nullptr;
+    D.rp_off = nullptr;
+    M->gbounds = false;
+    if (!lo) return QA_OK;
+    QA_CUDA(cudaMemcpy(M->kappa + G, hl.data(), (size_t)G * sizeof(long long), cudaMemcpyHostToDevice));
+    QA_CUDA(cudaMemcpy(M->kappa + 2 * G, hh.data(), (size_t)G * sizeof(long long), cudaMemcpyHostToDevice));
+    M->gbounds = true;
     return QA_OK;
 }
 

@@ -222,7 +222,9 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
     M->var_off.assign(num_models + 1, 0);
     M->cpl_off.assign(num_models + 1, 0);
     int64_t gpad = 0, gcount = 0;
+    bool bounds = false;   // some input carries interval bounds: every problem with groups gets them (equality: lo = hi = 0)
     for (int p = 0; p < num_models; ++p) {
+        bounds = bounds || models[p]->gbounds;
         M->var_off[p + 1] = M->var_off[p] + models[p]->n_total;
         M->cpl_off[p + 1] = M->cpl_off[p] + models[p]->m_total;
         M->max_deg = std::max(M->max_deg, models[p]->max_deg);
@@ -255,7 +257,8 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
         CAT_CUDA(cudaMalloc((void **)&M->grp, (size_t)std::max<int64_t>(gpad, 1) * sizeof(int32_t)));
         CAT_CUDA(cudaMalloc((void **)&M->coef, (size_t)std::max<int64_t>(gpad, 1) * sizeof(int32_t)));
         CAT_CUDA(cudaMalloc((void **)&M->lambda, (size_t)std::max<int64_t>(gcount, 1) * sizeof(double)));
-        CAT_CUDA(cudaMalloc((void **)&M->kappa, (size_t)std::max<int64_t>(gcount, 1) * sizeof(long long)));
+        CAT_CUDA(cudaMalloc((void **)&M->kappa, (size_t)std::max<int64_t>(gcount, 1) * (bounds ? 3 : 1) * sizeof(long long)));
+        M->gbounds = bounds;
     }
     const int tpb = 256;
     auto blocks = [&](int64_t c) { return (unsigned)std::max<int64_t>(1, (c + tpb - 1) / tpb); };
@@ -286,13 +289,19 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
         CAT_CUDA(cudaMemcpyAsync(M->grp + go, S->grp, (size_t)npad * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
         CAT_CUDA(cudaMemcpyAsync(M->coef + go, S->coef, (size_t)npad * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
         CAT_CUDA(cudaMemcpyAsync(M->lambda + gl, S->lambda, (size_t)S->ngroups * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        CAT_CUDA(cudaMemcpyAsync(M->kappa + gl, S->kappa, (size_t)S->ngroups * sizeof(long long), cudaMemcpyDeviceToDevice, ctx->stream));
+        const int64_t gk = bounds ? 3 * gl : gl;   // interval bounds: {kappa, lo, hi} of every problem stay together
+        CAT_CUDA(cudaMemcpyAsync(M->kappa + gk, S->kappa, (size_t)S->ngroups * sizeof(long long), cudaMemcpyDeviceToDevice, ctx->stream));
+        if (bounds) {
+            const size_t gb = 2 * (size_t)S->ngroups * sizeof(long long);
+            if (S->gbounds) CAT_CUDA(cudaMemcpyAsync(M->kappa + gk + S->ngroups, S->kappa + S->ngroups, gb, cudaMemcpyDeviceToDevice, ctx->stream));
+            else CAT_CUDA(cudaMemsetAsync(M->kappa + gk + S->ngroups, 0, gb, ctx->stream));   // equality groups: lo = hi = 0
+        }
         ProblemDesc &D = M->descs[p];
         D.ngroups = S->ngroups;
         D.grp = M->grp + go;
         D.coef = M->coef + go;
         D.lambda = M->lambda + gl;
-        D.kappa = M->kappa + gl;
+        D.kappa = M->kappa + gk;
         go += npad;
         gl += S->ngroups;
     }

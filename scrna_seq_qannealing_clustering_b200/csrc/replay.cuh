@@ -243,7 +243,8 @@ __device__ __forceinline__ void rp_stage_wait() {
 // One pass over all blocks.  MODE 0: replay sweep.  MODE 1: catch-up (pending later-neighbour updates only, no decisions).
 // MODE 2: push sweep (neal's eager form).  MODE 3: field set-up f[v] = h_v + sum_j J_vj s_j in neal's get_flip_energy order,
 // for models whose adjacency lists are ascending (then adjacency order = pre entries u < v0, seq entries, later entries).
-// GROUPS: 0 none, 1 rank-1 groups with 32-bit exact integer arithmetic (host-checked ranges), 2 with 64-bit.
+// GROUPS: 0 none, 1 rank-1 groups with 32-bit exact integer arithmetic (host-checked ranges), 2 with 64-bit, 3 interval groups
+// (64-bit; c.kap then holds {kappa, lo, hi} per group).
 template <int MODE, int GROUPS, int SLOTS>
 __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
     const int lane = threadIdx.x & 31;
@@ -391,6 +392,9 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                             const int m = c.Mcol[g * c.mstride] + reinterpret_cast<const int *>(c.kap)[2 * g];
                             const int t = ca * (ca - (up ? m : -m));
                             dE = dE + c.lam[g] * (double)t;
+                        } else if (GROUPS == 3) {
+                            const long long *kb = c.kap + 3 * g;
+                            dE = dE + interval_flip_cost(c.lam[g], ca, up, (long long)c.Mcol[g * c.mstride] + kb[0], kb[1], kb[2]);
                         } else {
                             const long long t = (long long)ca * ((long long)ca - (up ? 1 : -1) * ((long long)c.Mcol[g * c.mstride] + c.kap[g]));
                             dE = dE + c.lam[g] * (double)t;
@@ -503,6 +507,9 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                             const int m = c.Mcol[g * c.mstride] + reinterpret_cast<const int *>(c.kap)[2 * g];
                             const int t = ca * (ca - (up ? m : -m));
                             dE = dE + c.lam[g] * (double)t;
+                        } else if (GROUPS == 3) {
+                            const long long *kb = c.kap + 3 * g;
+                            dE = dE + interval_flip_cost(c.lam[g], ca, up, (long long)c.Mcol[g * c.mstride] + kb[0], kb[1], kb[2]);
                         } else {
                             const long long t = (long long)ca * ((long long)ca - (up ? 1 : -1) * ((long long)c.Mcol[g * c.mstride] + c.kap[g]));
                             dE = dE + c.lam[g] * (double)t;
@@ -596,14 +603,14 @@ __device__ __forceinline__ double rp_field_direct(const ProblemDesc &D, const ui
 // the shared window (so that a slot address is formed by OR), one slot region per warp, then one partial-sum region per warp.
 // `smem_base` is the shared-window offset of the dynamic allocation (1 KB on sm_100: the system-reserved bytes); the kernel
 // verifies the assumption.
-__host__ __device__ inline size_t rp_fixed_bytes(int nw, int max_groups) {
+__host__ __device__ inline size_t rp_fixed_bytes(int nw, int max_groups, bool interval = false) {
     size_t b = (size_t)RP_STAGES * RP_STAGE_BYTES + 8 * (2 * RP_STAGES) + 32;
-    b += (sizeof(double) + sizeof(long long)) * (size_t)max_groups;
+    b += (sizeof(double) + (interval ? 3 : 1) * sizeof(long long)) * (size_t)max_groups;   // interval: {kappa, lo, hi}
     b += sizeof(int) * (size_t)max_groups * nw * 32;
     return b;
 }
-__host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned smem_base, int slots) {
-    const size_t fixed = rp_fixed_bytes(nw, max_groups);
+__host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned smem_base, int slots, bool interval = false) {
+    const size_t fixed = rp_fixed_bytes(nw, max_groups, interval);
     const size_t sf = (size_t)rp_sf_bytes(slots);
     const size_t pad = (sf - (smem_base + fixed) % sf) % sf;
     return fixed + pad + (size_t)nw * (sf + RP_PS_BYTES);
@@ -618,7 +625,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     const int NW = blockDim.x >> 5;
     uint32_t raw_s;   // opaque to the compiler: it would otherwise re-derive the window address (S2R + LEA) inside the hot loops
     asm volatile("mov.u32 %0, %1;" : "=r"(raw_s) : "r"((uint32_t)__cvta_generic_to_shared(rp_raw)));
-    const uint32_t fixed = (uint32_t)rp_fixed_bytes(NW, P.max_groups);
+    const uint32_t fixed = (uint32_t)rp_fixed_bytes(NW, P.max_groups, GROUPS == 3);
     const uint32_t base_s = (raw_s + fixed + (uint32_t)RP_SF_BYTES - 1u) & ~((uint32_t)RP_SF_BYTES - 1u);    // warp regions
     {
         uint32_t dyn;
@@ -638,7 +645,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     unsigned *acc_sh = reinterpret_cast<unsigned *>(tail + 8 * (2 * RP_STAGES) + 16);   // [2]
     double *lam_sh = reinterpret_cast<double *>(tail + 8 * (2 * RP_STAGES) + 32);
     long long *kap_sh = reinterpret_cast<long long *>(lam_sh + P.max_groups);
-    int *M_all = reinterpret_cast<int *>(kap_sh + P.max_groups);
+    int *M_all = reinterpret_cast<int *>(kap_sh + (GROUPS == 3 ? 3 : 1) * P.max_groups);
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < RP_STAGES; ++s) {
@@ -654,7 +661,13 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
         const ProblemDesc &D0 = P.descs[0];
         for (int g = threadIdx.x; g < D0.ngroups; g += blockDim.x) {
             lam_sh[g] = D0.lambda[g];
-            kap_sh[g] = D0.kappa[g];
+            if (GROUPS == 3) {
+                kap_sh[3 * g] = D0.kappa[g];
+                kap_sh[3 * g + 1] = D0.kappa[D0.ngroups + g];
+                kap_sh[3 * g + 2] = D0.kappa[2 * D0.ngroups + g];
+            } else {
+                kap_sh[g] = D0.kappa[g];
+            }
         }
     }
     __syncthreads();

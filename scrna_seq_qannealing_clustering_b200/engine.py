@@ -287,6 +287,15 @@ class Context:
                                                C.byref(off)))
         return IsingModel._from_handle(self, hm), float(off.value)
 
+    def build_cqm_interval(self, graph, num_clusters: int, min_size: int, onehot_penalty: float, size_penalty: float):
+        """``clustering_cqm`` model with the size constraints as interval groups, no slack variables
+        (``qa_build_cqm_interval``: B * max(0, min_size - N_j)^2).  -> (IsingModel, offset)"""
+        n, m, eu, ev, w = self._graph_args(graph)
+        hm, off = C.c_void_p(), C.c_double()
+        check(_lib.load().qa_build_cqm_interval(self._h, n, m, ptr(eu), ptr(ev), ptr(w), int(num_clusters), int(min_size),
+                                                float(onehot_penalty), float(size_penalty), C.byref(hm), C.byref(off)))
+        return IsingModel._from_handle(self, hm), float(off.value)
+
     def build_dqm_onehot(self, graph, num_cases: int, gamma: float, penalty: float, semantics: str = "as_written"):
         """``clustering_dqm`` model (DQM_clustering.py:29-43), one-hot expanded and structured.  -> (IsingModel, offset)"""
         n, m, eu, ev, w = self._graph_args(graph)
@@ -424,7 +433,11 @@ class IsingModel:
         self.num_groups = 0
         return self
 
-    def set_groups(self, grp, coef, lam, kappa):
+    def set_groups(self, grp, coef, lam, kappa, lo=None, hi=None):
+        """Rank-1 groups (``qa_model_set_groups``); with ``lo`` / ``hi`` (int64 [G]) interval groups
+        (``qa_model_set_group_bounds``): lam/4 * max(lo - u, 0, u - hi)^2 instead of lam/4 * u^2."""
+        if (lo is None) != (hi is None):
+            raise ValueError("give both lo and hi, or neither")
         grp = np.ascontiguousarray(grp, dtype=np.int32)
         coef = np.ascontiguousarray(coef, dtype=np.int32)
         lam = np.ascontiguousarray(lam, dtype=np.float64)
@@ -433,6 +446,19 @@ class IsingModel:
             raise ValueError("grp/coef must have one entry per variable")
         check(_lib.load().qa_model_set_groups(self._h, int(lam.shape[0]), ptr(grp), ptr(coef), ptr(lam), ptr(kappa)))
         self.num_groups = int(lam.shape[0])
+        if lo is not None:
+            self.set_group_bounds(lo, hi)
+
+    def set_group_bounds(self, lo, hi):
+        """Interval bounds of the groups set last (``qa_model_set_group_bounds``); ``None, None``: equality groups again."""
+        if lo is None and hi is None:
+            check(_lib.load().qa_model_set_group_bounds(self._h, None, None))
+            return
+        lo = np.ascontiguousarray(lo, dtype=np.int64)
+        hi = np.ascontiguousarray(hi, dtype=np.int64)
+        if lo.shape != (self.num_groups,) or hi.shape != (self.num_groups,):
+            raise ValueError("lo/hi must have one entry per group")
+        check(_lib.load().qa_model_set_group_bounds(self._h, ptr(lo), ptr(hi)))
 
     def enable_dense(self, cases_per_cell: int = 1) -> bool:
         """Derive the dense k-way form (W, P) on the device; True when the model has it: ``mode=QA_MODE_THROUGHPUT`` then runs the

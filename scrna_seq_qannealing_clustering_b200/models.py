@@ -29,9 +29,19 @@ class Groups:
     coef: np.ndarray     # int32 [n]  a_v
     lam: np.ndarray      # float64 [G]
     kappa: np.ndarray    # int64 [G]
+    # interval groups (include/qanneal.h qa_model_set_group_bounds): lam/4 * d(u)^2 with u = sum a_v s_v + kappa and
+    # d(u) = max(lo - u, 0, u - hi); int64 [G], INT64_MIN / INT64_MAX for an open side.  None: equality groups (lam/4 * u^2)
+    lo: Optional[np.ndarray] = None
+    hi: Optional[np.ndarray] = None
+
+    @property
+    def interval(self) -> bool:
+        return self.lo is not None
 
     def astuple(self):
-        return self.grp, self.coef, self.lam, self.kappa
+        if self.lo is None:
+            return self.grp, self.coef, self.lam, self.kappa
+        return self.grp, self.coef, self.lam, self.kappa, self.lo, self.hi
 
 
 @dataclass
@@ -57,6 +67,8 @@ class LoweredModel:
         """Expand the rank-1 groups into explicit couplers (J_ij += lam a_i a_j / 2, h_i += lam kappa a_i / 2)."""
         if self.groups is None:
             return self
+        if self.groups.interval:
+            raise ValueError("interval groups are not quadratic: they have no coupler form")
         n = self.num_variables
         dense = np.zeros((n, n), dtype=np.float64)
         dense[self.starts, self.ends] = self.weights
@@ -89,7 +101,10 @@ class LoweredModel:
             for gi in range(len(g.lam)):
                 idx = g.grp == gi
                 M = s[:, idx] @ g.coef[idx].astype(np.float64)
-                e = e + g.lam[gi] / 4.0 * (M + float(g.kappa[gi])) ** 2
+                u = M + float(g.kappa[gi])
+                if g.interval:
+                    u = np.maximum(np.maximum(float(g.lo[gi]) - u, 0.0), u - float(g.hi[gi]))
+                e = e + g.lam[gi] / 4.0 * u ** 2
         return e
 
 
@@ -348,9 +363,22 @@ def slack_coefficients(upper: int) -> List[int]:
     return coeffs
 
 
+SIZE_LOWERINGS = ("slack", "interval")
+INT64_MIN, INT64_MAX = np.iinfo(np.int64).min, np.iinfo(np.int64).max
+
+
+def _cqm_size_penalty(A: float, n: int, size_lowering: str) -> float:
+    """Default B.  slack: B = A / n (see cqm_model).  interval: B = A -- a single flip gains less than A in objective (A is
+    above every cell's objective scale by construction), so one unit of size violation costs more than any flip can gain;
+    A / n was a workaround for frozen slack bits, which the interval form does not have."""
+    if size_lowering not in SIZE_LOWERINGS:
+        raise ValueError(f"size_lowering must be one of {SIZE_LOWERINGS}, not {size_lowering!r}")
+    return A if size_lowering == "interval" else A / max(n, 1)
+
+
 def cqm_model(G, num_of_clusters: int, min_size: int = 20, onehot_penalty: Optional[float] = None,
               size_penalty: Optional[float] = None, subindex: Optional[Sequence[int]] = None,
-              structured: bool = True) -> LoweredModel:
+              structured: bool = True, size_lowering: str = "slack") -> LoweredModel:
     """``clustering_cqm`` / ``clustering_cqm_2`` model (CQM_clustering.py:30-48, 62-84) lowered to penalties.
 
     objective  sum_edges sum_p (x_ip + x_jp - 2*w_ij*x_ip*x_jp)            (:40-44; linear coefficient is 1, not w)
@@ -360,6 +388,10 @@ def cqm_model(G, num_of_clusters: int, min_size: int = 20, onehot_penalty: Optio
     Variable (cell i, cluster p) -> i*K + p with label 'v_{i},{p}' (i = node label, or ``subindex`` for cqm_2);
     slack sigma_jb -> n*K + j*nb + b with label 'slack_cluster_size{j}_{b}'.  A and B are ours (Leap's CQM solver
     handles constraints natively; defaults A = max degree + max sum |2w| + 1, B = A / n) and are reported in ``meta``.
+
+    ``size_lowering="interval"``: no slack bits; each size constraint is an interval group with bounds [0, +inf) on
+    u = 2 (N_j - min_size), i.e. the term  B * max(0, min_size - N_j)^2, evaluated by the kernels from the group counter.
+    The cell part (h, couplers, offset) is the slack model's, bit for bit.  Default B = A (see ``_cqm_size_penalty``).
     """
     labels, eu, ev, w = graph_arrays(G)
     n, K = len(labels), int(num_of_clusters)
@@ -371,8 +403,9 @@ def cqm_model(G, num_of_clusters: int, min_size: int = 20, onehot_penalty: Optio
     # the binary slack bits (coefficients up to ~n/2) freeze at every temperature the objective cares about, the cell bits are
     # slaved to them and no read ends one-hot (measured: 0 of 100 000 reads on config 3); with B = A/n every read of the same
     # job is feasible.  The reference never meets this: Leap's CQM solver handles constraints natively.
-    B = A / max(n, 1) if size_penalty is None else float(size_penalty)
-    coeffs = slack_coefficients(n - min_size)
+    B = _cqm_size_penalty(A, n, size_lowering) if size_penalty is None else float(size_penalty)
+    interval = size_lowering == "interval"
+    coeffs = [] if interval else slack_coefficients(n - min_size)
     nb = len(coeffs)
     names = labels if subindex is None else list(subindex)
     var_labels: List[Hashable] = [f"v_{names[i]},{p}" for i in range(n) for p in range(K)]
@@ -398,8 +431,12 @@ def cqm_model(G, num_of_clusters: int, min_size: int = 20, onehot_penalty: Optio
         coef[sl] = -np.asarray(coeffs, dtype=np.int32)
     kappa = np.full(K, n - sum(coeffs) - 2 * min_size, dtype=np.int64)
     groups = Groups(grp, coef, np.full(K, B), kappa)
+    if interval:
+        groups.lo, groups.hi = np.zeros(K, dtype=np.int64), np.full(K, INT64_MAX, dtype=np.int64)
     meta = {"kind": "cqm", "builder": "cqm", "num_cases": K, "cells": labels, "names": list(names), "min_size": min_size,
-            "onehot_penalty": A, "size_penalty": B, "slack_coefficients": coeffs, "num_cell_variables": nx_}
+            "onehot_penalty": A, "size_penalty": B, "num_cell_variables": nx_, "size_lowering": size_lowering}
+    if not interval:
+        meta["slack_coefficients"] = coeffs
     model = LoweredModel(h, r, c, J, off + A * n, var_labels, groups, meta)
     return model if structured else model.materialise()
 
@@ -470,14 +507,18 @@ def device_spec(kind: str, G, **p) -> Dict:
         deg = _edge_order_sum(n, eu, ev, np.ones(len(w)))
         wdeg = _edge_order_sum(n, eu, ev, np.abs(2 * w))
         A = float(deg.max() + wdeg.max() + 1.0) if p.get("onehot_penalty") is None else float(p["onehot_penalty"])
-        B = A / max(n, 1) if p.get("size_penalty") is None else float(p["size_penalty"])      # see cqm_model
-        coeffs = slack_coefficients(n - min_size)
+        size_lowering = p.get("size_lowering", "slack")
+        B = _cqm_size_penalty(A, n, size_lowering) if p.get("size_penalty") is None else float(p["size_penalty"])  # see cqm_model
+        coeffs = [] if size_lowering == "interval" else slack_coefficients(n - min_size)
         names = labels if p.get("subindex") is None else list(p["subindex"])
         var_labels: List[Hashable] = [f"v_{names[i]},{q}" for i in range(n) for q in range(K)]
         var_labels += [f"slack_cluster_size{j}_{b}" for j in range(K) for b in range(len(coeffs))]
         meta = {"kind": "cqm", "builder": "cqm", "num_cases": K, "cells": labels, "names": list(names), "min_size": min_size,
-                "onehot_penalty": A, "size_penalty": B, "slack_coefficients": coeffs, "num_cell_variables": n * K}
-        return {"graph": graph, "labels": var_labels, "meta": meta, "onehot_penalty": A, "size_penalty": B, "min_size": min_size}
+                "onehot_penalty": A, "size_penalty": B, "num_cell_variables": n * K, "size_lowering": size_lowering}
+        if size_lowering != "interval":
+            meta["slack_coefficients"] = coeffs
+        return {"graph": graph, "labels": var_labels, "meta": meta, "onehot_penalty": A, "size_penalty": B, "min_size": min_size,
+                "size_lowering": size_lowering}
     raise ValueError(f"unknown model kind {kind!r}")
 
 

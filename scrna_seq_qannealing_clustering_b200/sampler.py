@@ -142,19 +142,22 @@ class B200SimulatedAnnealingSampler:
         return _decode_discrete(ss, model, dqm if isinstance(dqm, DiscreteQuadraticModel) else None)
 
     def sample_cqm(self, cqm, onehot_penalty: Optional[float] = None, constraint_penalty: Optional[float] = None,
-                   slack_init: str = "consistent", **parameters) -> SampleSet:
+                   slack_init: str = "consistent", size_lowering: str = "slack", **parameters) -> SampleSet:
         """``LeapHybridCQMSampler().sample_cqm`` stand-in (CQM_clustering.py:53,89): constraints lowered to penalties.
 
         Rows keep the binary variables ('v_{i},{k}' and slack bits); record fields ``is_feasible`` (one-hot and
         minimum-size constraints satisfied by the cell variables) and ``objective`` are added.
         ``slack_init='consistent'`` (default): generated initial states get slack bits that encode their own cluster sizes, so
         the size penalty starts at zero (``models.consistent_slack``); ``'random'``: dimod's uniformly random states.
+        ``size_lowering`` ('slack' or 'interval') lowers a ConstrainedQuadraticModel's linear constraints
+        (``ConstrainedQuadraticModel.to_lowered(lowering=)``); an already lowered model keeps its own lowering (models built
+        with ``size_lowering='interval'`` have no slack bits, and ``slack_init`` does not apply to them).
         """
         from .cqm import ConstrainedQuadraticModel
         if isinstance(cqm, (LoweredModel, DeviceModel)):
             model = cqm
         elif isinstance(cqm, ConstrainedQuadraticModel):
-            model = cqm.to_lowered(onehot_penalty, constraint_penalty)
+            model = cqm.to_lowered(onehot_penalty, constraint_penalty, lowering=size_lowering)
         else:
             raise TypeError("sample_cqm expects a ConstrainedQuadraticModel or a LoweredModel built by models.cqm_model")
         meta = getattr(model, "meta", {})
@@ -189,6 +192,9 @@ class B200SimulatedAnnealingSampler:
         elif kind == "dqm":
             gm, off = ctx.build_dqm_onehot(spec["graph"], params["num_of_clusters"], params["gamma"], spec["penalty"],
                                            params.get("semantics", "as_written"))
+        elif spec["size_lowering"] == "interval":
+            gm, off = ctx.build_cqm_interval(spec["graph"], params["num_of_clusters"], spec["min_size"], spec["onehot_penalty"],
+                                             spec["size_penalty"])
         else:
             gm, off = ctx.build_cqm_penalty(spec["graph"], params["num_of_clusters"], spec["min_size"], spec["onehot_penalty"],
                                             spec["size_penalty"])

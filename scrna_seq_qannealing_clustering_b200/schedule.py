@@ -19,7 +19,8 @@ def default_ising_beta_range(h: np.ndarray, irow: np.ndarray, icol: np.ndarray, 
     """neal ``_default_ising_beta_range``: hot = ln2 / max_v(|h_v| + sum_j |J_vj|), cold = ln100 / min nonzero |bias|.
 
     ``groups`` = (grp, coef, lam, kappa) adds the couplings a rank-1 term would contribute if it were
-    materialised (J_ij += lam*a_i*a_j/2, h_i += lam*kappa*a_i/2), so both forms get the same range.
+    materialised (J_ij += lam*a_i*a_j/2, h_i += lam*kappa*a_i/2), so both forms get the same range.  Interval groups
+    (grp, coef, lam, kappa, lo, hi) get the range of their equality form: the same scale of flip costs.
     """
     h = np.asarray(h, dtype=np.float64)
     q = np.asarray(qdata, dtype=np.float64)
@@ -30,7 +31,7 @@ def default_ising_beta_range(h: np.ndarray, irow: np.ndarray, icol: np.ndarray, 
         np.add.at(field, icol, np.abs(q))
     nz = [abs_h[abs_h != 0], np.abs(q[q != 0])]
     if groups is not None:
-        grp, coef, lam, kappa = groups
+        grp, coef, lam, kappa = groups[:4]
         grp = np.asarray(grp)
         coef = np.abs(np.asarray(coef, dtype=np.float64))
         for g in range(len(lam)):
