@@ -64,9 +64,11 @@ int launch_dense(Launch &L) {
 extern "C" {
 
 // Dense k-way form for k_anneal_dense: W[i][j] = J between (i,c) and (j,c), P = J between two cases of one cell, derived
-// from the device CSR and verified (every inter-cell coupler joins equal cases and does not depend on the case, every
-// intra-cell coupler equals P).  Returns 1 when the model has that structure (QA_MODE_THROUGHPUT then runs the
-// tensor-core kernel), 0 when it does not (nothing changes).
+// from the device CSR and verified: every inter-cell coupler joins equal cases, appears once, and a pair of cells is coupled in
+// all K cases with one weight or in none; every cell has all K(K-1)/2 intra-cell couplers once, each equal to P, or no cell
+// has any (P = 0).  The kernel anneals exactly that model, so anything else must stay on the reference-order kernels.
+// Returns 1 when the model has that structure (QA_MODE_THROUGHPUT then runs the tensor-core kernel), 0 when it does not
+// (nothing changes).
 int qa_model_enable_dense(qa_model *M, int32_t K) {
     if (!M) return fail(QA_ERR_ARG, "null model");
     if (K != 1 && K != 2 && K != 4 && K != 8) return fail(QA_ERR_ARG, "dense form: cases per cell must be 1, 2, 4 or 8");
@@ -98,24 +100,33 @@ int qa_model_enable_dense(qa_model *M, int32_t K) {
     QA_CUDA(cudaMalloc((void **)&M->dn_W, cells2 * sizeof(double)));
     unsigned long long *Wb = reinterpret_cast<unsigned long long *>(M->dn_W);
     unsigned long long *d_counts = nullptr;
-    QA_CUDA(cudaMalloc((void **)&d_counts, 2 * sizeof(unsigned long long)));
-    QA_CUDA(cudaMemsetAsync(d_counts, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    unsigned int *d_seen = nullptr;     // one byte per cell pair (ncp is a multiple of 32: whole words)
+    QA_CUDA(cudaMalloc((void **)&d_counts, 3 * sizeof(unsigned long long)));
+    cudaError_t ce = cudaMalloc((void **)&d_seen, cells2);
+    if (ce != cudaSuccess) {
+        cudaFree(d_counts);
+        return fail(QA_ERR_CUDA, std::string("dense form: ") + cudaGetErrorString(ce));
+    }
+    QA_CUDA(cudaMemsetAsync(d_counts, 0, 3 * sizeof(unsigned long long), ctx->stream));
+    QA_CUDA(cudaMemsetAsync(d_seen, 0, cells2, ctx->stream));
     QA_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 2 * sizeof(int), ctx->stream));
     const int tpb = 256;
     k_dense_fill<<<(unsigned)((cells2 + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(cells2, Wb);
     for (int pass = 0; pass < 2; ++pass)
         k_dense_scatter<<<(unsigned)((n + tpb - 1) / tpb), tpb, 0, ctx->stream>>>((int32_t)n, K, ncp, M->rowptr, M->col, M->val, Pj, Wb,
-                                                                                 ctx->d_flag, d_counts, pass);
+                                                                                 d_seen, ctx->d_flag, d_counts, pass);
     k_dense_finish<<<(unsigned)((cells2 + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(cells2, Wb);
     ctx->launches += 4;
     int flag = 0;
-    unsigned long long counts[2] = {0, 0};
-    cudaError_t ce = cudaMemcpyAsync(&flag, ctx->d_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
+    unsigned long long counts[3] = {0, 0, 0};
+    ce = cudaMemcpyAsync(&flag, ctx->d_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(counts, d_counts, sizeof(counts), cudaMemcpyDeviceToHost, ctx->stream);
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
     cudaFree(d_counts);
+    cudaFree(d_seen);
     if (ce != cudaSuccess) return fail(QA_ERR_CUDA, std::string("dense form: ") + cudaGetErrorString(ce));
-    if (flag != 0 || counts[0] * (unsigned long long)K != counts[1]) {
+    const unsigned long long onehot_full = (unsigned long long)n * (unsigned long long)(K - 1);
+    if (flag != 0 || counts[0] * (unsigned long long)K != counts[1] || (counts[2] != 0 && counts[2] != onehot_full)) {
         cudaFree(M->dn_W);
         M->dn_W = nullptr;
         return 0;

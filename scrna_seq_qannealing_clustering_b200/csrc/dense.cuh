@@ -133,7 +133,6 @@ __global__ void __launch_bounds__(128, (K >= 8 ? 2 : DN_MIN_CTAS)) k_anneal_dens
     uint32_t *SW = P.dn_spins + ((size_t)blockIdx.x * (blockDim.x >> 5) + wib) * (size_t)P.dn_stride;
     const int n = D.n, ncells = Dd.ncells;
     const double Pj = Dd.P;
-    const unsigned long long deg = (unsigned long long)(ncells - 1 + K - 1);
     unsigned long long tot[5] = {0, 0, 0, 0, 0};
 
     for (;;) {
@@ -194,6 +193,10 @@ __global__ void __launch_bounds__(128, (K >= 8 ? 2 : DN_MIN_CTAS)) k_anneal_dens
                         if (i >= ncells) break;
                         double f[K];
                         int s[K];
+                        // neighbour updates count neal's way: the CSR degree of the flipped variable (zeros of W are absent)
+                        int32_t rp[K + 1];
+#pragma unroll
+                        for (int c = 0; c <= K; ++c) rp[c] = __ldg(D.rowptr + (size_t)i * K + c);
 #pragma unroll
                         for (int c = 0; c < K; ++c) {
                             f[c] = Fb[m * LD + lane * K + c] + __ldg(D.h + (size_t)i * K + c);
@@ -211,7 +214,7 @@ __global__ void __launch_bounds__(128, (K >= 8 ? 2 : DN_MIN_CTAS)) k_anneal_dens
                             const bool acc = ls_accept(dE, cand, beta, s0, s1, st);
                             if (acc) {
                                 st.acc++;
-                                st.nbr += deg;
+                                st.nbr += (unsigned)(rp[c + 1] - rp[c]);
                                 s[c] = -s[c];
                                 wv[c] ^= 1u << (b0 + m);
                                 dirty = true;
@@ -297,7 +300,12 @@ __global__ void __launch_bounds__(128, (K >= 8 ? 2 : DN_MIN_CTAS)) k_anneal_dens
 
 // ---- structure detection: scatter the CSR of a one-hot k-way model into W, verifying the Kronecker form ---------------
 // flag bits: 1 = coupler between different cells AND different cases, 2 = case-dependent inter-cell coupling,
-//            4 = duplicate coupler, 8 = intra-cell couplings differ
+//            4 = duplicate inter-cell coupler, 8 = intra-cell couplings differ, 16 = a cell's one-hot couplers are neither all
+//            present once nor all absent
+// The host then requires (counts[0] = case-0 inter-cell entries, counts[1] = all same-case inter-cell entries, counts[2] =
+// intra-cell entries) counts[1] == K * counts[0] -- with no duplicates and every entry of row (i, c) found in row (i, 0), every
+// row (i, c) then holds exactly the cells of row (i, 0) -- and counts[2] == 0 or n * (K - 1): all cells complete, or none
+// has one-hot couplers (P = 0).
 constexpr unsigned long long DN_EMPTY = 0x7ff8dead00000001ull;   // a NaN payload no input produces
 
 __global__ void k_dense_fill(size_t count, unsigned long long *W) {
@@ -305,19 +313,25 @@ __global__ void k_dense_fill(size_t count, unsigned long long *W) {
     if (i < count) W[i] = DN_EMPTY;
 }
 
-// pass 0: case-0 entries claim their cell of W; intra-cell entries are compared with P
+// pass 0: case-0 entries write their cell of W, every same-case inter-cell entry sets bit c of seen[i][j] (a bit already set is
+// a duplicate), intra-cell entries are compared with P and must cover the other K - 1 cases exactly once or not at all;
+// pass 1: the entries of cases 1..K-1 are compared with W
 __global__ void k_dense_scatter(int32_t n, int32_t K, int32_t ncp, const int32_t *rowptr, const int32_t *col, const double *val,
-                                double P, unsigned long long *W, int *flag, unsigned long long *counts, int pass) {
+                                double P, unsigned long long *W, unsigned int *seen, int *flag, unsigned long long *counts,
+                                int pass) {
     const int v = blockIdx.x * blockDim.x + threadIdx.x;
     if (v >= n) return;
     const int i = v / K, c = v % K;
     unsigned long long n0 = 0, nall = 0;
+    unsigned int nintra = 0, cases = 0;
     for (int e = rowptr[v]; e < rowptr[v + 1]; ++e) {
         const int u = col[e];
         const int j = u / K, c2 = u % K;
         const unsigned long long bits = (unsigned long long)__double_as_longlong(val[e]);
         if (i == j) {
             if (pass == 0 && bits != (unsigned long long)__double_as_longlong(P)) atomicOr(flag, 8);
+            ++nintra;
+            cases |= 1u << c2;
             continue;
         }
         if (c != c2) {
@@ -325,19 +339,24 @@ __global__ void k_dense_scatter(int32_t n, int32_t K, int32_t ncp, const int32_t
             continue;
         }
         ++nall;
-        unsigned long long *cellp = W + (size_t)i * ncp + j;
+        const size_t cell = (size_t)i * ncp + j;
         if (pass == 0) {
+            // seen: one byte per (i, j), bit c = case c (K <= 8)
+            const unsigned int bit = 1u << ((cell & 3) * 8 + c);
+            if (atomicOr(seen + (cell >> 2), bit) & bit) atomicOr(flag, 4);
             if (c == 0) {
                 ++n0;
-                if (atomicCAS(cellp, DN_EMPTY, bits) != DN_EMPTY) atomicOr(flag, 4);
+                W[cell] = bits;      // two writers only for a duplicate, which is flagged
             }
         } else if (c != 0) {
-            if (*cellp != bits) atomicOr(flag, 2);
+            if (W[cell] != bits) atomicOr(flag, 2);
         }
     }
     if (pass == 0) {
+        if (nintra != 0 && (nintra != (unsigned)(K - 1) || cases != (((1u << K) - 1) & ~(1u << c)))) atomicOr(flag, 16);
         atomicAdd(counts, n0);
         atomicAdd(counts + 1, nall);
+        atomicAdd(counts + 2, (unsigned long long)nintra);
     }
 }
 
