@@ -134,6 +134,10 @@ int qa_model_set_group_bounds(qa_model *model, const int64_t *lo, const int64_t 
  * mma.sync f64; energies to 1e-12 relative of neal's order) --, 0 when it does not (nothing changes).  K in {1, 2, 4, 8};
  * K = 1 is a general dense Ising model. */
 int qa_model_enable_dense(qa_model *model, int32_t cases_per_cell);
+/* Replay kernel's coupling slabs, as the last sampling call on the replay kernel built them: the number of blocks that carry
+ * a k-way section (one-hot cells of K cases annealed in lockstep; 0: none, or the slabs are not built yet) and their K.
+ * QA_REPLAY_KWAY=0 in the environment when the context is created keeps every block in the generic form. */
+int64_t qa_model_replay_kway(const qa_model *model, int32_t *k_out);
 int qa_model_num_variables(const qa_model *model);
 int64_t qa_model_num_couplers(const qa_model *model);
 int qa_model_max_degree(const qa_model *model);

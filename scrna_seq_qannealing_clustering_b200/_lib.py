@@ -91,6 +91,7 @@ SIGNATURES = {
     "qa_model_set_groups": (C.c_int, [_p, _i32, _p, _p, _p, _p]),
     "qa_model_set_group_bounds": (C.c_int, [_p, _p, _p]),
     "qa_model_enable_dense": (C.c_int, [_p, _i32]),
+    "qa_model_replay_kway": (_i64, [_p, _p]),
     "qa_model_num_variables": (C.c_int, [_p]),
     "qa_model_num_couplers": (_i64, [_p]),
     "qa_model_max_degree": (C.c_int, [_p]),

@@ -19,10 +19,67 @@ namespace qa {
 // rows, then the seq parts of all rows.  Built once per model on the host from the device-built CSR (a setup step,
 // O(entries)).  Models whose blocks would hold fewer than 4 variables on average (dense rows, or sparse rows scattered over
 // many half-words) leave rp_ok false and run on the other kernels.
+//
+// K-way section.  One-hot k-way models (models.cqm_model, dqm_model: variable v = cell * K + case) have cells of K aligned
+// consecutive variables whose rows share one neighbour-cell list.  A cell CONFORMS when every row (i, p) has exactly the
+// other K - 1 cases of its own cell as intra-cell neighbours, each once, and otherwise only neighbours (j, p) of its own case,
+// each cell j once, with the same set of cells j and bitwise the same J_ij in all K rows.  Then row (i, p)'s pre part is
+//     (i, p') for p' > p  |  (j, p) for j > i ascending  |  (j, p) for j < v0 / K ascending
+// and the last two lists are the same for all K rows.  A block of whole conforming cells gets, behind its seq region, a
+// section with one RpEntry per (cell, neighbour cell) in that order (J, slot, j*K << RP_J_SHIFT, and in bits 0-4 the shift of
+// case K - 1; case p shifts 2 (K - 1 - p) more), counted against RP_CAP.  The batch phase then runs the K rows of a cell in
+// lockstep (replay.cuh: rp_kway_batch): one entry and one slot word per neighbour cell for K independent fp64 chains.  The
+// generic entries stay complete, so every other pass, and the intra-cell part of the batch phase, reads them as before.
+// rowptr / col / val of one problem (rows local); fills conf[cell] and returns the number of variables in conforming cells.
+static int64_t kway_conforming(int n, const int32_t *rowptr, const int32_t *col, const double *val, int K, std::vector<char> &conf) {
+    const int ncell = n / K;
+    conf.assign(ncell, 0);
+    int64_t nvar = 0;
+    std::vector<std::pair<int32_t, double>> first, cur;
+    for (int i = 0; i < ncell; ++i) {
+        const int b = i * K;
+        bool ok = true;
+        for (int p = 0; p < K && ok; ++p) {
+            const int v = b + p;
+            uint32_t intra = 0u;
+            cur.clear();
+            for (int64_t e = rowptr[v]; e < rowptr[v + 1] && ok; ++e) {
+                const int j = col[e];
+                if (j >= b && j < b + K) {
+                    const uint32_t bit = 1u << (j - b);
+                    ok = j != v && (intra & bit) == 0u;
+                    intra |= bit;
+                } else {
+                    ok = j % K == p;
+                    cur.push_back({j / K, val[e]});
+                }
+            }
+            ok = ok && intra == (((1u << K) - 1u) & ~(1u << p));
+            if (!ok) break;
+            std::sort(cur.begin(), cur.end(), [](const std::pair<int32_t, double> &a, const std::pair<int32_t, double> &c) {
+                return a.first < c.first;
+            });
+            for (size_t k = 1; k < cur.size() && ok; ++k) ok = cur[k].first != cur[k - 1].first;
+            if (p == 0) {
+                first = cur;
+            } else {
+                ok = ok && cur.size() == first.size();
+                for (size_t k = 0; k < cur.size() && ok; ++k)
+                    ok = cur[k].first == first[k].first && memcmp(&cur[k].second, &first[k].second, sizeof(double)) == 0;
+            }
+        }
+        if (ok) {
+            conf[i] = 1;
+            nvar += K;
+        }
+    }
+    return nvar;
+}
+
 // Pure host part of the slab construction (no CUDA calls: the CPU test-suite drives it through qa_debug_pack_slabs).
 // rowptr holds global entry positions per global row (problem p's rows start at var_off[p]), col local neighbour indices.
 bool pack_replay_slabs(int P, const int64_t *var_off, const int32_t *rowptr, const int32_t *col, const double *val, int ngroups,
-                       const std::vector<int32_t> &hg, const std::vector<int32_t> &hc, int slots, RpPacked &out) {
+                       const std::vector<int32_t> &hg, const std::vector<int32_t> &hc, int slots, RpPacked &out, bool kway) {
     const int RP_MAXBW = slots - 1;   // foreign half-words per block
     std::vector<uint32_t> &off = out.off;
     std::vector<unsigned char> &slabs = out.slabs;
@@ -32,16 +89,33 @@ bool pack_replay_slabs(int P, const int64_t *var_off, const int32_t *rowptr, con
     slabs.clear();
     out.uniform = true;
     out.adj_sorted = true;
+    out.kway_k = 0;
+    out.kway_blocks = 0;
     struct Nb { int32_t j; double J; };
     struct Row { std::vector<Nb> later, early, seq; };   // u > v | u < v0 | v0 <= u < v
     std::vector<int32_t> stamp, slot_of;
     std::vector<Row> rows(RP_D);
     std::vector<size_t> hdr_pos;
     std::vector<int32_t> row_words;
+    std::vector<char> conf, conf_k;
     for (int p = 0; p < P; ++p) {
         const int64_t v_off = var_off[p];
         const int n = (int)(var_off[p + 1] - v_off);
         if (n == 0 || n > RP_MAX_VARS) return false;   // the entry word holds a 20-bit neighbour index
+        // the cell size under which the most variables conform (ties: the larger K, more independent chains)
+        int K = 0;
+        conf.clear();
+        if (kway) {
+            int64_t best = 0;
+            for (int k : {2, 4, 8, 16}) {
+                const int64_t c = kway_conforming(n, rowptr + v_off, col, val, k, conf_k);
+                if (c > 0 && c >= best) {
+                    best = c;
+                    K = k;
+                    conf.swap(conf_k);
+                }
+            }
+        }
         const int nhw = (n + 15) / 16;
         const int npad = nhw * 16;
         out.blk_base[p] = (int64_t)off.size();
@@ -133,6 +207,33 @@ bool pack_replay_slabs(int P, const int64_t *var_off, const int32_t *rowptr, con
             H.seq_off = (int32_t)E.size();
             for (int i = 0; i < nv; ++i)
                 for (const Nb &nb : rows[i].seq) emit(nb);
+            // k-way section: whole conforming cells only
+            bool kw = K > 0 && v0 % K == 0 && nv % K == 0 && v0 + nv <= n;
+            for (int c = v0 / K; kw && c < (v0 + nv) / K; ++c) kw = conf[c] != 0;
+            if (kw) {
+                const size_t gen = E.size();
+                const int c0 = v0 / K;
+                for (int c = c0; c < (v0 + nv) / K; ++c) {
+                    const Row &R = rows[(c - c0) * K];   // case 0: its later / early lists hold the neighbour cells in order
+                    for (int part = 0; part < 2; ++part)
+                        for (const Nb &nb : (part == 0 ? R.later : R.early)) {
+                            if (nb.j >= c * K && nb.j < (c + 1) * K) continue;   // intra-cell
+                            const int wj = nb.j >> 4;
+                            RpEntry en;
+                            en.J = nb.J;
+                            en.zero = 0u;
+                            en.B = (uint32_t)(30 - 2 * ((nb.j + K - 1) & 15)) | ((uint32_t)(wj == own ? 0 : slot_of[wj]) << 7) |
+                                   ((uint32_t)nb.j << RP_J_SHIFT);
+                            E.push_back(en);
+                        }
+                }
+                if (E.size() <= (size_t)RP_CAP) {
+                    H.kway = (int32_t)((uint32_t)gen | ((uint32_t)K << 16));
+                    out.kway_blocks++;
+                } else {
+                    E.resize(gen);   // the section does not fit the stage: generic block
+                }
+            }
             H.nent = (int32_t)E.size();
             H.nbw = nbw;
             H.v0 = v0;
@@ -148,6 +249,7 @@ bool pack_replay_slabs(int P, const int64_t *var_off, const int32_t *rowptr, con
             v0 += nv;
         }
         out.nslabs[p] = b;
+        if (K > 0) out.kway_k = K;
         if ((int64_t)b * 4 > (int64_t)npad) return false;   // fewer than 4 variables per block on average: replaying does not pay
         // every slab also carries the half-word list of the next block (cyclic), staged while this block decides, and the slot
         // that holds the PREVIOUS block's half-word (the one word that staging cannot have up to date)
@@ -195,12 +297,15 @@ int build_replay_tables(qa_model *M) {
     }
     RpPacked pk;
     // 32 half-word slots per warp when the blocks fit (4 KB per warp), else 64 (scattered neighbourhoods)
+    const bool kw = ctx->replay_kway != 0;
     M->rp_slots = 32;
-    if (!pack_replay_slabs(M->num_problems, M->var_off.data(), rowptr.data(), col.data(), val.data(), M->ngroups, hg, hc, 32, pk)) {
+    if (!pack_replay_slabs(M->num_problems, M->var_off.data(), rowptr.data(), col.data(), val.data(), M->ngroups, hg, hc, 32, pk, kw)) {
         M->rp_slots = 64;
-        if (!pack_replay_slabs(M->num_problems, M->var_off.data(), rowptr.data(), col.data(), val.data(), M->ngroups, hg, hc, 64, pk))
+        if (!pack_replay_slabs(M->num_problems, M->var_off.data(), rowptr.data(), col.data(), val.data(), M->ngroups, hg, hc, 64, pk, kw))
             return QA_OK;   // the model does not fit the slab format: rp_ok stays false
     }
+    M->rp_kway_k = pk.kway_blocks > 0 ? pk.kway_k : 0;
+    M->rp_kway_blocks = pk.kway_blocks;
     const std::vector<uint32_t> &off = pk.off;
     const std::vector<unsigned char> &slabs = pk.slabs;
     const std::vector<int64_t> &blk_base = pk.blk_base;
@@ -257,15 +362,16 @@ int launch_replay(Launch &L) {
     const int64_t gpp = (tpp + nw - 1) / nw;
     const int64_t total_items = (int64_t)P * gpp;
     size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl);
+    // models with k-way blocks run the instance with the k-way batch phase; all others the generic one
+#define QA_RP_FN(G, S) (M->rp_kway_blocks > 0 ? (const void *)k_anneal_replay<G, S, true> : (const void *)k_anneal_replay<G, S, false>)
     const void *fn = nullptr;
     if (groups && L.interval)
-        fn = M->rp_slots == 32 ? (const void *)k_anneal_replay<3, 32> : (const void *)k_anneal_replay<3, 64>;
+        fn = M->rp_slots == 32 ? QA_RP_FN(3, 32) : QA_RP_FN(3, 64);
     else if (M->rp_slots == 32)
-        fn = !groups ? (const void *)k_anneal_replay<0, 32>
-                     : (M->groups_i32 ? (const void *)k_anneal_replay<1, 32> : (const void *)k_anneal_replay<2, 32>);
+        fn = !groups ? QA_RP_FN(0, 32) : (M->groups_i32 ? QA_RP_FN(1, 32) : QA_RP_FN(2, 32));
     else
-        fn = !groups ? (const void *)k_anneal_replay<0, 64>
-                     : (M->groups_i32 ? (const void *)k_anneal_replay<1, 64> : (const void *)k_anneal_replay<2, 64>);
+        fn = !groups ? QA_RP_FN(0, 64) : (M->groups_i32 ? QA_RP_FN(1, 64) : QA_RP_FN(2, 64));
+#undef QA_RP_FN
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, nw * 32, smem, cudaOccupancyDefault));

@@ -143,7 +143,7 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
     QA_CUDA(cudaMemcpyAsync(hs, ctx->d_stats, sizeof(hs), cudaMemcpyDeviceToHost, ctx->stream));
     QA_CUDA(cudaStreamSynchronize(ctx->stream));
 #ifdef QA_RP_PROFILE
-    fprintf(stderr, "[qa profile] cycles summed over warps: setup %llu slab-wait %llu stage-wait %llu prologue %llu entries %llu decide %llu pass %llu push-flip %llu\n",
+    fprintf(stderr, "[qa profile] cycles summed over warps: setup %llu slab-wait %llu stage-wait %llu prologue %llu batch %llu sequential %llu replay-passes %llu push-passes %llu\n",
             hs[QA_NSTAT + 1], hs[QA_NSTAT + 2], hs[QA_NSTAT + 3], hs[QA_NSTAT + 4], hs[QA_NSTAT + 5], hs[QA_NSTAT + 6], hs[QA_NSTAT + 7], hs[QA_NSTAT + 8]);
 #endif
     if (flag == QA_ERR_SMEM_BASE) return fail(QA_ERR_CUDA, "replay kernel: dynamic shared memory does not start where the layout assumed");
@@ -282,6 +282,7 @@ int qa_ctx_create(int device_id, qa_ctx **out) {
     ctx->num_sms = prop.multiProcessorCount;
     if (const char *e = getenv("QA_REPLAY_SWITCH_PERMILLE")) ctx->replay_switch_permille = atoi(e);  // development knobs
     if (const char *e = getenv("QA_REPLAY_WARPS")) ctx->replay_warps = atoi(e);
+    if (const char *e = getenv("QA_REPLAY_KWAY")) ctx->replay_kway = atoi(e);
     QA_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     for (auto &ev : ctx->ev) QA_CUDA(cudaEventCreate(&ev));
     QA_CUDA(cudaMalloc((void **)&ctx->d_stats, (QA_NSTAT + 1 + QA_NDEBUG) * sizeof(unsigned long long)));

@@ -158,6 +158,7 @@ struct qa_ctx {
     int kernel = 0;  // QA_KERNEL_*
     int replay_switch_permille = 20;  // replay -> push hand-over threshold (QA_REPLAY_SWITCH_PERMILLE overrides)
     int replay_warps = 0;             // warps per CTA of the replay kernel (0: automatic; QA_REPLAY_WARPS overrides)
+    int replay_kway = 1;              // k-way sections in the replay slabs (QA_REPLAY_KWAY=0: generic blocks only)
     int last_kernel = 0;              // QA_KERNEL_* the last sampling call ran on
     unsigned rp_smem_base = 1024;     // shared-window offset of dynamic shared memory (verified by the replay kernel)
     bool rp_base_checked = false;
@@ -203,6 +204,8 @@ struct qa_model {
     bool rp_uniform = false;   // every block holds exactly RP_D variables
     int rp_slots = 32;         // half-word slots per warp the slabs were packed for (32 or 64)
     bool rp_adj_sorted = false; // adjacency lists ascending: field set-up through the slab ring
+    int32_t rp_kway_k = 0;      // cell size of the k-way blocks (0: none)
+    int64_t rp_kway_blocks = 0; // slabs with a k-way section
     bool groups_i32 = false;   // every group term a*(a - s*(M+kappa)) fits 32-bit integers
     // dense k-way form (dense.cuh): W and P derived from the CSR by qa_model_enable_dense
     double *dn_W = nullptr;
@@ -335,8 +338,11 @@ struct RpPacked {
     std::vector<int32_t> nslabs;
     bool uniform = true;                // every block holds exactly RP_D variables
     bool adj_sorted = true;             // every adjacency list is ascending (dimod's vector order): slab order serves the set-up
+    int32_t kway_k = 0;                 // cell size of the k-way sections (anneal_replay.cu), 0: none
+    int64_t kway_blocks = 0;            // blocks that carry a k-way section
 };
+// kway = false: no k-way sections (every block in the generic form)
 bool pack_replay_slabs(int P, const int64_t *var_off, const int32_t *rowptr, const int32_t *col, const double *val, int ngroups,
-                       const std::vector<int32_t> &hg, const std::vector<int32_t> &hc, int slots, RpPacked &out);
+                       const std::vector<int32_t> &hg, const std::vector<int32_t> &hc, int slots, RpPacked &out, bool kway = true);
 
 }  // namespace qa

@@ -420,6 +420,13 @@ int qa_argmin_device(qa_ctx *ctx, int64_t count, const double *values, int64_t i
     return QA_OK;
 }
 
+int64_t qa_model_replay_kway(const qa_model *M, int32_t *k_out) {
+    if (!M) return fail(QA_ERR_ARG, "null model");
+    const bool on = M->rp_ok && M->rp_kway_blocks > 0;
+    if (k_out) *k_out = on ? M->rp_kway_k : 0;
+    return on ? M->rp_kway_blocks : 0;
+}
+
 /* Test hook, host only (no device needed): pack the replay kernel's coupling slabs for one problem whose CSR (adjacency order,
  * rowptr[n + 1], col, val) is in host memory.  Returns 1 when the model fits the slab format (0: it does not, negative: error);
  * on success *nslabs_out / *bytes_out / *uniform_out are set and, when the buffers are given (bytes_out reports the size to
@@ -440,8 +447,10 @@ int qa_debug_pack_slabs(int32_t n, const int32_t *rowptr, const int32_t *col, co
     }
     const int64_t var_off[2] = {0, n};
     RpPacked pk;
-    if (!pack_replay_slabs(1, var_off, rp.data(), col, val, ngroups, hg, hc, 32, pk) &&
-        !pack_replay_slabs(1, var_off, rp.data(), col, val, ngroups, hg, hc, 64, pk)) return 0;
+    const char *kw_env = getenv("QA_REPLAY_KWAY");   // as qa_ctx_create reads it
+    const bool kw = !(kw_env && atoi(kw_env) == 0);
+    if (!pack_replay_slabs(1, var_off, rp.data(), col, val, ngroups, hg, hc, 32, pk, kw) &&
+        !pack_replay_slabs(1, var_off, rp.data(), col, val, ngroups, hg, hc, 64, pk, kw)) return 0;
     *nslabs_out = pk.nslabs[0];
     *bytes_out = (int64_t)pk.slabs.size();
     *uniform_out = pk.uniform ? 1 : 0;

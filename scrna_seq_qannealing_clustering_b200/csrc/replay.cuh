@@ -62,6 +62,16 @@ constexpr int RP_SLOTS = 64;                  // half-word slots per warp, at mo
 #define RP_DIST 2     // slabs are requested this many blocks ahead of the first warp that will need them (< RP_STAGES)
 #endif
 static_assert(RP_DIST < RP_STAGES, "the ring must hold the block in use and the requested ones");
+// Development build (-DQA_RP_PROFILE): clock64() cycles summed per warp into the QA_NDEBUG counters behind the read counter,
+// printed by the host after every sampling call.  Slots: 0 set-up pass, 1 slab wait, 2 stage wait, 3 prologue (block start
+// to batch phase, waits excluded), 4 batch phase, 5 sequential phase, 6 replay passes, 7 catch-up and push passes.
+#ifdef QA_RP_PROFILE
+#define RP_CLK(t) const long long t = clock64()
+#define RP_PROF(k, d) (c.prof[k] += (d))
+#else
+#define RP_CLK(t)
+#define RP_PROF(k, d)
+#endif
 constexpr int RP_PS_BYTES = RP_D * 32 * 8;       // per warp: partial sums [row][lane] (push phase: the block's fields)
 __host__ __device__ constexpr int rp_sf_bytes(int slots) { return slots * 32 * 4; }   // per warp: [slot][lane] words, aligned to its size
 __host__ __device__ constexpr uint32_t rp_slot_mask(int slots) { return (uint32_t)(slots - 1) << 7; }
@@ -73,14 +83,14 @@ __host__ __device__ constexpr uint32_t rp_slot_mask(int slots) { return (uint32_
 #endif
 
 struct alignas(16) RpHdr {
-    int32_t nent;               // entry slots in this slab (pre region incl. padding, then seq region)
+    int32_t nent;               // entry slots in this slab (pre region incl. padding, seq region, k-way section)
     int32_t nbw;                // distinct neighbour half-words other than the block's own
     int32_t v0;                 // first variable of the block
     int32_t nv;                 // variables in the block (1 .. RP_D; v0 .. v0+nv-1 lie in one 16-variable half-word)
     int32_t prev_slot;          // slot holding the PREVIOUS block's half-word (0: not referenced / same half-word / first block)
     int32_t seq_off;            // entry slot where the seq region starts (multiple of 4)
     int32_t nbw_next;           // the half-word list of the NEXT block (cyclic): staged while this block decides
-    int32_t pad_;
+    int32_t kway;               // k-way section (anneal_replay.cu): entry slot where it starts (bits 0-15) | K << 16; 0: none
     uint32_t rowa[RP_D];        // pre rounds (bits 0-7) | seq entries (8-15) | degree (16-31)
     uint32_t rowb[RP_D];        // later entries u > v (0-15) | pre entries without padding (16-31)
     int32_t ga[RP_D];           // group (low byte, 255: none) | coefficient << 8
@@ -89,7 +99,7 @@ struct alignas(16) RpHdr {
 };
 static_assert(sizeof(RpHdr) % 16 == 0, "slab header layout");
 constexpr uint32_t RP_H_NBW = offsetof(RpHdr, nbw), RP_H_V0 = offsetof(RpHdr, v0), RP_H_NV = offsetof(RpHdr, nv),
-                   RP_H_PREV = offsetof(RpHdr, prev_slot), RP_H_SEQ = offsetof(RpHdr, seq_off),
+                   RP_H_PREV = offsetof(RpHdr, prev_slot), RP_H_SEQ = offsetof(RpHdr, seq_off), RP_H_KW = offsetof(RpHdr, kway),
                    RP_H_ROWA = offsetof(RpHdr, rowa), RP_H_ROWB = offsetof(RpHdr, rowb), RP_H_GA = offsetof(RpHdr, ga),
                    RP_H_BW = offsetof(RpHdr, bw), RP_H_NBWN = offsetof(RpHdr, nbw_next), RP_H_BWN = offsetof(RpHdr, bw_next);
 struct __align__(16) RpEntry {
@@ -170,6 +180,97 @@ __device__ __forceinline__ void rp_add_entry(double &f, const int4 &q, uint32_t 
     f = fma(__hiloint2double(q.y, q.x), __hiloint2double((int)(x & 0xC0000000u), q.z), f);   // q.z == 0
 }
 
+// Batch phase of a block with a k-way section (anneal_replay.cu): whole cells of K one-hot cases whose rows share one
+// neighbour-cell list.  The rows of a cell run in lockstep in chunks of KR = min(K, 8) rows (two chunks per cell for K = 16),
+// one accumulator per row: first each row's intra-cell later cases (its first entries in the generic pre region, read against
+// the register W, which holds the block's own half-word), then the section's neighbour cells: per neighbour cell one entry and
+// one slot word, loaded a step ahead, and per row SHF, LOP3, DFMA into its own chain.  Row p of a chunk adds the same terms in
+// the same order as its generic pre part, with no padding entries: the partial sums are bit-identical.  The fields of the next
+// chunk are copied (cp.async) into its partial-sum rows while this one runs; those of the first rows come from the block
+// look-ahead fq.  Returns the chg mask (partial sum != field), as the generic batch phase does.
+template <int KR, int SLOTS>
+__device__ __forceinline__ uint32_t rp_kway_batch(uint32_t hdr, uint32_t ent, uint32_t kw, int nv, const double *fB,
+                                                  const double (&fq)[RP_LA], uint32_t W, uint32_t sfb, uint32_t psb) {
+    const int K = (int)(kw >> 16);
+    uint32_t sec = ent + (kw & 0xffffu) * 16u;   // the current cell's neighbour-cell entries
+    uint32_t a = ent;                            // the current row's generic pre part
+    uint32_t chg = 0u;
+    const uint32_t lane = threadIdx.x & 31u;
+    // the warp's copy of row r (256 B): lanes 16 h .. 16 h + 15 copy 16 B each of row r + h
+    const uint32_t cp_dst = psb - 8u * lane + (lane >> 4) * 256u + (lane & 15u) * 16u;
+    const double *const cp_src = fB - lane + (lane >> 4) * 32 + (lane & 15u) * 2;
+    double acc[KR];
+#pragma unroll
+    for (int k = 0; k < KR; ++k) acc[k] = k < RP_LA ? fq[k] : __ldcg(fB + k * 32);
+#pragma unroll
+    for (int k = 0; k < KR; ++k) sts_f64(psb + (uint32_t)k * 256u, acc[k]);   // the fields, for the chg test
+#pragma unroll 1
+    for (int r0 = 0; r0 < nv; r0 += KR) {
+        if (r0 > 0) {   // this chunk's fields, copied into its partial-sum rows while the previous chunk ran
+            rp_cp_async_wait_all();
+            __syncwarp();
+#pragma unroll
+            for (int k = 0; k < KR; ++k) acc[k] = lds_f64(psb + (uint32_t)(r0 + k) * 256u);
+        }
+        if (r0 + KR < nv) {   // the next chunk's fields -> its partial-sum rows (no register staging)
+#pragma unroll
+            for (int k = 0; k < KR; k += 2) rp_cp_async16(cp_dst + (uint32_t)(r0 + KR + k) * 256u, cp_src + (r0 + KR + k) * 32);
+        }
+        // intra-cell later cases: row k of the chunk has xs + KR - 1 - k of them (xs = 8 for the first chunk of a 16-way cell)
+        const int xs = K - KR - r0 % K;
+        uint32_t ar[KR];
+#pragma unroll
+        for (int k = 0; k < KR; ++k) {
+            ar[k] = a;
+            a += (lds_u32(hdr + RP_H_ROWA + 4u * (uint32_t)(r0 + k)) & 255u) * 64u;
+        }
+#pragma unroll 1
+        for (int m = 0; m < xs; ++m) {
+#pragma unroll
+            for (int k = 0; k < KR; ++k) rp_add_entry(acc[k], lds_v4(ar[k] + 16u * (uint32_t)m), W);
+        }
+#pragma unroll
+        for (int m = 0; m < KR - 1; ++m) {
+#pragma unroll
+            for (int k = 0; k < KR - 1 - m; ++k) rp_add_entry(acc[k], lds_v4(ar[k] + 16u * (uint32_t)(xs + m)), W);
+        }
+        // neighbour cells: j > i ascending, then j < v0 / K ascending; the count is the pre part of the cell's last case
+        const int cl = r0 - r0 % K + K - 1;
+        const int nn = (int)(lds_u32(hdr + RP_H_ROWB + 4u * (uint32_t)cl) >> 16);
+        const uint32_t xsh = 2u * (uint32_t)xs;
+        auto step = [&](const int4 &q, uint32_t w) {
+            const uint32_t x = (w << ((uint32_t)q.w & 31u)) << xsh;   // case KR - 1 of the chunk at bits (31, 30)
+            const double J = __hiloint2double(q.y, q.x);
+#pragma unroll
+            for (int k = 0; k < KR; ++k)
+                acc[k] = fma(J, __hiloint2double((int)((x << (2 * (KR - 1 - k))) & 0xC0000000u), q.z), acc[k]);   // q.z == 0
+        };
+        uint32_t e = sec;
+        int4 qa = lds_v4(e);
+        uint32_t wa = lds_vu32(((uint32_t)qa.w & rp_slot_mask(SLOTS)) | sfb);
+        int t = 0;
+#pragma unroll 1
+        for (; t + 2 <= nn; t += 2) {   // reads up to two entries past the section: inside the stage's read-ahead slack
+            const int4 qb = lds_v4(e + 16u);
+            const uint32_t wb = lds_vu32(((uint32_t)qb.w & rp_slot_mask(SLOTS)) | sfb);
+            step(qa, wa);
+            qa = lds_v4(e + 32u);
+            wa = lds_vu32(((uint32_t)qa.w & rp_slot_mask(SLOTS)) | sfb);
+            step(qb, wb);
+            e += 32u;
+        }
+        if (t < nn) step(qa, wa);
+        if ((r0 + KR) % K == 0) sec += (uint32_t)nn * 16u;   // the cell is complete
+#pragma unroll
+        for (int k = 0; k < KR; ++k) {
+            const uint32_t pa = psb + (uint32_t)(r0 + k) * 256u;
+            if (acc[k] != lds_f64(pa)) chg |= 1u << (r0 + k);
+            sts_f64(pa, acc[k]);
+        }
+    }
+    return chg;
+}
+
 struct RpCtx {
     // ring (CTA-shared)
     uint32_t full_s, empty_s, stage_s;   // shared addresses: full[0], empty[0] (8 B apart), stage 0
@@ -191,6 +292,9 @@ struct RpCtx {
     LaneStats st;
     bool active;
     int n, nblk, npad;
+#ifdef QA_RP_PROFILE
+    long long prof[QA_NDEBUG];
+#endif
 };
 
 // lane 0 of any warp: request every slab up to running index `tgt` that nobody has requested yet and whose ring stage is
@@ -244,8 +348,9 @@ __device__ __forceinline__ void rp_stage_wait() {
 // MODE 2: push sweep (neal's eager form).  MODE 3: field set-up f[v] = h_v + sum_j J_vj s_j in neal's get_flip_energy order,
 // for models whose adjacency lists are ascending (then adjacency order = pre entries u < v0, seq entries, later entries).
 // GROUPS: 0 none, 1 rank-1 groups with 32-bit exact integer arithmetic (host-checked ranges), 2 with 64-bit, 3 interval groups
-// (64-bit; c.kap then holds {kappa, lo, hi} per group).
-template <int MODE, int GROUPS, int SLOTS>
+// (64-bit; c.kap then holds {kappa, lo, hi} per group).  KWAY: the slabs carry k-way sections (rp_kway_batch); false compiles
+// the replay sweep without the section test, so models without k-way blocks run exactly the generic kernel.
+template <int MODE, int GROUPS, int SLOTS, bool KWAY = false>
 __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
     const int lane = threadIdx.x & 31;
     const double thr = 44.36142 / beta;
@@ -266,6 +371,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
 
     const uint32_t g_last = c.gb + (uint32_t)nblk - 1u;   // running index of the last block of this pass
     for (int blk = 0; blk < nblk; ++blk) {
+        RP_CLK(t_top);
         const uint32_t stage = c.gb % RP_STAGES, phase = (c.gb / RP_STAGES) & 1u;
         if (lane == 0) {
             uint32_t tgt = c.gb + (uint32_t)RP_DIST;
@@ -273,9 +379,14 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
             rp_request(c, tgt, blk);
         }
         __syncwarp();
+        RP_CLK(t_sw);
         while (!mbar_try_wait(c.full_s + 8u * stage, phase)) {   // usually there; else make sure somebody has asked for it
             if (lane == 0) rp_request(c, c.gb, blk);
         }
+#ifdef QA_RP_PROFILE
+        long long t_wait = clock64() - t_sw;
+        RP_PROF(1, t_wait);
+#endif
         const uint32_t hdr = c.stage_s + stage * (uint32_t)RP_STAGE_BYTES;   // shared address of the slab
         const uint32_t ent = hdr + (uint32_t)sizeof(RpHdr);
         const int v0 = (int)lds_u32(hdr + RP_H_V0);
@@ -298,7 +409,12 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
         if (MODE != 2) {
             // the foreign half-words were requested while the previous block decided; the first block of a pass asks now
             if (blk == 0) rp_stage_issue(c, hdr + RP_H_BW, (int)lds_u32(hdr + RP_H_NBW));
+            RP_CLK(t_gw);
             rp_stage_wait();
+#ifdef QA_RP_PROFILE
+            RP_PROF(2, clock64() - t_gw);
+            t_wait += clock64() - t_gw;
+#endif
             const uint32_t ps = lds_u32(hdr + RP_H_PREV);
             if (blk != 0 && ps != 0u) sts_u32(sfb + ps * 128u, Wprev);   // the one word that copy could not have up to date
             sts_u32(sfb, W);
@@ -307,48 +423,58 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
         if (MODE == 0) {
             // ---- batch phase: pre parts of all rows; table entries are loaded one round ahead of their use (two buffers, rounds
             // in pairs: no register rotation); rows in groups of RP_LA so that the field look-ahead needs no rotation either
+            RP_CLK(t_batch);
+            RP_PROF(3, t_batch - t_top - t_wait);
             uint32_t a = ent;
             uint32_t chg = 0u;
+            const uint32_t kw = KWAY ? lds_u32(hdr + RP_H_KW) : 0u;
+            if (KWAY && kw != 0u) {
+                const int K = (int)(kw >> 16);
+                chg = K == 2 ? rp_kway_batch<2, SLOTS>(hdr, ent, kw, nv, fB, fq, W, sfb, psb)
+                    : K == 4 ? rp_kway_batch<4, SLOTS>(hdr, ent, kw, nv, fB, fq, W, sfb, psb)
+                             : rp_kway_batch<8, SLOTS>(hdr, ent, kw, nv, fB, fq, W, sfb, psb);
+            } else {
 #pragma unroll 1
-            for (int i0 = 0; i0 < nv; i0 += RP_LA) {
+                for (int i0 = 0; i0 < nv; i0 += RP_LA) {
 #pragma unroll
-                for (int kk = 0; kk < RP_LA; ++kk) {
-                    const int i = i0 + kk;
-                    if (i < nv) {
-                        double p = fq[kk];
-                        if (i + RP_LA < nv) fq[kk] = __ldcg(fB + (i + RP_LA) * 32);
-                        const double f0 = p;
-                        const int nr = (int)(lds_u32(hdr + RP_H_ROWA + 4u * (uint32_t)i) & 255u);
-                        int4 qa[4], qb[4];
-                        uint32_t w[4];
+                    for (int kk = 0; kk < RP_LA; ++kk) {
+                        const int i = i0 + kk;
+                        if (i < nv) {
+                            double p = fq[kk];
+                            if (i + RP_LA < nv) fq[kk] = __ldcg(fB + (i + RP_LA) * 32);
+                            const double f0 = p;
+                            const int nr = (int)(lds_u32(hdr + RP_H_ROWA + 4u * (uint32_t)i) & 255u);
+                            int4 qa[4], qb[4];
+                            uint32_t w[4];
 #pragma unroll
-                        for (int k = 0; k < 4; ++k) qa[k] = lds_v4(a + 16u * k);
-                        int r = 0;
+                            for (int k = 0; k < 4; ++k) qa[k] = lds_v4(a + 16u * k);
+                            int r = 0;
 #pragma unroll 1
-                        for (; r + 2 <= nr; r += 2) {
+                            for (; r + 2 <= nr; r += 2) {
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) qb[k] = lds_v4(a + 64u + 16u * k);
+                                for (int k = 0; k < 4; ++k) qb[k] = lds_v4(a + 64u + 16u * k);
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qa[k].w & rp_slot_mask(SLOTS)) | sfb);
+                                for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qa[k].w & rp_slot_mask(SLOTS)) | sfb);
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) rp_add_entry(p, qa[k], w[k]);
+                                for (int k = 0; k < 4; ++k) rp_add_entry(p, qa[k], w[k]);
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) qa[k] = lds_v4(a + 128u + 16u * k);
+                                for (int k = 0; k < 4; ++k) qa[k] = lds_v4(a + 128u + 16u * k);
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qb[k].w & rp_slot_mask(SLOTS)) | sfb);
+                                for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qb[k].w & rp_slot_mask(SLOTS)) | sfb);
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) rp_add_entry(p, qb[k], w[k]);
-                            a += 128u;
+                                for (int k = 0; k < 4; ++k) rp_add_entry(p, qb[k], w[k]);
+                                a += 128u;
+                            }
+                            if (r < nr) {
+#pragma unroll
+                                for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qa[k].w & rp_slot_mask(SLOTS)) | sfb);
+#pragma unroll
+                                for (int k = 0; k < 4; ++k) rp_add_entry(p, qa[k], w[k]);
+                                a += 64u;
+                            }
+                            sts_f64(psb + (uint32_t)i * 256u, p);
+                            if (p != f0) chg |= 1u << i;
                         }
-                        if (r < nr) {
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) w[k] = lds_vu32(((uint32_t)qa[k].w & rp_slot_mask(SLOTS)) | sfb);
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) rp_add_entry(p, qa[k], w[k]);
-                            a += 64u;
-                        }
-                        sts_f64(psb + (uint32_t)i * 256u, p);
-                        if (p != f0) chg |= 1u << i;
                     }
                 }
             }
@@ -360,6 +486,8 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 for (int k = 0; k < RP_LA; ++k) fq[k] = __ldcg(fN + k * 32);
             }
 
+            RP_CLK(t_seq);
+            RP_PROF(4, t_seq - t_batch);
             // ---- sequential phase: in-block earlier neighbours from the register, then neal's decision
             uint32_t as = ent + lds_u32(hdr + RP_H_SEQ) * 16u;
 #pragma unroll 1
@@ -417,6 +545,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                     }
                 }
             }
+            RP_PROF(5, clock64() - t_seq);
         } else if (MODE == 1) {
             // ---- catch-up: the pending later-neighbour updates (a prefix of every pre part), no decisions
             uint32_t a = ent;
@@ -616,7 +745,7 @@ __host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned
     return fixed + pad + (size_t)nw * (sf + RP_PS_BYTES);
 }
 
-template <int GROUPS, int SLOTS>
+template <int GROUPS, int SLOTS, bool KWAY>
 __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_replay(AnnealParams P) {
     constexpr uint32_t RP_SF_BYTES = (uint32_t)rp_sf_bytes(SLOTS);
     extern __shared__ __align__(16) unsigned char rp_raw[];
@@ -685,6 +814,9 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     c.lam = lam_sh;
     c.kap = kap_sh;
     c.st = {0, 0, 0, 0, 0};
+#ifdef QA_RP_PROFILE
+    for (int k = 0; k < QA_NDEBUG; ++k) c.prof[k] = 0;
+#endif
     const int64_t slot = (int64_t)blockIdx.x * NW + wib;
     c.fT = P.fT_scratch + slot * P.fT_stride + lane;
     c.SF = reinterpret_cast<uint32_t *>(P.sf_scratch) + slot * P.sf_stride + lane;
@@ -772,6 +904,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
         }
         // ---- local fields in neal's get_flip_energy order: through the slab ring when the adjacency lists are ascending,
         // else row by row from the CSR
+        RP_CLK(t_setup);
         if (P.rp_slab_init) {
             if (total_sweeps > 0) c.gb = rp_setup_pass<SLOTS>(c);
         } else {
@@ -782,6 +915,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
                 e0 = e1;
             }
         }
+        RP_PROF(0, clock64() - t_setup);
         // ---- the schedule: replay sweeps while flips are frequent, then one catch-up pass and push sweeps
         bool push = false;
         long long done = 0;
@@ -794,11 +928,14 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
                 if (blockIdx.x == 0 && threadIdx.x == 0)
                     printf("[qa sweep] %lld beta %.4g mode %s clock %lld\n", done, beta, push ? "push" : "replay", clock64());
 #endif
+                RP_CLK(t_pass);
                 if (push) {
                     rp_pass<2, GROUPS, SLOTS>(c, beta, more);
+                    RP_PROF(7, clock64() - t_pass);
                 } else {
                     const unsigned acc0 = c.st.acc;
-                    rp_pass<0, GROUPS, SLOTS>(c, beta, more);
+                    rp_pass<0, GROUPS, SLOTS, KWAY>(c, beta, more);
+                    RP_PROF(6, clock64() - t_pass);
                     if (more) {  // CTA-uniform hand-over decision
                         unsigned wacc = c.st.acc - acc0;
 #pragma unroll
@@ -809,7 +946,9 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
                         if (threadIdx.x == 0) acc_sh[acc_par ^ 1] = 0u;
                         acc_par ^= 1;
                         if (tot * 1000ull < (unsigned long long)P.switch_permille * (unsigned long long)n * (unsigned long long)cta_reads) {
+                            RP_CLK(t_cu);
                             rp_pass<1, 0, SLOTS>(c, beta, true);
+                            RP_PROF(7, clock64() - t_cu);
                             push = true;
                         }
                     }
@@ -859,5 +998,8 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
         atomicAdd(P.stats + ST_ACC, v[2]);
         atomicAdd(P.stats + ST_TIES, v[3]);
         atomicAdd(P.stats + ST_NBR, v[4]);
+#ifdef QA_RP_PROFILE
+        for (int k = 0; k < QA_NDEBUG; ++k) atomicAdd(P.stats + QA_NSTAT + 1 + k, (unsigned long long)c.prof[k]);
+#endif
     }
 }

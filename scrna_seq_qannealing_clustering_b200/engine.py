@@ -466,6 +466,13 @@ class IsingModel:
         return bool(check(_lib.load().qa_model_enable_dense(self._h, int(cases_per_cell))))
 
     @property
+    def replay_kway(self):
+        """(blocks with a k-way section, their K) of the replay kernel's slabs, (0, 0) before the first replay call."""
+        k = C.c_int32(0)
+        blocks = _lib.load().qa_model_replay_kway(self._h, C.byref(k))
+        return int(check(blocks)), int(k.value)
+
+    @property
     def max_degree(self) -> int:
         return check(_lib.load().qa_model_max_degree(self._h))
 
