@@ -242,7 +242,8 @@ int qa_graph_split(qa_ctx *ctx, int32_t n, int64_t m_edges, const int32_t *eu, c
 /* parent node of every node of child `problem` (problem < 0: all children back to back); host or device destination */
 int qa_graph_get_nodes(const qa_graph *graph, int32_t problem, int32_t *node_ids_out);
 /* single-problem models (rank-1 groups and their interval bounds included) -> one batched model for qa_sa_sample_model_batch;
- * the inputs stay valid and owned by the caller.  Batched models with groups run on the warp-per-read kernel. */
+ * the inputs stay valid and owned by the caller.  Batched models with groups run on the warp-per-read kernel; problems with
+ * and without groups, equality and interval groups, may be mixed in one batch. */
 int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa_model **out);
 /* qa_sa_sample_ising_batch on a resident batched model.  betas_per_problem = 0: beta_schedules is one schedule [num_betas] for
  * every problem; 1: [num_problems][num_betas], problem p anneals with its own schedule (what separate sampler calls with
@@ -254,7 +255,8 @@ int qa_sa_sample_model_batch(qa_ctx *ctx, qa_model *model, int32_t reads_per_pro
 /* ---- SampleSet post-processing on the device (what the reference does with a SampleSet after the call:
  * energy-sorted iteration and k-th best energies BQM_clustering.py:93-146, the 16 best samples plot_and_save.py:105-126,
  * one-hot decode of DQM / CQM samples plot_and_save.py:46-63).  Pointers may be host or device memory. ---- */
-/* order_out[r] = index of the r-th best read: ascending energy, ties in read order (stable) */
+/* order_out[r] = index of the r-th best read: ascending energy, ties in read order (stable); -0.0 and +0.0 tie; every NaN,
+ * whatever its sign and payload, comes after +inf, NaNs in read order -- numpy's argsort(energies, kind="stable") */
 int qa_sort_reads(qa_ctx *ctx, int32_t num_reads, const double *energies, int32_t *order_out);
 /* samples_out[r][0..n) = states[order[r]][0..n) for r < k: only the k best samples leave the device */
 int qa_gather_samples(qa_ctx *ctx, int32_t n, int32_t num_reads, const int8_t *states, int32_t k, const int32_t *order,
@@ -267,8 +269,10 @@ int qa_decode_onehot(qa_ctx *ctx, int32_t cells, int32_t K, int64_t stride, int3
 
 /* Duplicate aggregation (dimod SampleSet.aggregate(): identical samples merged, num_occurrences summed) on the device:
  * rows are hashed (2 x 64 bit), sorted by hash, neighbours compared byte for byte.  first_index_out[u] = the first read of
- * the u-th distinct sample, in order of first occurrence; count_out[u] = its number of occurrences (both sized num_reads).
- * Only 8 bytes per read leave the device. */
+ * the u-th distinct sample, in order of first occurrence; count_out[u] = its number of occurrences (both sized num_reads,
+ * host memory).  Only 8 bytes per read leave the device.  n = 0: one group (0, num_reads), states not read.  Exact unless
+ * two distinct rows share the 64-bit first hash and their reads interleave (about num_reads^2 / 2^65 per call): then one
+ * sample is reported as two groups. */
 int qa_aggregate_reads(qa_ctx *ctx, int32_t n, int32_t num_reads, const int8_t *states, int32_t *num_unique_out,
                        int32_t *first_index_out, int32_t *count_out);
 
@@ -283,10 +287,13 @@ int qa_dev_copy(qa_ctx *ctx, void *dst, const void *src, int64_t bytes);   /* an
 int qa_random_states(qa_ctx *ctx, uint64_t seed, int64_t first_read, int32_t num_reads, int32_t n, int8_t *states_out);
 
 /* Lowest value and its first index (SampleSet.first; the per-rank half of the multi-GPU best-sample gather, SURVEY 8e):
- * warp-shuffle min-reduction, ties to the lower index.  values: host or device pointer. */
+ * warp-shuffle min-reduction in the order of qa_sort_reads, so best_index == order_out[0]: a NaN loses to every number, ties
+ * (-0.0 == +0.0) go to the lower index, every value NaN gives (values[0], 0); the value is returned bit for bit.  count = 0:
+ * (+inf, -1).  values: host or device pointer. */
 int qa_argmin(qa_ctx *ctx, int64_t count, const double *values, double *best_value, int64_t *best_index);
 /* The same reduction with its result left on the device: out_device[0] = lowest value, out_device[1] = (double)(index_offset +
- * its first index) -- the 16-byte send buffer of the per-rank all_gather, filled without a host round trip. */
+ * its first index) -- the 16-byte send buffer of the per-rank all_gather, filled without a host round trip.  count >= 1, so
+ * the offset is always added to an index in [0, count). */
 int qa_argmin_device(qa_ctx *ctx, int64_t count, const double *values, int64_t index_offset, double *out_device);
 
 /* Test hook, host only (no device needed): the coupling slabs the replay kernel would get for a CSR in host memory

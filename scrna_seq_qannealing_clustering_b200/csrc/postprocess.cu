@@ -15,45 +15,57 @@ using namespace qa;
 
 namespace {
 
-// warp-shuffle min / argmin (lowest index wins ties, like a stable sort by energy -> SampleSet.first)
+// (x, i) comes before (e, j) in the order of qa_sort_reads: a NaN after every number, equal values (-0.0 == +0.0) and two
+// NaNs by index
+__device__ __forceinline__ bool argmin_before(double x, long long i, double e, long long j) {
+    const bool xn = x != x, en = e != e;
+    if (xn != en) return en;
+    return xn ? i < j : (x < e || (x == e && i < j));
+}
+
+// warp-shuffle min / argmin in the order of the sort (-> SampleSet.first).  A thread without values holds (NaN, INT64_MAX),
+// which every value passes, so for count >= 1 the result is a value of the input and its index; all NaN: (values[0], 0).
 __global__ void __launch_bounds__(1024) k_argmin(const double *energies, int64_t count, double *best_e, long long *best_i) {
     __shared__ double se[32];
     __shared__ long long si[32];
-    double e = INFINITY;
+    const double none = __longlong_as_double(0x7ff8000000000000ll);
+    double e = none;
     long long idx = 0x7fffffffffffffffll;
     for (int64_t i = threadIdx.x; i < count; i += blockDim.x) {
         const double x = energies[i];
-        if (x < e || (x == e && i < idx)) { e = x; idx = i; }
+        if (argmin_before(x, i, e, idx)) { e = x; idx = i; }
     }
     for (int off = 16; off > 0; off >>= 1) {
         const double oe = __shfl_xor_sync(FULL_MASK, e, off);
         const long long oi = __shfl_xor_sync(FULL_MASK, idx, off);
-        if (oe < e || (oe == e && oi < idx)) { e = oe; idx = oi; }
+        if (argmin_before(oe, oi, e, idx)) { e = oe; idx = oi; }
     }
     if ((threadIdx.x & 31) == 0) { se[threadIdx.x >> 5] = e; si[threadIdx.x >> 5] = idx; }
     __syncthreads();
     if (threadIdx.x < 32) {
         const int nw = (blockDim.x + 31) >> 5;
-        e = threadIdx.x < nw ? se[threadIdx.x] : INFINITY;
+        e = threadIdx.x < nw ? se[threadIdx.x] : none;
         idx = threadIdx.x < nw ? si[threadIdx.x] : 0x7fffffffffffffffll;
         for (int off = 16; off > 0; off >>= 1) {
             const double oe = __shfl_xor_sync(FULL_MASK, e, off);
             const long long oi = __shfl_xor_sync(FULL_MASK, idx, off);
-            if (oe < e || (oe == e && oi < idx)) { e = oe; idx = oi; }
+            if (argmin_before(oe, oi, e, idx)) { e = oe; idx = oi; }
         }
         if (threadIdx.x == 0) { *best_e = e; *best_i = idx; }
     }
 }
 
-// order-preserving map double -> uint64 (ascending); NaNs sort last
+// order-preserving map double -> uint64 (ascending): x + 0.0 turns -0.0 into +0.0, so the two tie; every NaN, whatever its
+// sign and payload, gets the largest key and so sorts after +inf (in read order: the radix sort is stable)
 __global__ void k_energy_keys(int32_t count, const double *e, unsigned long long *keys, int32_t *idx) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     idx[i] = i;
     if (!e) return;   // index ramp only
-    unsigned long long b = (unsigned long long)__double_as_longlong(e[i] + 0.0);   // -0.0 and +0.0 tie
+    const double x = e[i];
+    unsigned long long b = (unsigned long long)__double_as_longlong(x + 0.0);
     b = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-    keys[i] = b;
+    keys[i] = x != x ? ~0ull : b;
 }
 
 // samples_out[r] = states[order[r]] for r < k  (one block per output row, coalesced 16-byte copies when aligned)
@@ -156,7 +168,7 @@ __global__ void k_mark_heads(int32_t n, const int8_t *states, const unsigned lon
 // stage `bytes` of a caller buffer (host or device) on the device; returns the device pointer to use
 __global__ void k_argmin_pack(const double *best_e, const long long *best_i, long long offset, double *out) {
     out[0] = *best_e;
-    out[1] = (double)(*best_i + offset);   // read indices are < 2^53: exact
+    out[1] = (double)(*best_i + offset);   // k_argmin of count >= 1 values gives an index in [0, count); read indices are < 2^53: exact
 }
 
 int stage_in(qa_ctx *ctx, DevBuf &buf, const void *p, size_t bytes, const void **dev) {
@@ -331,10 +343,17 @@ int qa_aggregate_reads(qa_ctx *ctx, int32_t n, int32_t num_reads, const int8_t *
     if (!num_unique_out) return fail(QA_ERR_ARG, "null num_unique_out");
     *num_unique_out = 0;
     if (num_reads == 0) return QA_OK;
-    if (!states || !first_index_out || !count_out) return fail(QA_ERR_ARG, "null states / outputs");
+    if (!first_index_out || !count_out) return fail(QA_ERR_ARG, "null outputs");
+    if (n == 0) {   // every read is the empty sample: one group, nothing to read
+        first_index_out[0] = 0;
+        count_out[0] = num_reads;
+        *num_unique_out = 1;
+        return QA_OK;
+    }
+    if (!states) return fail(QA_ERR_ARG, "null states");
     QA_CUDA(cudaSetDevice(ctx->device));
     const void *d_states = nullptr;
-    int rc = stage_in(ctx, ctx->states, states, (size_t)num_reads * std::max(n, 1), &d_states);
+    int rc = stage_in(ctx, ctx->states, states, (size_t)num_reads * n, &d_states);
     if (rc) return rc;
     const size_t R = (size_t)num_reads;
     // scratch: h1, h1s, h2 (u64), idx, idxs, head (i32)
@@ -358,9 +377,9 @@ int qa_aggregate_reads(qa_ctx *ctx, int32_t n, int32_t num_reads, const int8_t *
     QA_CUDA(cudaMemcpyAsync(hidx.data(), idxs, R * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     QA_CUDA(cudaMemcpyAsync(hhead.data(), head, R * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     QA_CUDA(cudaStreamSynchronize(ctx->stream));
-    // groups are runs of the hash-sorted order (stable: inside a run reads ascend); two DIFFERENT samples with equal 128-bit
-    // hashes would split a run of a third one -- merge runs of the same representative by comparing against all run heads
-    // of the same h1 (the full-row compare above already separated them, so this only matters for interleaved collisions)
+    // groups are runs of the h1-sorted order (stable: inside a run reads ascend), split where k_mark_heads found a different
+    // row.  Exact unless two distinct rows share the 64-bit h1 and their reads interleave (A, B, A in read order): then A's
+    // reads form two groups.  No merge pass for that: the chance of an h1 collision is about R^2 / 2^65 per call.
     std::vector<std::pair<int32_t, int32_t>> groups;   // (first read index, count)
     for (size_t p = 0; p < R; ++p) {
         if (hhead[p]) groups.emplace_back(hidx[p], 1);

@@ -229,10 +229,8 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
         M->cpl_off[p + 1] = M->cpl_off[p] + models[p]->m_total;
         M->max_deg = std::max(M->max_deg, models[p]->max_deg);
         M->ngroups = std::max(M->ngroups, models[p]->ngroups);
-        if (models[p]->ngroups > 0) {
-            gpad += (int64_t)models[p]->descs[0].nch * 32;
-            gcount += models[p]->ngroups;
-        }
+        gpad += (int64_t)models[p]->descs[0].nch * 32;   // group-free problems too: see the group copy below
+        gcount += std::max(models[p]->ngroups, 0);
     }
     M->n_total = M->var_off[num_models];
     M->m_total = M->cpl_off[num_models];
@@ -282,10 +280,22 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
     int rc = finalize_descs(M);
     if (rc) return bail(rc);
     int64_t go = 0, gl = 0;
-    for (int p = 0; p < num_models; ++p) {
+    for (int p = 0; p < num_models && M->ngroups > 0; ++p) {
         const qa_model *S = models[p];
-        if (S->ngroups <= 0) continue;
         const int64_t npad = (int64_t)S->descs[0].nch * 32;
+        ProblemDesc &D = M->descs[p];
+        if (S->ngroups <= 0) {
+            // the group kernels read grp[v] of every problem of the batch: a group-free problem gets grp = -1 everywhere
+            // (ngroups stays 0, so lambda / kappa are never read)
+            k_fill_i32<<<blocks(npad), tpb, 0, ctx->stream>>>(npad, -1, M->grp + go);
+            CAT_CUDA(cudaGetLastError());
+            CAT_CUDA(cudaMemsetAsync(M->coef + go, 0, (size_t)npad * sizeof(int32_t), ctx->stream));
+            ctx->launches++;
+            D.grp = M->grp + go;
+            D.coef = M->coef + go;
+            go += npad;
+            continue;
+        }
         CAT_CUDA(cudaMemcpyAsync(M->grp + go, S->grp, (size_t)npad * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
         CAT_CUDA(cudaMemcpyAsync(M->coef + go, S->coef, (size_t)npad * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
         CAT_CUDA(cudaMemcpyAsync(M->lambda + gl, S->lambda, (size_t)S->ngroups * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -296,7 +306,6 @@ int qa_model_concat(qa_ctx *ctx, int32_t num_models, qa_model *const *models, qa
             if (S->gbounds) CAT_CUDA(cudaMemcpyAsync(M->kappa + gk + S->ngroups, S->kappa + S->ngroups, gb, cudaMemcpyDeviceToDevice, ctx->stream));
             else CAT_CUDA(cudaMemsetAsync(M->kappa + gk + S->ngroups, 0, gb, ctx->stream));   // equality groups: lo = hi = 0
         }
-        ProblemDesc &D = M->descs[p];
         D.ngroups = S->ngroups;
         D.grp = M->grp + go;
         D.coef = M->coef + go;

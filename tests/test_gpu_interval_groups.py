@@ -81,6 +81,27 @@ def test_two_sided_mixed_sign(kctx, graph256):
     _assert_exact(*_run(kctx, m.h, m.starts, m.ends, m.weights, g, 64, 30, 11))
 
 
+@pytest.mark.parametrize("bounds", ["equality", "interval"])
+def test_max_groups_wide_coefficients(kctx, graph256, bounds):
+    """QA_MAX_GROUPS = 64 groups (the size of the per-read group sums in every kernel), holes (grp = -1) and coefficients of
+    2^19 .. 2^20: the 64-bit integer path.  Interval bounds two-sided, lower only and upper only."""
+    m = models.subsampling_model(graph256, 7.0)
+    n, G = m.num_variables, 64
+    rng = np.random.default_rng(64)
+    grp = np.where(rng.random(n) < 0.2, -1, rng.integers(0, G, size=n)).astype(np.int32)
+    coef = (rng.choice([-1, 1], size=n) * rng.integers(1 << 19, 1 << 20, size=n)).astype(np.int32)
+    lam = rng.uniform(2e-14, 2e-13, size=G)           # flip costs of order 1 at |u| ~ 2^22
+    kap = rng.integers(-(1 << 21), 1 << 21, size=G).astype(np.int64)
+    g = (grp, coef, lam, kap)
+    if bounds == "interval":
+        lo = rng.integers(-(1 << 22), 1 << 22, size=G).astype(np.int64)
+        hi = lo + rng.integers(0, 1 << 22, size=G)
+        side = np.arange(G) % 3
+        g += (np.where(side == 2, I64.min, lo), np.where(side == 1, I64.max, hi))
+    _assert_exact(*_run(kctx, m.h, m.starts, m.ends, m.weights, g, 64, 30, 19))
+    assert kctx.last_kernel == kctx.requested_kernel
+
+
 def test_le_constraint_model(kctx):
     cqm = ConstrainedQuadraticModel()
     x = [Binary(f"x{i}") for i in range(200)]
