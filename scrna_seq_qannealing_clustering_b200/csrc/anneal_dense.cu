@@ -15,16 +15,6 @@ int launch_dense(Launch &L) {
     qa_ctx *ctx = L.ctx;
     qa_model *M = L.M;
     AnnealParams &A = L.A;
-    const int P = M->num_problems;
-    const int32_t reads_per_problem = L.reads_per_problem;
-    const int64_t total_reads = L.total_reads;
-    const bool groups = L.groups;
-    const int32_t seed_mode = L.seed_mode;
-    qa_stats *st = L.st;
-    int64_t &done = L.done;
-    bool &interrupted = L.interrupted;
-    int rc = QA_OK;
-    (void)P; (void)reads_per_problem; (void)total_reads; (void)groups; (void)seed_mode; (void)interrupted; (void)rc;
     // dense k-way: one warp = 32 reads, fields of a block of 8 cells by fp64 tensor-core MMAs over all cells (dense.cuh)
     const int K = M->dn.K;
     const int warps = 4;
@@ -36,26 +26,26 @@ int launch_dense(Launch &L) {
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, warps * 32, smem, cudaOccupancyDefault));
     if (bps < 1) return fail(QA_ERR_CUDA, "dense kernel does not fit on an SM");
-    const int64_t total_tiles = (reads_per_problem + 31) / 32;
+    const int64_t total_tiles = (A.reads_per_problem + 31) / 32;
     // every warp pulls 32-read tiles from a counter; no more CTAs than the tiles can fill (warps without a tile leave at once)
     bps = std::min(bps, 2);   // 8 warps per SM beat 12 (measured, see dense.cuh)
     const int64_t grid = std::min<int64_t>((int64_t)bps * ctx->num_sms, (total_tiles + warps - 1) / warps);
     const int64_t stride = (int64_t)M->dn.ngrp * 32 * K;
-    rc = ensure(ctx->sf, (size_t)grid * warps * stride * sizeof(uint32_t));
+    const int rc = ensure(ctx->sf, (size_t)grid * warps * stride * sizeof(uint32_t));
     if (rc) return rc;
     A.dn_spins = (uint32_t *)ctx->sf.p;
     A.dn_stride = stride;
     A.total_tiles = total_tiles;
     A.read_begin = 0;
-    A.read_end = total_reads;
+    A.read_end = A.total_reads;
     QA_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
     QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));
     void *args[] = {&A, &M->dn};
     QA_CUDA(cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(warps * 32), args, smem, ctx->stream));
     QA_CUDA(cudaGetLastError());
     ctx->launches++;
-    if (st) st->anneal_launches++;
-    done = total_reads;
+    if (L.st) L.st->anneal_launches++;
+    L.done = A.total_reads;
     return QA_OK;
 }
 

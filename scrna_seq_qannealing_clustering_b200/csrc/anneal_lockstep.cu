@@ -7,20 +7,17 @@ using namespace qa;
 namespace {
 
 // ------------------------------------------------------------------------------------------------
-// lockstep kernels: one warp = 32 reads of the same problem; the lanes walk the variables together, every lane
+// lockstep kernel: one warp = 32 reads of the same problem; the lanes walk the variables together, every lane
 // owning one read (its own xorshift128+ state, its own spins, its own decisions).  The CSR row of the current
 // variable is shared by the warp, so a neighbour update is ONE coalesced 256-byte reduction for up to 32 reads
-// instead of 32 scattered 8-byte ones, and exp()/RNG run on all lanes at once.
-//   VARIANT 0 "push": local fields f[v][lane] (fp64, read-interleaved) are kept in HBM and updated by
-//                     red.global.add.f64 exactly like the warp-per-read kernel -> bit-exact against the oracle.
-//   VARIANT 2 "init": one pass that evaluates f[v] = h_v + sum_j J_vj s_j from the bit-packed spins through per-block
-//                     tables of distinct spin words (neal's get_flip_energy order) -- the set-up of the push variant.
-//   (A former VARIANT 1 re-evaluated the fields at every attempt as a non-bit-exact throughput mode for sparse models; the
-//   exact replay kernel overtook it and it was retired, DESIGN.md 4.4.  QA_MODE_THROUGHPUT now means the dense tensor-core
-//   kernel of dense.cuh.)
+// instead of 32 scattered 8-byte ones, and exp()/RNG run on all lanes at once.  A tile runs two kinds of pass:
+//   LS_FIELD_SETUP  once: evaluates f[v] = h_v + sum_j J_vj s_j from the bit-packed spins through per-block tables of
+//                   distinct spin words (neal's get_flip_energy order) and stores it.
+//   LS_PUSH         every sweep: local fields f[v][lane] (fp64, read-interleaved) are kept in HBM and updated by
+//                   red.global.add.f64 exactly like the warp-per-read kernel -> bit-exact against the oracle.
 // Spins live in the read-transposed packed layout packedT[word][read] the energy kernel consumes.
 // ------------------------------------------------------------------------------------------------
-constexpr int QA_LS_TPB = 128;   // threads per block of the lockstep kernels
+constexpr int QA_LS_TPB = 128;   // threads per block of the lockstep kernel
 constexpr int QA_LS_WPB = QA_LS_TPB / 32;
 constexpr int QA_LS_D = 16;      // variables per staged block
 constexpr int QA_LS_CAP = 384;   // CSR entries staged per block (longer blocks fall back to global loads)
@@ -36,7 +33,7 @@ struct LsStage {
     int am[QA_LS_D];
     int pad_;
 };
-struct LsStagePull {                            // field (re-)evaluation from spins: init pass and pull variant
+struct LsSetupStage {                           // field set-up pass: field evaluation from the spins
     double hb[2][QA_LS_D];                      // h of the block's variables
     unsigned int slotw[2][QA_LS_CAP / 2 + 2];   // per-entry (slot | bit << 8) as 16-bit pairs; slot 255 = own word
     int bw[2][QA_LS_CAPW];                      // distinct spin words referenced by the block
@@ -51,7 +48,7 @@ struct LsCtx {
     int *Mcol;
     double *cur;            // smem, per warp [QA_LS_D][32], this lane's column
     LsStage &sg;
-    LsStagePull &sp;
+    LsSetupStage &sp;
     uint32_t *words;        // smem [QA_LS_CAPW][32], this lane's column; aliases `cur` (never live at the same time)
     const double *lam_sh;
     const long long *kap_sh;
@@ -81,16 +78,19 @@ __device__ __forceinline__ double ls_field_direct(const ProblemDesc &D, const ui
     return fv;
 }
 
-// Runs the schedule from (bi, swi) on.  VARIANT 0 = push sweeps (bit-exact), 2 = one pass that only evaluates the local fields
-// from the spins and stores them (neal get_flip_energy order): the initialisation of the push variant.
-// GROUPS: 0 none, 1 rank-1 groups, 2 rank-1 groups with interval bounds (kap_sh then holds {kappa, lo, hi} per group).
-template <int VARIANT, int GROUPS>
-__device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, unsigned long long &s0,
-                          unsigned long long &s1, LaneStats &st) {
+enum LsPass { LS_PUSH, LS_FIELD_SETUP };
+
+// LS_PUSH: the whole schedule of push sweeps (bit-exact).  LS_FIELD_SETUP: one pass that only evaluates the local fields
+// from the spins and stores them (neal get_flip_energy order), before the push sweeps.
+// GROUPS: GK_NONE, GK_EQ64 (equality groups of both widths) or GK_INTERVAL (kap_sh then holds {kappa, lo, hi} per group).
+// The loop counters bi / swi are the caller's variables, both 0 on entry: with counters local to this function nvcc orders
+// a few instructions of the kernel differently, and the kernel's measured numbers (DESIGN.md 4.2) are for this SASS.
+template <LsPass PASS, GroupKind GROUPS>
+__device__ void ls_sweeps(const LsCtx &c, int &bi, int &swi, unsigned long long &s0, unsigned long long &s1, LaneStats &st) {
     const ProblemDesc &D = c.D;
     const AnnealParams &P = c.P;
     LsStage &sg = c.sg;
-    LsStagePull &sp = c.sp;
+    LsSetupStage &sp = c.sp;
     const int lane = threadIdx.x & 31;
     const int n = D.n;
     const int nch = D.nch;
@@ -100,13 +100,13 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
     double *cur = c.cur;
     int *Mcol = c.Mcol;
     const bool active = c.active;
-    const bool tables = VARIANT >= 1 && D.bw_ptr != nullptr;
+    const bool tables = PASS == LS_FIELD_SETUP && D.bw_ptr != nullptr;
     const int nblk = nch * (32 / QA_LS_D);
 
     // software pipeline over blocks of QA_LS_D variables:
-    //   rows (and, for pull, h / slot bytes / distinct-word list) of block b+1 are copied to shared memory by cp.async while
-    //   block b is processed; row pointers and group metadata run two blocks ahead in registers; (push) the local fields
-    //   of block b+1 are prefetched into registers and moved to shared memory at the switch.
+    //   rows (and, for the set-up pass, h / slot bytes / distinct-word list) of block b+1 are copied to shared memory by
+    //   cp.async while block b is processed; row pointers and group metadata run two blocks ahead in registers; (push) the
+    //   local fields of block b+1 are prefetched into registers and moved to shared memory at the switch.
     auto load_meta = [&](int blk, int &rp, int &gmv, int &amv) {
         const int v = blk * QA_LS_D + lane;
         rp = 0;
@@ -114,7 +114,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
         else if (tables && lane <= QA_LS_D + 2) rp = __ldg(D.bw_ptr + blk + (lane - QA_LS_D - 1));
         gmv = -1;
         amv = 0;
-        if (GROUPS) {
+        if (GROUPS != GK_NONE) {
             if (lane < QA_LS_D) {
                 gmv = __ldg(D.grp + v);
                 amv = __ldg(D.coef + v);
@@ -130,7 +130,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                 cp_async4(&sg.ej[buf][k], D.col + eb + k);
                 cp_async8(&sg.eJ[buf][k], D.val + eb + k);
             }
-            if (VARIANT >= 1) {
+            if (PASS == LS_FIELD_SETUP) {
                 if (tables) {
                     const int b0 = __shfl_sync(FULL_MASK, rp, QA_LS_D + 1);
                     const int b1 = __shfl_sync(FULL_MASK, rp, QA_LS_D + 2);
@@ -141,7 +141,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                 }
             }
         }
-        if (VARIANT >= 1) {
+        if (PASS == LS_FIELD_SETUP) {
             const int v = blk * QA_LS_D + lane;
             if (lane < QA_LS_D && v < n) cp_async8(&sp.hb[buf][lane], D.h + v);
         }
@@ -153,17 +153,16 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
     __syncwarp();
     stage_rows(0, 0, rp_cur);
     double nr[QA_LS_D];
-    if (VARIANT == 0) {
+    if (PASS == LS_PUSH) {
 #pragma unroll
         for (int i = 0; i < QA_LS_D; ++i) nr[i] = __ldcg(fT + (int64_t)i * 32 + lane);
     }
     int parity = 0;
-    bool finished = true;
 
-    const int nbeta = VARIANT == 2 ? 1 : P.num_betas;
-    const int nspb = VARIANT == 2 ? 1 : P.sweeps_per_beta;
+    const int nbeta = PASS == LS_FIELD_SETUP ? 1 : P.num_betas;
+    const int nspb = PASS == LS_FIELD_SETUP ? 1 : P.sweeps_per_beta;
     for (; bi < nbeta; ++bi, swi = 0) {
-        const double beta = VARIANT == 2 ? 1.0 : (D.betas ? D.betas : P.betas)[bi];
+        const double beta = PASS == LS_FIELD_SETUP ? 1.0 : (D.betas ? D.betas : P.betas)[bi];
         const double thr = 44.36142 / beta;
         for (; swi < nspb; ++swi) {
             uint32_t w = 0;
@@ -186,7 +185,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                 int rp_nn, gm_nn, am_nn;
                 load_meta(nb2, rp_nn, gm_nn, am_nn);
                 if (lane <= QA_LS_D) sg.rowp[lane] = rp_cur;
-                if (GROUPS) {
+                if (GROUPS != GK_NONE) {
                     if (lane < QA_LS_D) {
                         sg.gm[lane] = gm_cur;
                         sg.am[lane] = am_cur;
@@ -194,7 +193,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                 }
                 bool stale = false;
                 bool blk_dirty = false;
-                if (VARIANT == 0) {
+                if (PASS == LS_PUSH) {
 #pragma unroll
                     for (int i = 0; i < QA_LS_D; ++i) cur[i * 32] = nr[i];
 #pragma unroll
@@ -208,7 +207,7 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                 const double *eJ = sg.eJ[parity];
                 bool tabled = false;
                 const unsigned short *slots = nullptr;
-                if (VARIANT >= 1) {
+                if (PASS == LS_FIELD_SETUP) {
                     if (tables && staged) {
                         const int nbw = __shfl_sync(FULL_MASK, rp_cur, QA_LS_D + 2) - __shfl_sync(FULL_MASK, rp_cur, QA_LS_D + 1);
                         tabled = !(nbw == 1 && sp.bw[parity][0] < 0);
@@ -233,10 +232,10 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                     const int e0 = sg.rowp[i], e1 = sg.rowp[i + 1];
                     const bool up = (w >> (sub + i)) & 1u;
                     double fv;
-                    if (VARIANT == 0) {
+                    if (PASS == LS_PUSH) {
                         fv = cur[i * 32];
                     } else {
-                        // re-evaluate the local field from the spins: h_v + sum_j (+-J) in adjacency order
+                        // evaluate the local field from the spins: h_v + sum_j (+-J) in adjacency order
                         if (tabled) {
                             fv = sp.hb[parity][i];
 #pragma unroll 4
@@ -251,24 +250,18 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                         } else {
                             fv = ls_field_direct(D, pk, rpad, v, e0, e1, wi, w);
                         }
-                        if (VARIANT == 2) {
-                            __stcg(fT + (int64_t)v * 32 + lane, fv);
-                            continue;
-                        }
+                        __stcg(fT + (int64_t)v * 32 + lane, fv);
+                        continue;
                     }
                     double dE = up ? -2.0 * fv : 2.0 * fv;
                     int g = -1, a = 0;
-                    if (GROUPS) {
+                    if (GROUPS != GK_NONE) {
                         g = sg.gm[i];
                         if (g >= 0) {
                             a = sg.am[i];
-                            if (GROUPS == 2) {
-                                const long long *kb = c.kap_sh + 3 * g;
-                                dE = dE + interval_flip_cost(c.lam_sh[g], a, up, (long long)Mcol[g * QA_LS_TPB] + kb[0], kb[1], kb[2]);
-                            } else {
-                                const long long t = (long long)a * ((long long)a - (up ? 1 : -1) * ((long long)Mcol[g * QA_LS_TPB] + c.kap_sh[g]));
-                                dE = dE + c.lam_sh[g] * (double)t;
-                            }
+                            const long long *kb = c.kap_sh + kappa_words(GROUPS) * g;
+                            dE = dE + group_flip_cost<GROUPS>(c.lam_sh[g], a, up, (long long)Mcol[g * QA_LS_TPB] + kb[0],
+                                                              GROUPS == GK_INTERVAL ? kb[1] : 0, GROUPS == GK_INTERVAL ? kb[2] : 0);
                         }
                     }
                     const bool cand = active && !(dE >= thr);
@@ -281,52 +274,50 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
                         st.acc++;
                         st.nbr += (unsigned long long)(e1 - e0);
                     }
-                    if (VARIANT == 0) {
-                        const double cf = up ? -2.0 : 2.0;  // f[j] += -2*s_v*J  <=> neal dE[j] += 4*s_v*J*s_j
-                        double *fTl = fT + lane;
-                        const int nbv0 = nb * QA_LS_D;
-                        unsigned hit_next = 0;
-                        // neighbours inside the staged block are updated in shared memory only (the block is written back
-                        // once, below); all others get one predicated fire-and-forget reduction
-                        if (staged) {
+                    const double cf = up ? -2.0 : 2.0;  // f[j] += -2*s_v*J  <=> neal dE[j] += 4*s_v*J*s_j
+                    double *fTl = fT + lane;
+                    const int nbv0 = nb * QA_LS_D;
+                    unsigned hit_next = 0;
+                    // neighbours inside the staged block are updated in shared memory only (the block is written back
+                    // once, below); all others get one predicated fire-and-forget reduction
+                    if (staged) {
 #pragma unroll 4
-                            for (int k = e0 - eb; k < e1 - eb; ++k) {
-                                const int j = ej[k];
-                                const double d = cf * eJ[k];
-                                const unsigned rel = (unsigned)(j - v0);          // uniform
-                                if (rel < (unsigned)QA_LS_D) {
-                                    if (acc) cur[rel * 32] += d;
-                                    blk_dirty = true;
-                                } else {
-                                    red_add_f64_if(fTl + (int64_t)j * 32, d, acc);
-                                    hit_next |= (unsigned)((unsigned)(j - nbv0) < (unsigned)QA_LS_D);
-                                }
-                            }
-                        } else {
-                            for (int e = e0; e < e1; ++e) {
-                                const int j = __ldg(D.col + e);
-                                const double d = cf * __ldg(D.val + e);
-                                const unsigned rel = (unsigned)(j - v0);
-                                if (rel < (unsigned)QA_LS_D) {
-                                    if (acc) cur[rel * 32] += d;
-                                    blk_dirty = true;
-                                } else {
-                                    red_add_f64_if(fTl + (int64_t)j * 32, d, acc);
-                                    hit_next |= (unsigned)((unsigned)(j - nbv0) < (unsigned)QA_LS_D);
-                                }
+                        for (int k = e0 - eb; k < e1 - eb; ++k) {
+                            const int j = ej[k];
+                            const double d = cf * eJ[k];
+                            const unsigned rel = (unsigned)(j - v0);          // uniform
+                            if (rel < (unsigned)QA_LS_D) {
+                                if (acc) cur[rel * 32] += d;
+                                blk_dirty = true;
+                            } else {
+                                red_add_f64_if(fTl + (int64_t)j * 32, d, acc);
+                                hit_next |= (unsigned)((unsigned)(j - nbv0) < (unsigned)QA_LS_D);
                             }
                         }
-                        stale = stale || (hit_next != 0);  // prefetched registers of the next block are stale
+                    } else {
+                        for (int e = e0; e < e1; ++e) {
+                            const int j = __ldg(D.col + e);
+                            const double d = cf * __ldg(D.val + e);
+                            const unsigned rel = (unsigned)(j - v0);
+                            if (rel < (unsigned)QA_LS_D) {
+                                if (acc) cur[rel * 32] += d;
+                                blk_dirty = true;
+                            } else {
+                                red_add_f64_if(fTl + (int64_t)j * 32, d, acc);
+                                hit_next |= (unsigned)((unsigned)(j - nbv0) < (unsigned)QA_LS_D);
+                            }
+                        }
                     }
+                    stale = stale || (hit_next != 0);  // prefetched registers of the next block are stale
                     if (acc) {
                         w ^= 1u << (sub + i);
                         dirty = true;
-                        if (GROUPS) {
+                        if (GROUPS != GK_NONE) {
                             if (g >= 0) Mcol[g * QA_LS_TPB] -= 2 * a * (up ? 1 : -1);
                         }
                     }
                 }
-                if (VARIANT == 0) {
+                if (PASS == LS_PUSH) {
                     if (blk_dirty) {  // uniform: write the staged fields of this block back (coalesced 256 B rows)
 #pragma unroll
                         for (int i = 0; i < QA_LS_D; ++i) __stcg(fT + ((int64_t)v0 + i) * 32 + lane, cur[i * 32]);
@@ -345,10 +336,9 @@ __device__ bool ls_sweeps(const LsCtx &c, int &bi, int &swi, bool allow_switch, 
     }
     cp_async_wait<0>();
     __syncwarp();
-    return finished;
 }
 
-template <int VARIANT, int GROUPS>
+template <GroupKind GROUPS>
 __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned long long &s1, LaneStats &st, int *error_flag) {
     const ProblemDesc &D = c.D;
     const int n = D.n;
@@ -371,7 +361,7 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
         }
         pk[(int64_t)wi * rpad] = w;
     }
-    if (GROUPS) {
+    if (GROUPS != GK_NONE) {
         for (int g = 0; g < D.ngroups; ++g) c.Mcol[g * QA_LS_TPB] = 0;
         for (int wi = 0; wi < nch; ++wi) {
             const uint32_t w = pk[(int64_t)wi * rpad];
@@ -385,13 +375,9 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
             }
         }
     }
-    int bi = 0, swi = 0;
-    bool finished = false;
-    if (!finished) {
-        int ib = 0, is = 0;
-        ls_sweeps<2, 0>(c, ib, is, false, s0, s1, st);  // local fields from the current spins
-        ls_sweeps<0, GROUPS>(c, bi, swi, false, s0, s1, st);
-    }
+    int setup_bi = 0, setup_swi = 0, bi = 0, swi = 0;
+    ls_sweeps<LS_FIELD_SETUP, GK_NONE>(c, setup_bi, setup_swi, s0, s1, st);  // local fields from the current spins
+    ls_sweeps<LS_PUSH, GROUPS>(c, bi, swi, s0, s1, st);
 
     // ---- final spins back to the caller's +-1 rows
     if (c.active) {
@@ -404,50 +390,38 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
     }
 }
 
-__host__ __device__ inline size_t ls_smem_bytes(int max_groups, bool interval = false) {
-    size_t b = sizeof(double) * QA_LS_D * QA_LS_TPB;   // cur (push phases) / spin words (field evaluation phases)
-    b += (sizeof(LsStage) + sizeof(LsStagePull)) * QA_LS_WPB;
-    b += (sizeof(double) + (interval ? 3 : 1) * sizeof(long long)) * (size_t)max_groups;
+__host__ __device__ inline size_t ls_smem_bytes(int max_groups, GroupKind gk) {
+    size_t b = sizeof(double) * QA_LS_D * QA_LS_TPB;   // cur (push sweeps) / spin words (field set-up pass)
+    b += (sizeof(LsStage) + sizeof(LsSetupStage)) * QA_LS_WPB;
+    b += (sizeof(double) + kappa_words(gk) * sizeof(long long)) * (size_t)max_groups;
     b += sizeof(int) * (size_t)max_groups * QA_LS_TPB;
     return b;
 }
 
-template <int VARIANT, int GROUPS>
+template <GroupKind GROUPS>
 __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P) {
     extern __shared__ __align__(16) unsigned char ls_smem[];
-    // layout: [cur: D x TPB doubles, aliased by the spin words] [LsStage x warps] [LsStagePull x warps] [lambda] [kappa] [M]
+    // layout: [cur: D x TPB doubles, aliased by the spin words] [LsStage x warps] [LsSetupStage x warps] [lambda] [kappa] [M]
     // (interval groups: [kappa] is {kappa, lo, hi} per group)
     unsigned char *sp = ls_smem;
     double *cur_all = reinterpret_cast<double *>(sp);
     sp += sizeof(double) * QA_LS_D * QA_LS_TPB;
     LsStage *stages = reinterpret_cast<LsStage *>(sp);
     sp += sizeof(LsStage) * QA_LS_WPB;
-    LsStagePull *pstages = reinterpret_cast<LsStagePull *>(sp);
-    sp += sizeof(LsStagePull) * QA_LS_WPB;
+    LsSetupStage *setup_stages = reinterpret_cast<LsSetupStage *>(sp);
+    sp += sizeof(LsSetupStage) * QA_LS_WPB;
     uint32_t *words_all = reinterpret_cast<uint32_t *>(cur_all);
     double *lam_sh = reinterpret_cast<double *>(sp);
     sp += sizeof(double) * P.max_groups;
     long long *kap_sh = reinterpret_cast<long long *>(sp);
-    sp += (GROUPS == 2 ? 3 : 1) * sizeof(long long) * P.max_groups;
+    sp += kappa_words(GROUPS) * sizeof(long long) * P.max_groups;
     int *M_all = reinterpret_cast<int *>(sp);
     __shared__ unsigned long long next_tile[QA_LS_WPB];
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
     const int64_t slot = (int64_t)blockIdx.x * QA_LS_WPB + wib;
     double *fT = P.fT_scratch ? P.fT_scratch + slot * P.fT_stride : nullptr;
-    if (GROUPS) {  // groups exist only on single-problem models: one copy of lambda / kappa per block
-        const ProblemDesc &D0 = P.descs[0];
-        for (int g = threadIdx.x; g < D0.ngroups; g += blockDim.x) {
-            lam_sh[g] = D0.lambda[g];
-            if (GROUPS == 2) {
-                kap_sh[3 * g] = D0.kappa[g];
-                kap_sh[3 * g + 1] = D0.kappa[D0.ngroups + g];
-                kap_sh[3 * g + 2] = D0.kappa[2 * D0.ngroups + g];
-            } else {
-                kap_sh[g] = D0.kappa[g];
-            }
-        }
-    }
+    if (GROUPS != GK_NONE) stage_group_params<GROUPS>(P.descs[0], lam_sh, kap_sh);
     __syncthreads();
     LaneStats st = {0, 0, 0, 0, 0};
     for (;;) {
@@ -464,25 +438,14 @@ __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P
         const unsigned long long sd = active ? P.seeds[D.read_base + r] : 1ull;
         unsigned long long s0 = sd ? sd : ~0ull, s1 = 0;
         const LsCtx c = {D, P, r, active, fT, M_all + threadIdx.x, cur_all + wib * (QA_LS_D * 32) + lane, stages[wib],
-                         pstages[wib], words_all + wib * (QA_LS_CAPW * 32) + lane, lam_sh, kap_sh};
-        lockstep_tile<VARIANT, GROUPS>(c, s0, s1, st, P.error_flag);
+                         setup_stages[wib], words_all + wib * (QA_LS_CAPW * 32) + lane, lam_sh, kap_sh};
+        lockstep_tile<GROUPS>(c, s0, s1, st, P.error_flag);
     }
-    // warp-reduce the per-lane counters
-    unsigned long long v[5] = {st.cand, st.draws, st.acc, st.ties, st.nbr};
-#pragma unroll
-    for (int q = 0; q < 5; ++q)
-        for (int off = 16; off > 0; off >>= 1) v[q] += __shfl_xor_sync(FULL_MASK, v[q], off);
-    if (lane == 0) {
-        atomicAdd(P.stats + ST_CAND, v[0]);
-        atomicAdd(P.stats + ST_DRAWS, v[1]);
-        atomicAdd(P.stats + ST_ACC, v[2]);
-        atomicAdd(P.stats + ST_TIES, v[3]);
-        atomicAdd(P.stats + ST_NBR, v[4]);
-    }
+    flush_lane_stats(P, st);
 }
 
-// Block word tables for the pull variant: per block of QA_LS_D variables the distinct spin words (32 variables each) its
-// CSR rows refer to, and per CSR entry the slot of its word in that list.  Built once per model on the host from the
+// Block word tables for the field set-up pass: per block of QA_LS_D variables the distinct spin words (32 variables each)
+// its CSR rows refer to, and per CSR entry the slot of its word in that list.  Built once per model on the host from the
 // device-built CSR (a setup step, O(entries)); blocks that exceed the shared-memory capacities get a -1 sentinel.
 int build_word_tables(qa_model *M) {
     if (M->tables_built) return QA_OK;
@@ -560,23 +523,13 @@ int launch_lockstep(Launch &L) {
     qa_ctx *ctx = L.ctx;
     qa_model *M = L.M;
     AnnealParams &A = L.A;
-    const int P = M->num_problems;
-    const int32_t reads_per_problem = L.reads_per_problem;
-    const int64_t total_reads = L.total_reads;
-    const bool groups = L.groups;
-    const int32_t seed_mode = L.seed_mode;
-    qa_stats *st = L.st;
-    int64_t &done = L.done;
-    bool &interrupted = L.interrupted;
-    int rc = QA_OK;
-    (void)P; (void)reads_per_problem; (void)total_reads; (void)groups; (void)seed_mode; (void)interrupted; (void)rc;
     // lockstep: one warp = 32 reads of one problem
-    const int tpp = (reads_per_problem + 31) / 32;
-    const int64_t total_tiles = (int64_t)P * tpp;
-    const size_t smem = ls_smem_bytes(std::max(M->ngroups, 1), groups && L.interval);
-    const void *fn = nullptr;
-    fn = !groups ? (const void *)k_anneal_lockstep<0, 0>
-                 : (L.interval ? (const void *)k_anneal_lockstep<0, 2> : (const void *)k_anneal_lockstep<0, 1>);
+    const int tpp = (A.reads_per_problem + 31) / 32;
+    const int64_t total_tiles = (int64_t)A.num_problems * tpp;
+    const size_t smem = ls_smem_bytes(std::max(M->ngroups, 1), L.gk);
+    // EQ32 models run the 64-bit instance: this kernel has no 32-bit one
+    const void *fn = L.gk == GK_NONE ? (const void *)k_anneal_lockstep<GK_NONE>
+                   : L.gk == GK_INTERVAL ? (const void *)k_anneal_lockstep<GK_INTERVAL> : (const void *)k_anneal_lockstep<GK_EQ64>;
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, QA_LS_TPB, smem, cudaOccupancyDefault));
@@ -588,7 +541,7 @@ int launch_lockstep(Launch &L) {
     if (need < grid) grid = std::min<int64_t>(grid, std::max<int64_t>(need, std::min<int64_t>(total_tiles, (int64_t)ctx->num_sms)));
     const int64_t fT_stride = (int64_t)M->nch_max * 32 * 32;
     {
-        // read-interleaved local fields for the resident tiles (push kernel; push phase of the throughput mode)
+        // read-interleaved local fields for the resident tiles
         size_t free_b = 0, total_b = 0;
         QA_CUDA(cudaMemGetInfo(&free_b, &total_b));
         const size_t per_slot = (size_t)fT_stride * sizeof(double);
@@ -596,27 +549,27 @@ int launch_lockstep(Launch &L) {
         int64_t max_slots = (int64_t)(budget / per_slot);
         if (max_slots < wpb) return fail(QA_ERR_CUDA, "not enough device memory for one block of local fields");
         if (grid * wpb > max_slots) grid = max_slots / wpb;
-        rc = ensure(ctx->fT, (size_t)grid * wpb * per_slot);
+        const int rc = ensure(ctx->fT, (size_t)grid * wpb * per_slot);
         if (rc) return rc;
         A.fT_scratch = (double *)ctx->fT.p;
     }
-    rc = build_word_tables(M);  // field evaluation from spins (init pass of push, pull variant) runs on these
+    const int rc = build_word_tables(M);  // the field set-up pass runs on these
     if (rc) return rc;
-    QA_CUDA(cudaMemcpyAsync(M->d_descs, M->descs.data(), P * sizeof(ProblemDesc), cudaMemcpyHostToDevice, ctx->stream));
+    QA_CUDA(cudaMemcpyAsync(M->d_descs, M->descs.data(), A.num_problems * sizeof(ProblemDesc), cudaMemcpyHostToDevice, ctx->stream));
     A.fT_stride = fT_stride;
     A.tiles_per_problem = tpp;
     A.total_tiles = total_tiles;
     A.max_groups = std::max(M->ngroups, 1);
     A.read_begin = 0;
-    A.read_end = total_reads;
+    A.read_end = A.total_reads;
     QA_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
     QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));
     void *args[] = {&A};
     QA_CUDA(cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(QA_LS_TPB), args, smem, ctx->stream));
     QA_CUDA(cudaGetLastError());
     ctx->launches++;
-    if (st) st->anneal_launches++;
-    done = total_reads;
+    if (L.st) L.st->anneal_launches++;
+    L.done = A.total_reads;
     return QA_OK;
 }
 

@@ -16,8 +16,8 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // one read, reference order.  Restates neal simulated_annealing_run() for one `state`.
 // ------------------------------------------------------------------------------------------------
-// GROUPS: 0 none, 1 rank-1 groups, 2 rank-1 groups with interval bounds (read per problem, like lambda / kappa)
-template <int GROUPS>
+// GROUPS: GK_NONE, GK_EQ64 (equality groups of both widths) or GK_INTERVAL; lambda / kappa / bounds are read per problem
+template <GroupKind GROUPS>
 __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t r_local, double *__restrict__ f,
                             uint32_t *__restrict__ spw, unsigned long long &s0, unsigned long long &s1,
                             long long *Mw, WarpStats &st, int *error_flag) {
@@ -60,7 +60,7 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
         }
         __stcg(f + v, fv);
     }
-    if (GROUPS) {
+    if (GROUPS != GK_NONE) {
         for (int g = lane; g < D.ngroups; g += 32) Mw[g] = 0;
         __syncwarp();
         for (int c = 0; c < nch; ++c) {
@@ -100,13 +100,13 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                 int g = -1;
                 long long a = 0, kap = 0, glo = 0, ghi = 0;
                 double lam = 0.0;
-                if (GROUPS) {
+                if (GROUPS != GK_NONE) {
                     g = __ldg(D.grp + v);
                     if (g >= 0) {
                         a = __ldg(D.coef + v);
                         lam = __ldg(D.lambda + g);
                         kap = __ldg(D.kappa + g);
-                        if (GROUPS == 2) {
+                        if (GROUPS == GK_INTERVAL) {
                             glo = __ldg(D.kappa + D.ngroups + g);
                             ghi = __ldg(D.kappa + 2 * D.ngroups + g);
                         }
@@ -116,15 +116,8 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                 auto flip_cost = [&](uint32_t word) -> double {
                     const bool up = (word >> lane) & 1u;
                     double d = up ? -2.0 * fv : 2.0 * fv;
-                    if (GROUPS) {
-                        if (g >= 0) {
-                            if (GROUPS == 2) {
-                                d = d + interval_flip_cost(lam, a, up, Mw[g] + kap, glo, ghi);
-                            } else {
-                                const long long t = a * (a - (up ? 1 : -1) * (Mw[g] + kap));
-                                d = d + lam * (double)t;
-                            }
-                        }
+                    if (GROUPS != GK_NONE) {
+                        if (g >= 0) d = d + group_flip_cost<GROUPS>(lam, a, up, Mw[g] + kap, glo, ghi);
                     }
                     return d;
                 };
@@ -187,7 +180,7 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                             w ^= 1u << l;
                             gdirty = true;
                             if (lane == k) wg = w;
-                            if (GROUPS) {
+                            if (GROUPS != GK_NONE) {
                                 const int gl = __shfl_sync(FULL_MASK, g, l);
                                 if (gl >= 0) {
                                     const long long al = __shfl_sync(FULL_MASK, a, l);
@@ -221,16 +214,16 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
     for (int c = lane; c < nch; c += 32) D.packedT[(int64_t)c * D.rpad + r_local] = __ldcg(spw + c);
 }
 
-template <int GROUPS>
+template <GroupKind GROUPS>
 __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
-    __shared__ long long Msh[GROUPS ? (QA_TPB_MAX / 32) * QA_MAX_GROUPS : 1];
+    __shared__ long long Msh[GROUPS != GK_NONE ? (QA_TPB_MAX / 32) * QA_MAX_GROUPS : 1];
     __shared__ unsigned long long next_read[QA_TPB_MAX / 32];
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
     const int64_t slot = (int64_t)blockIdx.x * (blockDim.x >> 5) + wib;
     double *f = P.f_scratch + slot * P.f_stride;
     uint32_t *spw = P.spw_scratch + slot * P.spw_stride;
-    long long *Mw = GROUPS ? (Msh + wib * QA_MAX_GROUPS) : Msh;
+    long long *Mw = GROUPS != GK_NONE ? (Msh + wib * QA_MAX_GROUPS) : Msh;
     WarpStats st = {0, 0, 0, 0, 0, 0, 0};
 
     if (P.seed_mode == QA_SEED_STREAM) {
@@ -273,45 +266,35 @@ namespace qa {
 
 int ref_resident_reads(qa_ctx *ctx, int *out) {
     int bps = 0;
-    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<0>, QA_TPB_MAX, 0));
+    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<GK_NONE>, QA_TPB_MAX, 0));
     *out = bps * ctx->num_sms * (QA_TPB_MAX / 32);
     return QA_OK;
 }
 
 int launch_ref(Launch &L) {
     qa_ctx *ctx = L.ctx;
-    qa_model *M = L.M;
     AnnealParams &A = L.A;
-    const int P = M->num_problems;
-    const int32_t reads_per_problem = L.reads_per_problem;
-    const int64_t total_reads = L.total_reads;
-    const bool groups = L.groups;
-    const int32_t seed_mode = L.seed_mode;
-    qa_interrupt_fn interrupt = L.interrupt;
-    void *iuser = L.iuser;
-    qa_stats *st = L.st;
-    int64_t &done = L.done;
-    bool &interrupted = L.interrupted;
-    int rc = QA_OK;
-    (void)P; (void)reads_per_problem; (void)total_reads; (void)groups; (void)seed_mode; (void)interrupt; (void)iuser; (void)interrupted; (void)rc;
+    const int64_t total_reads = A.total_reads;
+    // EQ32 models run the 64-bit instance: this kernel has no 32-bit one
+    void (*const fn)(AnnealParams) = L.gk == GK_NONE ? k_anneal_ref<GK_NONE>
+                                   : L.gk == GK_INTERVAL ? k_anneal_ref<GK_INTERVAL> : k_anneal_ref<GK_EQ64>;
+    const bool stream = A.seed_mode == QA_SEED_STREAM;
     // launch geometry: persistent grid, one warp per resident read
     int wpb = QA_TPB_MAX / 32;
-    if (seed_mode == QA_SEED_STREAM) wpb = 1;
+    if (stream) wpb = 1;
     else if (total_reads < (int64_t)ctx->num_sms * wpb) wpb = (int)std::max<int64_t>(1, (total_reads + ctx->num_sms - 1) / ctx->num_sms);
     const int tpb = wpb * 32;
     int bps = 0;
-    if (groups && L.interval) QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<2>, tpb, 0));
-    else if (groups) QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<1>, tpb, 0));
-    else QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<0>, tpb, 0));
+    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, fn, tpb, 0));
     if (bps < 1) return fail(QA_ERR_CUDA, "annealing kernel does not fit on an SM");
     int64_t grid = (int64_t)bps * ctx->num_sms;  // multiple of the SM count
     const int64_t need = (total_reads + wpb - 1) / wpb;
     if (need < grid) grid = need;
-    if (seed_mode == QA_SEED_STREAM) grid = 1;
+    if (stream) grid = 1;
     const int64_t slots = grid * wpb;
-    const int64_t f_stride = (int64_t)M->nch_max * 32;
-    const int64_t spw_stride = ((int64_t)M->nch_max + 31) & ~31ll;
-    rc = ensure(ctx->f, (size_t)slots * f_stride * sizeof(double));
+    const int64_t f_stride = (int64_t)L.M->nch_max * 32;
+    const int64_t spw_stride = ((int64_t)L.M->nch_max + 31) & ~31ll;
+    int rc = ensure(ctx->f, (size_t)slots * f_stride * sizeof(double));
     if (!rc) rc = ensure(ctx->spw, (size_t)slots * spw_stride * sizeof(uint32_t));
     if (rc) return rc;
     A.f_scratch = (double *)ctx->f.p;
@@ -320,22 +303,20 @@ int launch_ref(Launch &L) {
     A.spw_stride = spw_stride;
 
     // without an interrupt callback the whole job is one launch; with one, read waves of `slots` reads
-    const int64_t wave = (interrupt && seed_mode != QA_SEED_STREAM) ? slots : total_reads;
+    const int64_t wave = (L.interrupt && !stream) ? slots : total_reads;
     QA_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    while (done < total_reads) {
-        A.read_begin = done;
-        A.read_end = std::min(total_reads, done + wave);
+    while (L.done < total_reads) {
+        A.read_begin = L.done;
+        A.read_end = std::min(total_reads, L.done + wave);
         QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));
-        if (groups && L.interval) k_anneal_ref<2><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
-        else if (groups) k_anneal_ref<1><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
-        else k_anneal_ref<0><<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
+        fn<<<(unsigned)grid, tpb, 0, ctx->stream>>>(A);
         QA_CUDA(cudaGetLastError());
         ctx->launches++;
-        if (st) st->anneal_launches++;
-        done = A.read_end;
-        if (interrupt && done < total_reads) {
+        if (L.st) L.st->anneal_launches++;
+        L.done = A.read_end;
+        if (L.interrupt && L.done < total_reads) {
             QA_CUDA(cudaStreamSynchronize(ctx->stream));
-            if (interrupt(iuser)) { interrupted = true; break; }
+            if (L.interrupt(L.iuser)) { L.interrupted = true; break; }
         }
     }
     return QA_OK;

@@ -327,31 +327,36 @@ int build_replay_tables(qa_model *M) {
     return QA_OK;
 }
 
+template <int SLOTS, bool KWAY>
+static const void *replay_instance(GroupKind gk) {
+    switch (gk) {
+    case GK_NONE: return (const void *)k_anneal_replay<GK_NONE, SLOTS, KWAY>;
+    case GK_EQ32: return (const void *)k_anneal_replay<GK_EQ32, SLOTS, KWAY>;
+    case GK_EQ64: return (const void *)k_anneal_replay<GK_EQ64, SLOTS, KWAY>;
+    default: return (const void *)k_anneal_replay<GK_INTERVAL, SLOTS, KWAY>;
+    }
+}
+
+// the instance for the model's group kind and slot count; models with k-way blocks run the one with the k-way batch phase
+static const void *replay_kernel(const qa_model *M, GroupKind gk) {
+    const bool kway = M->rp_kway_blocks > 0;
+    if (M->rp_slots == 32) return kway ? replay_instance<32, true>(gk) : replay_instance<32, false>(gk);
+    return kway ? replay_instance<64, true>(gk) : replay_instance<64, false>(gk);
+}
+
 int launch_replay(Launch &L) {
     qa_ctx *ctx = L.ctx;
     qa_model *M = L.M;
     AnnealParams &A = L.A;
-    const int P = M->num_problems;
-    const int32_t reads_per_problem = L.reads_per_problem;
-    const int64_t total_reads = L.total_reads;
-    const bool groups = L.groups;
-    const int32_t seed_mode = L.seed_mode;
-    qa_interrupt_fn interrupt = L.interrupt;
-    void *iuser = L.iuser;
-    qa_stats *st = L.st;
-    int64_t &done = L.done;
-    bool &interrupted = L.interrupted;
-    int rc = QA_OK;
-    (void)P; (void)reads_per_problem; (void)total_reads; (void)groups; (void)seed_mode; (void)interrupt; (void)iuser; (void)interrupted; (void)rc;
+    const int P = A.num_problems;
     // replay: one CTA = `nw` consecutive 32-read tiles of one problem, coupling slabs shared through a TMA ring
-    const int tpp = (reads_per_problem + 31) / 32;
+    const int tpp = (A.reads_per_problem + 31) / 32;
     const int mg = std::max(M->ngroups, 1);
-    const bool ivl = groups && L.interval;
     int nw = ctx->replay_warps;
     if (nw < 1 || nw > RP_MAX_WARPS) {
         nw = 1;
         while (nw < RP_MAX_WARPS && nw < tpp) nw *= 2;
-        while (nw > 1 && rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl) > (size_t)(226 * 1024 / RP_MIN_CTAS - 1024)) nw /= 2;   // RP_MIN_CTAS CTAs per SM
+        while (nw > 1 && rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, L.gk) > (size_t)(226 * 1024 / RP_MIN_CTAS - 1024)) nw /= 2;   // RP_MIN_CTAS CTAs per SM
         // less than one full wave of 8-warp CTAs: 4-warp CTAs (3 per SM) balance the SMs better -- measured on config 3
         // (profiles/r2_probe_strong_scaling_read_counts.log): 50 000 reads 7.4e10 against 6.8e10 with 8 warps, 25 000 and 12 500
         // reads within 1 % of the best choice; 1- and 2-warp CTAs are residency-limited by the slab ring's shared memory
@@ -361,17 +366,8 @@ int launch_replay(Launch &L) {
     }
     const int64_t gpp = (tpp + nw - 1) / nw;
     const int64_t total_items = (int64_t)P * gpp;
-    size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl);
-    // models with k-way blocks run the instance with the k-way batch phase; all others the generic one
-#define QA_RP_FN(G, S) (M->rp_kway_blocks > 0 ? (const void *)k_anneal_replay<G, S, true> : (const void *)k_anneal_replay<G, S, false>)
-    const void *fn = nullptr;
-    if (groups && L.interval)
-        fn = M->rp_slots == 32 ? QA_RP_FN(3, 32) : QA_RP_FN(3, 64);
-    else if (M->rp_slots == 32)
-        fn = !groups ? QA_RP_FN(0, 32) : (M->groups_i32 ? QA_RP_FN(1, 32) : QA_RP_FN(2, 32));
-    else
-        fn = !groups ? QA_RP_FN(0, 64) : (M->groups_i32 ? QA_RP_FN(1, 64) : QA_RP_FN(2, 64));
-#undef QA_RP_FN
+    size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, L.gk);
+    const void *fn = replay_kernel(M, L.gk);
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, nw * 32, smem, cudaOccupancyDefault));
@@ -387,7 +383,7 @@ int launch_replay(Launch &L) {
         const int64_t max_slots = (int64_t)(budget / per_slot);
         if (max_slots < nw) return fail(QA_ERR_CUDA, "not enough device memory for one CTA of local fields");
         if (grid * nw > max_slots) grid = max_slots / nw;
-        rc = ensure(ctx->fT, (size_t)grid * nw * fT_stride * sizeof(double) + 4096);   // + the look-ahead rows of the last slot
+        int rc = ensure(ctx->fT, (size_t)grid * nw * fT_stride * sizeof(double) + 4096);   // + the look-ahead rows of the last slot
         if (!rc) rc = ensure(ctx->sf, (size_t)grid * nw * sf_stride * sizeof(uint32_t));
         if (rc) return rc;
     }
@@ -402,8 +398,8 @@ int launch_replay(Launch &L) {
     A.switch_permille = ctx->replay_switch_permille;
     A.rp_slab_init = M->rp_adj_sorted ? 1 : 0;
     A.read_begin = 0;
-    A.read_end = total_reads;
-    if (interrupt) {
+    A.read_end = A.total_reads;
+    if (L.interrupt) {
         *ctx->h_iflag = 0;
         A.interrupt_flag = ctx->d_iflag;
     }
@@ -420,7 +416,7 @@ int launch_replay(Launch &L) {
             QA_CUDA(cudaStreamSynchronize(ctx->stream));
             if (fl[0] == QA_ERR_SMEM_BASE) {
                 ctx->rp_smem_base = (unsigned)fl[1];
-                smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, ivl);
+                smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, L.gk);
                 QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
                 QA_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 2 * sizeof(int), ctx->stream));
                 QA_CUDA(cudaMemsetAsync(A.counter, 0, sizeof(unsigned long long), ctx->stream));
@@ -432,26 +428,26 @@ int launch_replay(Launch &L) {
             ctx->rp_base_checked = true;
         }
     }
-    if (st) st->anneal_launches++;
-    done = total_reads;
-    if (interrupt) {   // poll the callback while the launch runs; CTAs stop pulling work once the flag is up
+    if (L.st) L.st->anneal_launches++;
+    L.done = A.total_reads;
+    if (L.interrupt) {   // poll the callback while the launch runs; CTAs stop pulling work once the flag is up
         QA_CUDA(cudaEventRecord(ctx->ev[3], ctx->stream));
         for (;;) {
             const cudaError_t q = cudaEventQuery(ctx->ev[3]);
             if (q == cudaSuccess) break;
             if (q != cudaErrorNotReady) return fail(QA_ERR_CUDA, std::string("replay kernel: ") + cudaGetErrorString(q));
-            if (!interrupted && interrupt(iuser)) {
+            if (!L.interrupted && L.interrupt(L.iuser)) {
                 *reinterpret_cast<volatile int *>(ctx->h_iflag) = 1;
-                interrupted = true;
+                L.interrupted = true;
             }
             struct timespec ts = {0, 200000};
             nanosleep(&ts, nullptr);
         }
-        if (interrupted) {   // groups are handed out in read order: the first `pulled` groups are complete
+        if (L.interrupted) {   // groups are handed out in read order: the first `pulled` groups are complete
             unsigned long long pulled = 0;
             QA_CUDA(cudaMemcpyAsync(&pulled, A.counter, sizeof(pulled), cudaMemcpyDeviceToHost, ctx->stream));
             QA_CUDA(cudaStreamSynchronize(ctx->stream));
-            done = std::min<int64_t>(total_reads, (int64_t)std::min<unsigned long long>(pulled, (unsigned long long)total_items) * nw * 32);
+            L.done = std::min<int64_t>(A.total_reads, (int64_t)std::min<unsigned long long>(pulled, (unsigned long long)total_items) * nw * 32);
         }
     }
     return QA_OK;

@@ -25,6 +25,52 @@ int check_schedule(int32_t num_betas, const double *betas, int32_t sweeps_per_be
     return QA_OK;
 }
 
+// The annealing kernel of a call.  The rules, in order; the first that applies decides:
+//   1. DENSE          QA_MODE_THROUGHPUT on a model with the dense k-way form: one problem, per-read seeds, no interrupt
+//                     callback (the tensor-core kernel, tolerance parity).  Every other model runs a reference-order kernel:
+//                     for sparse models the exact replay kernel is faster than any recompute or graph-coloured update
+//                     (DESIGN.md 4.4), and bit-exact results meet the statistical bar trivially.
+//   2. WARP_PER_READ  stream seeding (one xorshift128+ stream across reads), and batched models with rank-1 groups
+//                     (qa_model_concat): the lockstep and replay kernels keep one copy of lambda / kappa per CTA, the
+//                     warp-per-read kernel reads them per problem.
+//   3. REPLAY         (deferred exact updates) when requested, or under AUTO from 32 reads per problem and 6144 reads in all
+//                     (measured on B200, config 3: 1.26e10 vs 7.5e9 attempts/s for the warp-per-read kernel at 12 500 reads,
+//                     4.3e9 vs 5.9e9 at 4096), if the model fits the slab format (build_replay_tables) and an interrupt
+//                     callback comes with a single problem: the kernel polls a host-mapped flag whenever a CTA pulls its
+//                     next group of reads.
+//   4. a requested REPLAY that rule 3 refused (dense rows: the slab format does not apply) runs LOCKSTEP, or
+//      WARP_PER_READ with an interrupt callback.
+//   5. LOCKSTEP       when requested, or under AUTO from 32 reads per problem and 3.5 tiles of 32 reads per SM, without an
+//                     interrupt callback: the lockstep kernel has no stopping point.
+//   6. WARP_PER_READ  otherwise: any read count; with an interrupt callback it runs in read waves and polls between them.
+int pick_kernel(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int64_t total_reads, int32_t seed_mode, int32_t mode,
+                bool interrupt, int *kernel) {
+    const int P = M->num_problems;
+    const bool auto_ok = ctx->kernel == QA_KERNEL_AUTO && reads_per_problem >= 32;
+    if (mode == QA_MODE_THROUGHPUT && M->dn_ok && P == 1 && !interrupt && seed_mode == QA_SEED_PER_READ) {
+        *kernel = QA_KERNEL_DENSE;
+        return QA_OK;
+    }
+    *kernel = QA_KERNEL_WARP_PER_READ;
+    if (seed_mode != QA_SEED_PER_READ || (P > 1 && M->ngroups > 0)) return QA_OK;
+    if ((ctx->kernel == QA_KERNEL_REPLAY || (auto_ok && total_reads >= 6144)) && (!interrupt || P == 1)) {
+        const int rc = build_replay_tables(M);
+        if (rc) return rc;
+        if (M->rp_ok) {
+            *kernel = QA_KERNEL_REPLAY;
+            QA_CUDA(cudaMemcpyAsync(M->d_descs, M->descs.data(), P * sizeof(ProblemDesc), cudaMemcpyHostToDevice, ctx->stream));
+            return QA_OK;
+        }
+    }
+    if (ctx->kernel == QA_KERNEL_REPLAY) {
+        if (!interrupt) *kernel = QA_KERNEL_LOCKSTEP_PUSH;
+        return QA_OK;
+    }
+    if ((ctx->kernel == QA_KERNEL_LOCKSTEP_PUSH || (auto_ok && 2 * total_reads >= (int64_t)ctx->num_sms * 32 * 7)) && !interrupt)
+        *kernel = QA_KERNEL_LOCKSTEP_PUSH;
+    return QA_OK;
+}
+
 // core: anneal all reads of all problems of a model; states/energies already on the device
 int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_states, double *d_energies,
                int32_t num_betas, const double *d_betas, int32_t sweeps_per_beta, const unsigned long long *d_seeds,
@@ -58,39 +104,9 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
         QA_CUDA(cudaMemcpyAsync(M->d_descs, M->descs.data(), P * sizeof(ProblemDesc), cudaMemcpyHostToDevice, ctx->stream));
     }
 
-    const bool groups = M->ngroups > 0;
-    // kernel choice: warp-per-read (any read count, stream seeding) or lockstep (32 reads per warp)
-    // QA_MODE_THROUGHPUT: a model with the dense k-way form runs the tensor-core kernel (tolerance parity); every other model
-    // runs the reference-order kernels below -- for sparse models the exact replay kernel is faster than any recompute or
-    // graph-coloured update (DESIGN.md 4.4), and bit-exact results meet the statistical bar trivially
-    int kernel = QA_KERNEL_WARP_PER_READ;
-    if (mode == QA_MODE_THROUGHPUT && M->dn_ok && P == 1 && !interrupt && seed_mode == QA_SEED_PER_READ) kernel = QA_KERNEL_DENSE;
-    else if (ctx->kernel == QA_KERNEL_LOCKSTEP_PUSH && seed_mode == QA_SEED_PER_READ) kernel = QA_KERNEL_LOCKSTEP_PUSH;
-    else if (ctx->kernel == QA_KERNEL_AUTO && seed_mode == QA_SEED_PER_READ && (int64_t)reads_per_problem >= 32 &&
-             2 * total_reads >= (int64_t)ctx->num_sms * 32 * 7)
-        kernel = QA_KERNEL_LOCKSTEP_PUSH;
-    // replay kernel (deferred exact updates): sparse models whose blocks fit the slab format; explicit choice, or automatic
-    // from 6144 reads on (measured on B200, config 3: 1.26e10 vs 7.5e9 attempts/s for the warp-per-read kernel at 12 500
-    // reads, 4.3e9 vs 5.9e9 at 4096)
-    // an interrupt callback: the warp-per-read kernel runs in read waves and polls between them; the replay kernel polls a
-    // host-mapped flag whenever a CTA pulls its next group of reads; the lockstep push kernel has no stopping point
-    if (interrupt && kernel == QA_KERNEL_LOCKSTEP_PUSH) kernel = QA_KERNEL_WARP_PER_READ;
-    // batched models with rank-1 groups (qa_model_concat): the lockstep and replay kernels keep one copy of lambda / kappa per
-    // CTA, so those run on the warp-per-read kernel, which reads them per problem
-    if (P > 1 && groups) kernel = QA_KERNEL_WARP_PER_READ;
-    if (kernel != QA_KERNEL_DENSE && seed_mode == QA_SEED_PER_READ && (!interrupt || P == 1) && !(P > 1 && groups) &&
-        (ctx->kernel == QA_KERNEL_REPLAY ||
-         (ctx->kernel == QA_KERNEL_AUTO && (int64_t)reads_per_problem >= 32 && total_reads >= 6144))) {
-        rc = build_replay_tables(M);
-        if (rc) return rc;
-        if (M->rp_ok) {
-            kernel = QA_KERNEL_REPLAY;
-            QA_CUDA(cudaMemcpyAsync(M->d_descs, M->descs.data(), P * sizeof(ProblemDesc), cudaMemcpyHostToDevice, ctx->stream));
-        } else if (ctx->kernel == QA_KERNEL_REPLAY) {
-            kernel = interrupt ? QA_KERNEL_WARP_PER_READ : QA_KERNEL_LOCKSTEP_PUSH;  // dense model: the slab format does not apply
-        }
-    }
-
+    int kernel = 0;
+    rc = pick_kernel(ctx, M, reads_per_problem, total_reads, seed_mode, mode, interrupt != nullptr, &kernel);
+    if (rc) return rc;
     ctx->last_kernel = kernel;
     QA_CUDA(cudaMemsetAsync(ctx->d_stats, 0, (QA_NSTAT + 1 + QA_NDEBUG) * sizeof(unsigned long long), ctx->stream));
     QA_CUDA(cudaMemsetAsync(ctx->d_flag, 0, 2 * sizeof(int), ctx->stream));
@@ -115,11 +131,7 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
     L.ctx = ctx;
     L.M = M;
     L.A = A;
-    L.reads_per_problem = reads_per_problem;
-    L.total_reads = total_reads;
-    L.groups = groups;
-    L.interval = groups && M->gbounds;
-    L.seed_mode = seed_mode;
+    L.gk = M->ngroups == 0 ? GK_NONE : M->gbounds ? GK_INTERVAL : M->groups_i32 ? GK_EQ32 : GK_EQ64;
     L.interrupt = interrupt;
     L.iuser = iuser;
     L.st = st;

@@ -72,8 +72,8 @@ struct ProblemDesc {
     int8_t *states;         // [reads][n]
     uint32_t *packedT;      // [nch][rpad] final spins, bit i of word (c, r) = spin of variable 32c+i (1: +1)
     double *energies;       // [reads]
-    // block word tables of the pull variant (null until built): for every block of 16 variables the distinct spin words
-    // its CSR rows refer to, and per CSR entry the index of its word in that list (255 = the block's own word)
+    // block word tables of the lockstep kernel's field set-up pass (null until built): for every block of 16 variables the
+    // distinct spin words its CSR rows refer to, and per CSR entry the index of its word in that list (255 = the block's own word)
     const int32_t *bw_ptr;      // [nblk + 1], this problem's first block at index 0 (values are global offsets)
     const int32_t *bw_words;    // global array
     const unsigned short *ent_slot; // indexed like col: slot | (bit << 8)
@@ -193,7 +193,7 @@ struct qa_model {
     std::vector<int64_t> gumin, gumax;         // host: reachable range kappa -+ sum |a| of every group (single-problem models)
     qa::ProblemDesc *d_descs = nullptr;
     std::vector<qa::ProblemDesc> descs;  // host mirror (pointers are device pointers)
-    // block word tables of the pull variant (built on first use)
+    // block word tables of the lockstep kernel's field set-up pass (built on first use)
     int32_t *bw_ptr = nullptr, *bw_words = nullptr;
     unsigned short *ent_slot = nullptr;
     bool tables_built = false;
@@ -281,6 +281,29 @@ __host__ __device__ __forceinline__ double interval_flip_cost(double lam, long l
     return lam * ((double)(d1 * d1 - d0 * d0) * 0.25);
 }
 
+// Kind of a model's rank-1 group term, decided once per launch (run_anneal) and the GROUPS template argument of every
+// annealing kernel.  EQ32: equality groups whose terms the host proved to fit 32-bit integers (qa_model::groups_i32).
+enum GroupKind { GK_NONE = 0, GK_EQ32 = 1, GK_EQ64 = 2, GK_INTERVAL = 3 };
+
+// 64-bit words of kappa staged per group in shared memory: {kappa, lo, hi} for interval groups, kappa otherwise
+__host__ __device__ constexpr int kappa_words(GroupKind gk) { return gk == GK_INTERVAL ? 3 : 1; }
+
+// Change of the group term when a variable with coefficient a and spin up / down flips, u = M_g + kappa_g.  Equality groups:
+// lambda * (double)(a * (a - s u)), in 32-bit integers for GK_EQ32 (u then holds a 32-bit sum).  lo / hi are read for
+// interval groups only.
+template <GroupKind GK>
+__host__ __device__ __forceinline__ double group_flip_cost(double lam, long long a, bool up, long long u, long long lo,
+                                                           long long hi) {
+    if (GK == GK_INTERVAL) return interval_flip_cost(lam, a, up, u, lo, hi);
+    if (GK == GK_EQ32) {
+        const int m = (int)u;
+        const int t = (int)a * ((int)a - (up ? m : -m));
+        return lam * (double)t;
+    }
+    const long long t = a * (a - (up ? 1 : -1) * u);
+    return lam * (double)t;
+}
+
 inline unsigned blocks_for(int64_t count, int tpb = 256) { return (unsigned)std::max<int64_t>(1, (count + tpb - 1) / tpb); }
 
 // device scratch of one build, freed on every path
@@ -308,12 +331,8 @@ int sample_common(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *s
 struct Launch {
     qa_ctx *ctx;
     qa_model *M;
-    AnnealParams A;
-    int32_t reads_per_problem;
-    int64_t total_reads;
-    bool groups;
-    bool interval;         // the groups carry interval bounds
-    int32_t seed_mode;
+    AnnealParams A;        // also the launch's shape: reads_per_problem, total_reads, seed_mode
+    GroupKind gk;
     qa_interrupt_fn interrupt;
     void *iuser;
     qa_stats *st;

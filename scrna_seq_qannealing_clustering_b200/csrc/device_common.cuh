@@ -1,5 +1,6 @@
 // device_common.cuh -- device helpers shared by the annealing kernels: neal's xorshift128+ step, the accept test with its
-// single-precision screen, L2 prefetch / fp64 reduction wrappers, cp.async wrappers, per-lane event counters.
+// single-precision screen, L2 prefetch / fp64 reduction wrappers, cp.async wrappers, per-lane event counters, group
+// parameters in shared memory.
 #pragma once
 
 #include "common.cuh"
@@ -86,6 +87,37 @@ __device__ __forceinline__ bool ls_accept(double dE, bool cand, double beta, uns
         }
     }
     return acc;
+}
+
+// lambda / kappa of every group into shared memory, kappa_words(GK) words of kappa per group ({kappa, lo, hi} for interval
+// groups).  Groups exist only on single-problem models, so the lockstep and replay kernels keep one copy per block.
+template <GroupKind GK>
+__device__ __forceinline__ void stage_group_params(const ProblemDesc &D0, double *lam_sh, long long *kap_sh) {
+    for (int g = threadIdx.x; g < D0.ngroups; g += blockDim.x) {
+        lam_sh[g] = D0.lambda[g];
+        if (GK == GK_INTERVAL) {
+            kap_sh[3 * g] = D0.kappa[g];
+            kap_sh[3 * g + 1] = D0.kappa[D0.ngroups + g];
+            kap_sh[3 * g + 2] = D0.kappa[2 * D0.ngroups + g];
+        } else {
+            kap_sh[g] = D0.kappa[g];
+        }
+    }
+}
+
+// warp-reduce the per-lane counters and add them to the launch's totals
+__device__ __forceinline__ void flush_lane_stats(const AnnealParams &P, const LaneStats &st) {
+    unsigned long long v[5] = {st.cand, st.draws, st.acc, st.ties, st.nbr};
+#pragma unroll
+    for (int q = 0; q < 5; ++q)
+        for (int off = 16; off > 0; off >>= 1) v[q] += __shfl_xor_sync(FULL_MASK, v[q], off);
+    if ((threadIdx.x & 31) == 0) {
+        atomicAdd(P.stats + ST_CAND, v[0]);
+        atomicAdd(P.stats + ST_DRAWS, v[1]);
+        atomicAdd(P.stats + ST_ACC, v[2]);
+        atomicAdd(P.stats + ST_TIES, v[3]);
+        atomicAdd(P.stats + ST_NBR, v[4]);
+    }
 }
 
 }  // namespace qa

@@ -344,13 +344,30 @@ __device__ __forceinline__ void rp_stage_wait() {
     __syncwarp();
 }
 
+// group term of a decision: M_g + kappa_g and the bounds from shared memory
+template <GroupKind GROUPS>
+__device__ __forceinline__ double rp_group_flip_cost(const RpCtx &c, int g, int ca, bool up) {
+    if (GROUPS == GK_EQ32) {   // kappa's low 32-bit word, added in 32-bit arithmetic (the host checked the ranges)
+        const int m = c.Mcol[g * c.mstride] + reinterpret_cast<const int *>(c.kap)[2 * g];
+        return group_flip_cost<GK_EQ32>(c.lam[g], ca, up, m, 0, 0);
+    }
+    if (GROUPS == GK_EQ64) {
+        // group_flip_cost's form, written out: with M_g + kappa_g formed before the product, nvcc allocates the registers
+        // of the k-way instances (which spill) differently
+        const long long t = (long long)ca * ((long long)ca - (up ? 1 : -1) * ((long long)c.Mcol[g * c.mstride] + c.kap[g]));
+        return c.lam[g] * (double)t;
+    }
+    const long long *kb = c.kap + 3 * g;
+    return group_flip_cost<GK_INTERVAL>(c.lam[g], ca, up, (long long)c.Mcol[g * c.mstride] + kb[0], kb[1], kb[2]);
+}
+
 // One pass over all blocks.  MODE 0: replay sweep.  MODE 1: catch-up (pending later-neighbour updates only, no decisions).
 // MODE 2: push sweep (neal's eager form).  MODE 3: field set-up f[v] = h_v + sum_j J_vj s_j in neal's get_flip_energy order,
 // for models whose adjacency lists are ascending (then adjacency order = pre entries u < v0, seq entries, later entries).
-// GROUPS: 0 none, 1 rank-1 groups with 32-bit exact integer arithmetic (host-checked ranges), 2 with 64-bit, 3 interval groups
-// (64-bit; c.kap then holds {kappa, lo, hi} per group).  KWAY: the slabs carry k-way sections (rp_kway_batch); false compiles
-// the replay sweep without the section test, so models without k-way blocks run exactly the generic kernel.
-template <int MODE, int GROUPS, int SLOTS, bool KWAY = false>
+// GROUPS: the group term (GK_INTERVAL: c.kap holds {kappa, lo, hi} per group).  KWAY: the slabs carry k-way sections
+// (rp_kway_batch); false compiles the replay sweep without the section test, so models without k-way blocks run exactly the
+// generic kernel.
+template <int MODE, GroupKind GROUPS, int SLOTS, bool KWAY = false>
 __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
     const int lane = threadIdx.x & 31;
     const double thr = 44.36142 / beta;
@@ -511,22 +528,12 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 const bool up = (W & db) == 0u;
                 double dE = up ? -2.0 * fv : 2.0 * fv;
                 int g = 255, ca = 0;
-                if (GROUPS) {
+                if (GROUPS != GK_NONE) {
                     const int ga = (int)lds_u32(hdr + RP_H_GA + 4u * (uint32_t)i);
                     g = ga & 255;
                     if (g != 255) {
                         ca = ga >> 8;
-                        if (GROUPS == 1) {
-                            const int m = c.Mcol[g * c.mstride] + reinterpret_cast<const int *>(c.kap)[2 * g];
-                            const int t = ca * (ca - (up ? m : -m));
-                            dE = dE + c.lam[g] * (double)t;
-                        } else if (GROUPS == 3) {
-                            const long long *kb = c.kap + 3 * g;
-                            dE = dE + interval_flip_cost(c.lam[g], ca, up, (long long)c.Mcol[g * c.mstride] + kb[0], kb[1], kb[2]);
-                        } else {
-                            const long long t = (long long)ca * ((long long)ca - (up ? 1 : -1) * ((long long)c.Mcol[g * c.mstride] + c.kap[g]));
-                            dE = dE + c.lam[g] * (double)t;
-                        }
+                        dE = dE + rp_group_flip_cost<GROUPS>(c, g, ca, up);
                     }
                 }
                 const bool cand = active && !(dE >= thr);
@@ -540,7 +547,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 if (acc) {
                     c.st.acc++;
                     c.st.nbr += (unsigned long long)(ra >> 16);
-                    if (GROUPS) {
+                    if (GROUPS != GK_NONE) {
                         if (g != 255) c.Mcol[g * c.mstride] -= 2 * ca * (up ? 1 : -1);
                     }
                 }
@@ -627,22 +634,12 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 const bool up = (W & db) == 0u;
                 double dE = up ? -2.0 * fv : 2.0 * fv;
                 int g = 255, ca = 0;
-                if (GROUPS) {
+                if (GROUPS != GK_NONE) {
                     const int ga = (int)lds_u32(hdr + RP_H_GA + 4u * (uint32_t)i);
                     g = ga & 255;
                     if (g != 255) {
                         ca = ga >> 8;
-                        if (GROUPS == 1) {
-                            const int m = c.Mcol[g * c.mstride] + reinterpret_cast<const int *>(c.kap)[2 * g];
-                            const int t = ca * (ca - (up ? m : -m));
-                            dE = dE + c.lam[g] * (double)t;
-                        } else if (GROUPS == 3) {
-                            const long long *kb = c.kap + 3 * g;
-                            dE = dE + interval_flip_cost(c.lam[g], ca, up, (long long)c.Mcol[g * c.mstride] + kb[0], kb[1], kb[2]);
-                        } else {
-                            const long long t = (long long)ca * ((long long)ca - (up ? 1 : -1) * ((long long)c.Mcol[g * c.mstride] + c.kap[g]));
-                            dE = dE + c.lam[g] * (double)t;
-                        }
+                        dE = dE + rp_group_flip_cost<GROUPS>(c, g, ca, up);
                     }
                 }
                 const bool cand = active && !(dE >= thr);
@@ -676,7 +673,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                     W ^= db;
                     c.st.acc++;
                     c.st.nbr += (unsigned long long)(ra >> 16);
-                    if (GROUPS) {
+                    if (GROUPS != GK_NONE) {
                         if (g != 255) c.Mcol[g * c.mstride] -= 2 * ca * (up ? 1 : -1);
                     }
                 }
@@ -702,7 +699,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
 // loops.
 template <int SLOTS>
 __device__ __noinline__ uint32_t rp_setup_pass(RpCtx c) {
-    rp_pass<3, 0, SLOTS>(c, 1.0, true);
+    rp_pass<3, GK_NONE, SLOTS>(c, 1.0, true);
     return c.gb;
 }
 
@@ -732,20 +729,20 @@ __device__ __forceinline__ double rp_field_direct(const ProblemDesc &D, const ui
 // the shared window (so that a slot address is formed by OR), one slot region per warp, then one partial-sum region per warp.
 // `smem_base` is the shared-window offset of the dynamic allocation (1 KB on sm_100: the system-reserved bytes); the kernel
 // verifies the assumption.
-__host__ __device__ inline size_t rp_fixed_bytes(int nw, int max_groups, bool interval = false) {
+__host__ __device__ inline size_t rp_fixed_bytes(int nw, int max_groups, GroupKind gk) {
     size_t b = (size_t)RP_STAGES * RP_STAGE_BYTES + 8 * (2 * RP_STAGES) + 32;
-    b += (sizeof(double) + (interval ? 3 : 1) * sizeof(long long)) * (size_t)max_groups;   // interval: {kappa, lo, hi}
+    b += (sizeof(double) + kappa_words(gk) * sizeof(long long)) * (size_t)max_groups;
     b += sizeof(int) * (size_t)max_groups * nw * 32;
     return b;
 }
-__host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned smem_base, int slots, bool interval = false) {
-    const size_t fixed = rp_fixed_bytes(nw, max_groups, interval);
+__host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned smem_base, int slots, GroupKind gk) {
+    const size_t fixed = rp_fixed_bytes(nw, max_groups, gk);
     const size_t sf = (size_t)rp_sf_bytes(slots);
     const size_t pad = (sf - (smem_base + fixed) % sf) % sf;
     return fixed + pad + (size_t)nw * (sf + RP_PS_BYTES);
 }
 
-template <int GROUPS, int SLOTS, bool KWAY>
+template <GroupKind GROUPS, int SLOTS, bool KWAY>
 __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_replay(AnnealParams P) {
     constexpr uint32_t RP_SF_BYTES = (uint32_t)rp_sf_bytes(SLOTS);
     extern __shared__ __align__(16) unsigned char rp_raw[];
@@ -754,7 +751,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     const int NW = blockDim.x >> 5;
     uint32_t raw_s;   // opaque to the compiler: it would otherwise re-derive the window address (S2R + LEA) inside the hot loops
     asm volatile("mov.u32 %0, %1;" : "=r"(raw_s) : "r"((uint32_t)__cvta_generic_to_shared(rp_raw)));
-    const uint32_t fixed = (uint32_t)rp_fixed_bytes(NW, P.max_groups, GROUPS == 3);
+    const uint32_t fixed = (uint32_t)rp_fixed_bytes(NW, P.max_groups, GROUPS);
     const uint32_t base_s = (raw_s + fixed + (uint32_t)RP_SF_BYTES - 1u) & ~((uint32_t)RP_SF_BYTES - 1u);    // warp regions
     {
         uint32_t dyn;
@@ -774,7 +771,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     unsigned *acc_sh = reinterpret_cast<unsigned *>(tail + 8 * (2 * RP_STAGES) + 16);   // [2]
     double *lam_sh = reinterpret_cast<double *>(tail + 8 * (2 * RP_STAGES) + 32);
     long long *kap_sh = reinterpret_cast<long long *>(lam_sh + P.max_groups);
-    int *M_all = reinterpret_cast<int *>(kap_sh + (GROUPS == 3 ? 3 : 1) * P.max_groups);
+    int *M_all = reinterpret_cast<int *>(kap_sh + kappa_words(GROUPS) * P.max_groups);
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < RP_STAGES; ++s) {
@@ -786,19 +783,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
         acc_sh[1] = 0u;
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (GROUPS) {  // groups exist only on single-problem models: one copy of lambda / kappa per block
-        const ProblemDesc &D0 = P.descs[0];
-        for (int g = threadIdx.x; g < D0.ngroups; g += blockDim.x) {
-            lam_sh[g] = D0.lambda[g];
-            if (GROUPS == 3) {
-                kap_sh[3 * g] = D0.kappa[g];
-                kap_sh[3 * g + 1] = D0.kappa[D0.ngroups + g];
-                kap_sh[3 * g + 2] = D0.kappa[2 * D0.ngroups + g];
-            } else {
-                kap_sh[g] = D0.kappa[g];
-            }
-        }
-    }
+    if (GROUPS != GK_NONE) stage_group_params<GROUPS>(P.descs[0], lam_sh, kap_sh);
     __syncthreads();
 
     RpCtx c;
@@ -888,7 +873,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
                 __stcg(c.SF + (int64_t)hw * 32, w);
             }
         }
-        if (GROUPS) {
+        if (GROUPS != GK_NONE) {
             for (int g = 0; g < D.ngroups; ++g) c.Mcol[g * c.mstride] = 0;
             for (int hw = 0; hw < nhw; ++hw) {
                 const uint32_t w = __ldcg(c.SF + (int64_t)hw * 32);
@@ -947,7 +932,7 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
                         acc_par ^= 1;
                         if (tot * 1000ull < (unsigned long long)P.switch_permille * (unsigned long long)n * (unsigned long long)cta_reads) {
                             RP_CLK(t_cu);
-                            rp_pass<1, 0, SLOTS>(c, beta, true);
+                            rp_pass<1, GK_NONE, SLOTS>(c, beta, true);
                             RP_PROF(7, clock64() - t_cu);
                             push = true;
                         }
@@ -987,19 +972,9 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
             }
         }
     }
-    // warp-reduce the per-lane counters
-    unsigned long long v[5] = {c.st.cand, c.st.draws, c.st.acc, c.st.ties, c.st.nbr};
-#pragma unroll
-    for (int q = 0; q < 5; ++q)
-        for (int off = 16; off > 0; off >>= 1) v[q] += __shfl_xor_sync(FULL_MASK, v[q], off);
-    if (lane == 0) {
-        atomicAdd(P.stats + ST_CAND, v[0]);
-        atomicAdd(P.stats + ST_DRAWS, v[1]);
-        atomicAdd(P.stats + ST_ACC, v[2]);
-        atomicAdd(P.stats + ST_TIES, v[3]);
-        atomicAdd(P.stats + ST_NBR, v[4]);
+    flush_lane_stats(P, c.st);
 #ifdef QA_RP_PROFILE
+    if (lane == 0)
         for (int k = 0; k < QA_NDEBUG; ++k) atomicAdd(P.stats + QA_NSTAT + 1 + k, (unsigned long long)c.prof[k]);
 #endif
-    }
 }
