@@ -70,6 +70,24 @@ extern "C" {
 #define QA_KERNEL_DENSE 5          /* QA_MODE_THROUGHPUT on a model with the dense k-way form (qa_model_enable_dense):
                                       local fields of 8-cell blocks by fp64 tensor-core MMAs (DMMA) over all cells */
 
+/* var_order / proposal (qa_sa_sample_model_ex, qa_sa_sample_ising_ex): dwave-samplers >= 1.0's sample options
+ * randomize_order and proposal_acceptance_criteria, as SURVEY.md Appendix C.8 recalls its cpu_sa.cpp (not pinned against the
+ * package).  Per beta thr = 44.36142 / beta; per attempt:
+ *   QA_ORDER_SEQUENTIAL      attempt k of a sweep visits variable k (neal)
+ *   QA_ORDER_RANDOM          attempt k visits v = r % n (unsigned 64-bit) for r = the read's next xorshift128+ output, drawn
+ *                            before anything else; still n attempts per sweep
+ *   QA_PROPOSAL_METROPOLIS   skip if dE >= thr; accept if dE <= 0; else draw r, accept iff exp(-dE*beta) * 2^64 > (double)r
+ *   QA_PROPOSAL_GIBBS        skip if dE >= thr; accept if dE <= -thr; else draw r, accept iff 2^64 > (double)r * (1 + exp(dE*beta))
+ * dE includes the rank-1 group terms.  Every combination is bit-exact against the CPU reference of the tests
+ * (tests/native/proposals_sa_ref.cpp, which at the defaults reproduces the oracle bit for bit).
+ * Kernels: random order always runs QA_KERNEL_WARP_PER_READ, whatever qa_ctx_set_kernel asked for (the lockstep and replay
+ * kernels walk 32 reads through one shared variable order).  Sequential Gibbs runs the kernel the usual rules pick, except
+ * that QA_MODE_THROUGHPUT never picks QA_KERNEL_DENSE: with either option the tensor-core kernel is not used. */
+#define QA_ORDER_SEQUENTIAL 0
+#define QA_ORDER_RANDOM 1
+#define QA_PROPOSAL_METROPOLIS 0
+#define QA_PROPOSAL_GIBBS 1
+
 #define QA_MAX_GROUPS 64
 
 typedef struct qa_ctx qa_ctx;
@@ -78,13 +96,14 @@ typedef struct qa_model qa_model;
 /* Counters and device-side phase timings (CUDA events on the context's stream). */
 typedef struct qa_stats {
     uint64_t attempts;      /* n * num_sweeps * num_reads */
-    uint64_t candidates;    /* attempts with dE <  44.36142/beta  (reached the accept test) */
-    uint64_t draws;         /* xorshift128+ outputs consumed (0 < dE < threshold) */
+    uint64_t candidates;    /* attempts with dE <  44.36142/beta  (reached the accept test; Gibbs too) */
+    uint64_t draws;         /* xorshift128+ outputs consumed: accept draws (Metropolis 0 < dE < thr, Gibbs -thr < dE < thr)
+                               and, with QA_ORDER_RANDOM, one order draw per attempt */
     uint64_t accepted;      /* spin flips performed */
     uint64_t nbr_updates;   /* sum of deg(v) over accepted flips */
-    uint64_t active_chunks; /* 32-variable chunks that had >= 1 candidate */
-    uint64_t chunks;        /* 32-variable chunks streamed */
-    uint64_t near_ties;     /* accept tests decided by < 2^-48 relative margin */
+    uint64_t active_chunks; /* 32-variable chunks that had >= 1 candidate (0 under QA_ORDER_RANDOM) */
+    uint64_t chunks;        /* 32-variable chunks streamed (0 under QA_ORDER_RANDOM) */
+    uint64_t near_ties;     /* accept tests decided by < 2^-48 relative margin (Gibbs: |2^64 - r (1 + exp)| <= 2^16) */
     double ms_h2d;          /* host->device copies (0 when inputs are device resident) */
     double ms_build;        /* CSR construction */
     double ms_anneal;       /* annealing kernel(s) */
@@ -156,6 +175,14 @@ int qa_sa_sample_model(qa_ctx *ctx, qa_model *model, int32_t num_reads, int8_t *
                        int32_t mode, qa_interrupt_fn interrupt, void *interrupt_user,
                        qa_stats *stats_out);
 
+/* qa_sa_sample_model with dwave-samplers' variable order and acceptance rule (QA_ORDER_*, QA_PROPOSAL_*; any other value:
+ * QA_ERR_ARG).  (QA_ORDER_SEQUENTIAL, QA_PROPOSAL_METROPOLIS) is qa_sa_sample_model. */
+int qa_sa_sample_model_ex(qa_ctx *ctx, qa_model *model, int32_t num_reads, int8_t *states_inout,
+                          double *energies_out, int32_t num_betas, const double *beta_schedule,
+                          int32_t sweeps_per_beta, const uint64_t *seeds, int32_t seed_mode,
+                          int32_t mode, int32_t var_order, int32_t proposal, qa_interrupt_fn interrupt,
+                          void *interrupt_user, qa_stats *stats_out);
+
 /* One-shot form mirroring neal's general_simulated_annealing, argument for argument (model built and freed inside):
  * interrupt / interrupt_user are neal's interrupt_callback / interrupt_function (may be NULL); the return value is the number
  * of reads completed. */
@@ -165,13 +192,21 @@ int qa_sa_sample_ising(qa_ctx *ctx, int32_t n, const double *h, int64_t m, const
                        const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
                        int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *interrupt_user,
                        qa_stats *stats_out);
+/* The same for dwave-samplers >= 1.0's general_simulated_annealing, which takes varorder and proposal_acceptance_criteria
+ * after the seed and before the interrupt callback (that argument order is recalled, not verified against the package). */
+int qa_sa_sample_ising_ex(qa_ctx *ctx, int32_t n, const double *h, int64_t m, const int32_t *starts,
+                          const int32_t *ends, const double *weights, int32_t num_reads,
+                          int8_t *states_inout, double *energies_out, int32_t num_betas,
+                          const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
+                          int32_t seed_mode, int32_t mode, int32_t var_order, int32_t proposal,
+                          qa_interrupt_fn interrupt, void *interrupt_user, qa_stats *stats_out);
 
 /* Many independent problems in one launch (QA_subsampling.py:24 called per sub-graph).
  * Problem p owns variables [var_offsets[p], var_offsets[p+1]) of h and couplers
  * [coupler_offsets[p], coupler_offsets[p+1]) (indices local to the problem); every problem
  * runs reads_per_problem reads.  states: [num_problems][reads_per_problem][n_p] packed
  * back to back in problem order; energies: [num_problems][reads_per_problem];
- * seeds: [num_problems * reads_per_problem] (per-read seeding only). */
+ * seeds: [num_problems * reads_per_problem] (per-read seeding only).  Sequential order, Metropolis acceptance. */
 int qa_sa_sample_ising_batch(qa_ctx *ctx, int32_t num_problems, const int64_t *var_offsets,
                              const int64_t *coupler_offsets, const double *h, const int32_t *starts,
                              const int32_t *ends, const double *weights, int32_t reads_per_problem,

@@ -26,6 +26,10 @@ QA_KERNEL_LOCKSTEP_PUSH = 2
 QA_KERNEL_LOCKSTEP_PULL = 3
 QA_KERNEL_REPLAY = 4
 QA_KERNEL_DENSE = 5
+QA_ORDER_SEQUENTIAL = 0
+QA_ORDER_RANDOM = 1
+QA_PROPOSAL_METROPOLIS = 0
+QA_PROPOSAL_GIBBS = 1
 QA_MAX_GROUPS = 64
 
 ERROR_NAMES = {
@@ -98,7 +102,10 @@ SIGNATURES = {
     "qa_model_get_ising": (C.c_int, [_p, _p, _p, _p, _p]),
     "qa_model_destroy": (C.c_int, [_p]),
     "qa_sa_sample_model": (C.c_int, [_p, _p, _i32, _p, _p, _i32, _p, _i32, _p, _i32, _i32, _p, _p, C.POINTER(QAStats)]),
+    "qa_sa_sample_model_ex": (C.c_int, [_p, _p, _i32, _p, _p, _i32, _p, _i32, _p, _i32, _i32, _i32, _i32, _p, _p, C.POINTER(QAStats)]),
     "qa_sa_sample_ising": (C.c_int, [_p, _i32, _p, _i64, _p, _p, _p, _i32, _p, _p, _i32, _p, _i32, _p, _i32, _i32, _p, _p, C.POINTER(QAStats)]),
+    "qa_sa_sample_ising_ex": (C.c_int, [_p, _i32, _p, _i64, _p, _p, _p, _i32, _p, _p, _i32, _p, _i32, _p, _i32, _i32, _i32, _i32, _p, _p,
+                                        C.POINTER(QAStats)]),
     "qa_sa_sample_ising_batch": (C.c_int, [_p, _i32, _p, _p, _p, _p, _p, _p, _i32, _p, _p, _i32, _p, _i32, _p, C.POINTER(QAStats)]),
     "qa_build_cut_balance": (C.c_int, [_p, _i32, _i64, _p, _p, _p, C.c_double, C.c_double, C.POINTER(_p), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "qa_build_cut_linear": (C.c_int, [_p, _i32, _i64, _p, _p, _p, C.c_double, C.c_double, C.POINTER(_p), C.POINTER(C.c_double), C.POINTER(C.c_double)]),

@@ -83,9 +83,10 @@ enum LsPass { LS_PUSH, LS_FIELD_SETUP };
 // LS_PUSH: the whole schedule of push sweeps (bit-exact).  LS_FIELD_SETUP: one pass that only evaluates the local fields
 // from the spins and stores them (neal get_flip_energy order), before the push sweeps.
 // GROUPS: GK_NONE, GK_EQ64 (equality groups of both widths) or GK_INTERVAL (kap_sh then holds {kappa, lo, hi} per group).
+// PROP: the acceptance rule of the push sweeps (the set-up pass decides nothing).
 // The loop counters bi / swi are the caller's variables, both 0 on entry: with counters local to this function nvcc orders
 // a few instructions of the kernel differently, and the kernel's measured numbers (DESIGN.md 4.2) are for this SASS.
-template <LsPass PASS, GroupKind GROUPS>
+template <LsPass PASS, GroupKind GROUPS, Proposal PROP>
 __device__ void ls_sweeps(const LsCtx &c, int &bi, int &swi, unsigned long long &s0, unsigned long long &s1, LaneStats &st) {
     const ProblemDesc &D = c.D;
     const AnnealParams &P = c.P;
@@ -267,7 +268,7 @@ __device__ void ls_sweeps(const LsCtx &c, int &bi, int &swi, unsigned long long 
                     const bool cand = active && !(dE >= thr);
                     if (!__any_sync(FULL_MASK, cand)) continue;
                     if (cand) st.cand++;
-                    const bool acc = ls_accept(dE, cand, beta, s0, s1, st);
+                    const bool acc = accept_test<PROP>(dE, cand, beta, thr, s0, s1, st);
                     const unsigned accm = __ballot_sync(FULL_MASK, acc);
                     if (accm == 0) continue;
                     if (acc) {
@@ -338,7 +339,7 @@ __device__ void ls_sweeps(const LsCtx &c, int &bi, int &swi, unsigned long long 
     __syncwarp();
 }
 
-template <GroupKind GROUPS>
+template <GroupKind GROUPS, Proposal PROP>
 __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned long long &s1, LaneStats &st, int *error_flag) {
     const ProblemDesc &D = c.D;
     const int n = D.n;
@@ -376,8 +377,8 @@ __device__ void lockstep_tile(const LsCtx &c, unsigned long long &s0, unsigned l
         }
     }
     int setup_bi = 0, setup_swi = 0, bi = 0, swi = 0;
-    ls_sweeps<LS_FIELD_SETUP, GK_NONE>(c, setup_bi, setup_swi, s0, s1, st);  // local fields from the current spins
-    ls_sweeps<LS_PUSH, GROUPS>(c, bi, swi, s0, s1, st);
+    ls_sweeps<LS_FIELD_SETUP, GK_NONE, PROP>(c, setup_bi, setup_swi, s0, s1, st);  // local fields from the current spins
+    ls_sweeps<LS_PUSH, GROUPS, PROP>(c, bi, swi, s0, s1, st);
 
     // ---- final spins back to the caller's +-1 rows
     if (c.active) {
@@ -398,7 +399,7 @@ __host__ __device__ inline size_t ls_smem_bytes(int max_groups, GroupKind gk) {
     return b;
 }
 
-template <GroupKind GROUPS>
+template <GroupKind GROUPS, Proposal PROP>
 __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P) {
     extern __shared__ __align__(16) unsigned char ls_smem[];
     // layout: [cur: D x TPB doubles, aliased by the spin words] [LsStage x warps] [LsSetupStage x warps] [lambda] [kappa] [M]
@@ -439,7 +440,7 @@ __global__ void __launch_bounds__(QA_LS_TPB, 3) k_anneal_lockstep(AnnealParams P
         unsigned long long s0 = sd ? sd : ~0ull, s1 = 0;
         const LsCtx c = {D, P, r, active, fT, M_all + threadIdx.x, cur_all + wib * (QA_LS_D * 32) + lane, stages[wib],
                          setup_stages[wib], words_all + wib * (QA_LS_CAPW * 32) + lane, lam_sh, kap_sh};
-        lockstep_tile<GROUPS>(c, s0, s1, st, P.error_flag);
+        lockstep_tile<GROUPS, PROP>(c, s0, s1, st, P.error_flag);
     }
     flush_lane_stats(P, st);
 }
@@ -528,8 +529,13 @@ int launch_lockstep(Launch &L) {
     const int64_t total_tiles = (int64_t)A.num_problems * tpp;
     const size_t smem = ls_smem_bytes(std::max(M->ngroups, 1), L.gk);
     // EQ32 models run the 64-bit instance: this kernel has no 32-bit one
-    const void *fn = L.gk == GK_NONE ? (const void *)k_anneal_lockstep<GK_NONE>
-                   : L.gk == GK_INTERVAL ? (const void *)k_anneal_lockstep<GK_INTERVAL> : (const void *)k_anneal_lockstep<GK_EQ64>;
+    const void *fn = L.prop == PROP_GIBBS
+                         ? (L.gk == GK_NONE ? (const void *)k_anneal_lockstep<GK_NONE, PROP_GIBBS>
+                            : L.gk == GK_INTERVAL ? (const void *)k_anneal_lockstep<GK_INTERVAL, PROP_GIBBS>
+                                                  : (const void *)k_anneal_lockstep<GK_EQ64, PROP_GIBBS>)
+                         : (L.gk == GK_NONE ? (const void *)k_anneal_lockstep<GK_NONE, PROP_METROPOLIS>
+                            : L.gk == GK_INTERVAL ? (const void *)k_anneal_lockstep<GK_INTERVAL, PROP_METROPOLIS>
+                                                  : (const void *)k_anneal_lockstep<GK_EQ64, PROP_METROPOLIS>);
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, QA_LS_TPB, smem, cudaOccupancyDefault));

@@ -7,6 +7,8 @@
 //   * the 32 lanes of a chunk decide "candidate" (dE < 44.36142/beta) in parallel; candidates are then resolved in variable
 //     order with a warp-uniform xorshift128+ stream, so the sequence of RNG draws, accepts and fp64 roundings is exactly neal's.
 //   * persistent grid (multiple of the SM count), reads pulled from an atomic counter; only resident warps own fp64 scratch.
+//   * dwave-samplers >= 1.0's sample options (include/qanneal.h): Gibbs acceptance in the chunked loop, and a random-order
+//     loop of its own (random_order_sweeps) -- the only kernel that runs random order.
 #include "device_common.cuh"
 
 using namespace qa;
@@ -14,10 +16,85 @@ using namespace qa;
 namespace {
 
 // ------------------------------------------------------------------------------------------------
+// random variable order (dwave-samplers randomize_order=True): per attempt one warp-uniform xorshift128+ draw picks
+// v = r % n, then the decision of v as in the chunked loop -- every lane computes it from the same loads and the same RNG
+// state, so it is warp-uniform without a shuffle.  There is no chunk register cache: f[v] and the spin word are read from
+// the read's scratch at every attempt, and an accepted flip's neighbour reductions are ordered before the next attempt's
+// loads by __syncwarp (the next v may be a neighbour just pushed).
+// ------------------------------------------------------------------------------------------------
+template <GroupKind GROUPS, Proposal PROP>
+__device__ void random_order_sweeps(const ProblemDesc &D, const AnnealParams &P, double *__restrict__ f,
+                                    uint32_t *__restrict__ spw, unsigned long long &s0, unsigned long long &s1, long long *Mw,
+                                    WarpStats &st) {
+    const int lane = threadIdx.x & 31;
+    const int n = D.n;
+    for (int b = 0; b < P.num_betas; ++b) {
+        const double beta = (D.betas ? D.betas : P.betas)[b];
+        const double thr = 44.36142 / beta;
+        for (int sw = 0; sw < P.sweeps_per_beta; ++sw) {
+            for (int k = 0; k < n; ++k) {
+                const int v = (int)(rng_next(s0, s1) % (unsigned long long)n);   // the order draw comes first
+                st.draws++;
+                const double fv = __ldcg(f + v);
+                const uint32_t wv = __ldcg(spw + (v >> 5));
+                const bool up = (wv >> (v & 31)) & 1u;
+                double dE = up ? -2.0 * fv : 2.0 * fv;
+                int g = -1;
+                long long a = 0;
+                if (GROUPS != GK_NONE) {
+                    g = __ldg(D.grp + v);
+                    if (g >= 0) {
+                        a = __ldg(D.coef + v);
+                        const long long kap = __ldg(D.kappa + g);
+                        long long glo = 0, ghi = 0;
+                        if (GROUPS == GK_INTERVAL) {
+                            glo = __ldg(D.kappa + D.ngroups + g);
+                            ghi = __ldg(D.kappa + 2 * D.ngroups + g);
+                        }
+                        dE = dE + group_flip_cost<GROUPS>(__ldg(D.lambda + g), a, up, Mw[g] + kap, glo, ghi);
+                    }
+                }
+                if (dE >= thr) continue;
+                st.cand++;
+                bool acc = true;
+                if (PROP == PROP_GIBBS ? !(dE <= -thr) : dE > 0.0) {
+                    const double rd = __ull2double_rn(rng_next(s0, s1));
+                    st.draws++;
+                    if (PROP == PROP_GIBBS) {
+                        const double q = rd * (1.0 + exp(dE * beta));
+                        acc = QA_TWO64 > q;
+                        if (fabs(QA_TWO64 - q) <= QA_TWO64 * 3.5527136788005009e-15) st.ties++;
+                    } else {
+                        const double p = exp(-dE * beta) * QA_TWO64;
+                        acc = p > rd;
+                        if (fabs(p - rd) <= p * 3.5527136788005009e-15) st.ties++;
+                    }
+                }
+                if (!acc) continue;
+                st.acc++;
+                const int r0 = __ldg(D.rowptr + v), r1 = __ldg(D.rowptr + v + 1);
+                const double cf = up ? -2.0 : 2.0;  // f[j] += -2*s_v*J  <=> dE[j] += 4*s_v*J*s_j
+                st.nbr += (unsigned long long)(r1 - r0);
+                for (int e = r0 + lane; e < r1; e += 32) red_add_f64(f + __ldg(D.col + e), cf * __ldg(D.val + e));
+                __syncwarp();   // every lane has read spw / Mw of this attempt before lane 0 changes them
+                if (lane == 0) {
+                    __stcg(spw + (v >> 5), wv ^ (1u << (v & 31)));
+                    if (GROUPS != GK_NONE) {
+                        if (g >= 0) Mw[g] -= 2 * a * (up ? 1 : -1);
+                    }
+                }
+                __syncwarp();   // the reductions and lane 0's stores before the next attempt's loads
+            }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // one read, reference order.  Restates neal simulated_annealing_run() for one `state`.
 // ------------------------------------------------------------------------------------------------
-// GROUPS: GK_NONE, GK_EQ64 (equality groups of both widths) or GK_INTERVAL; lambda / kappa / bounds are read per problem
-template <GroupKind GROUPS>
+// GROUPS: GK_NONE, GK_EQ64 (equality groups of both widths) or GK_INTERVAL; lambda / kappa / bounds are read per problem.
+// PROP: the acceptance rule.  RANDOM: random variable order (random_order_sweeps) instead of the chunked sequential loop.
+template <GroupKind GROUPS, Proposal PROP, bool RANDOM>
 __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t r_local, double *__restrict__ f,
                             uint32_t *__restrict__ spw, unsigned long long &s0, unsigned long long &s1,
                             long long *Mw, WarpStats &st, int *error_flag) {
@@ -76,8 +153,9 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
     }
     __syncwarp();
 
-    // ---- the anneal: for beta: for sweep: for var (neal order)
-    for (int b = 0; b < P.num_betas; ++b) {
+    // ---- the anneal: for beta: for sweep: for var (neal order; random order: random_order_sweeps, and no chunked sweep)
+    if (RANDOM) random_order_sweeps<GROUPS, PROP>(D, P, f, spw, s0, s1, Mw, st);
+    for (int b = 0; b < (RANDOM ? 0 : P.num_betas); ++b) {
         const double beta = (D.betas ? D.betas : P.betas)[b];
         const double thr = 44.36142 / beta;
         for (int sw = 0; sw < P.sweeps_per_beta; ++sw) {
@@ -135,19 +213,29 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
                         st.cand++;
                         const double dEl = __shfl_sync(FULL_MASK, dE, l);
                         bool acc = true;
-                        if (dEl > 0.0) {
+                        if (PROP == PROP_GIBBS ? !(dEl <= -thr) : dEl > 0.0) {
                             const uint32_t pv = __ballot_sync(FULL_MASK, pvalid);
                             if (!((pv >> l) & 1u)) {
-                                // exp(-dE*beta)*2^64 for every lane that may need it (one SIMT pass)
-                                if (!pvalid && cand && dE > 0.0) p = exp(-dE * beta) * QA_TWO64;
+                                // exp(-dE*beta)*2^64 (Gibbs: 1 + exp(dE*beta)) for every lane that may need it (one SIMT pass)
+                                if (PROP == PROP_GIBBS) {
+                                    if (!pvalid && cand && !(dE <= -thr)) p = 1.0 + exp(dE * beta);
+                                } else {
+                                    if (!pvalid && cand && dE > 0.0) p = exp(-dE * beta) * QA_TWO64;
+                                }
                                 pvalid = true;
                             }
                             const unsigned long long rnd = rng_next(s0, s1);
                             st.draws++;
                             const double pl = __shfl_sync(FULL_MASK, p, l);
                             const double rd = __ull2double_rn(rnd);
-                            acc = pl > rd;  // neal: exp(-dE*beta) * RANDMAX > rand
-                            if (fabs(pl - rd) <= pl * 3.5527136788005009e-15) st.ties++;
+                            if (PROP == PROP_GIBBS) {
+                                const double q = rd * pl;
+                                acc = QA_TWO64 > q;  // dwave-samplers Gibbs: 1 / (1 + exp(dE*beta)) > rand / 2^64
+                                if (fabs(QA_TWO64 - q) <= QA_TWO64 * 3.5527136788005009e-15) st.ties++;
+                            } else {
+                                acc = pl > rd;  // neal: exp(-dE*beta) * RANDMAX > rand
+                                if (fabs(pl - rd) <= pl * 3.5527136788005009e-15) st.ties++;
+                            }
                         }
                         if (acc) {
                             st.acc++;
@@ -214,7 +302,7 @@ __device__ void anneal_read(const ProblemDesc &D, const AnnealParams &P, int64_t
     for (int c = lane; c < nch; c += 32) D.packedT[(int64_t)c * D.rpad + r_local] = __ldcg(spw + c);
 }
 
-template <GroupKind GROUPS>
+template <GroupKind GROUPS, Proposal PROP, bool RANDOM>
 __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
     __shared__ long long Msh[GROUPS != GK_NONE ? (QA_TPB_MAX / 32) * QA_MAX_GROUPS : 1];
     __shared__ unsigned long long next_read[QA_TPB_MAX / 32];
@@ -233,7 +321,7 @@ __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
         for (int64_t r = P.read_begin; r < P.read_end; ++r) {
             const int p = (int)(r / P.reads_per_problem);
             const ProblemDesc D = P.descs[p];
-            anneal_read<GROUPS>(D, P, r - D.read_base, f, spw, s0, s1, Mw, st, P.error_flag);
+            anneal_read<GROUPS, PROP, RANDOM>(D, P, r - D.read_base, f, spw, s0, s1, Mw, st, P.error_flag);
         }
     } else {
         for (;;) {
@@ -246,7 +334,7 @@ __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
             const ProblemDesc D = P.descs[p];
             const unsigned long long sd = P.seeds[r];
             unsigned long long s0 = sd ? sd : ~0ull, s1 = 0;  // neal: rng_state = {seed ? seed : RANDMAX, 0}
-            anneal_read<GROUPS>(D, P, r - D.read_base, f, spw, s0, s1, Mw, st, P.error_flag);
+            anneal_read<GROUPS, PROP, RANDOM>(D, P, r - D.read_base, f, spw, s0, s1, Mw, st, P.error_flag);
         }
     }
     if (lane == 0) {
@@ -260,13 +348,25 @@ __global__ void __launch_bounds__(QA_TPB_MAX, 4) k_anneal_ref(AnnealParams P) {
     }
 }
 
+// EQ32 models run the 64-bit instance: this kernel has no 32-bit one
+template <Proposal PROP, bool RANDOM>
+void (*ref_instance(GroupKind gk))(AnnealParams) {
+    return gk == GK_NONE ? k_anneal_ref<GK_NONE, PROP, RANDOM>
+         : gk == GK_INTERVAL ? k_anneal_ref<GK_INTERVAL, PROP, RANDOM> : k_anneal_ref<GK_EQ64, PROP, RANDOM>;
+}
+
+void (*ref_kernel(GroupKind gk, Proposal prop, bool random_order))(AnnealParams) {
+    if (random_order) return prop == PROP_GIBBS ? ref_instance<PROP_GIBBS, true>(gk) : ref_instance<PROP_METROPOLIS, true>(gk);
+    return prop == PROP_GIBBS ? ref_instance<PROP_GIBBS, false>(gk) : ref_instance<PROP_METROPOLIS, false>(gk);
+}
+
 }  // namespace
 
 namespace qa {
 
 int ref_resident_reads(qa_ctx *ctx, int *out) {
     int bps = 0;
-    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<GK_NONE>, QA_TPB_MAX, 0));
+    QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_anneal_ref<GK_NONE, PROP_METROPOLIS, false>, QA_TPB_MAX, 0));
     *out = bps * ctx->num_sms * (QA_TPB_MAX / 32);
     return QA_OK;
 }
@@ -275,9 +375,7 @@ int launch_ref(Launch &L) {
     qa_ctx *ctx = L.ctx;
     AnnealParams &A = L.A;
     const int64_t total_reads = A.total_reads;
-    // EQ32 models run the 64-bit instance: this kernel has no 32-bit one
-    void (*const fn)(AnnealParams) = L.gk == GK_NONE ? k_anneal_ref<GK_NONE>
-                                   : L.gk == GK_INTERVAL ? k_anneal_ref<GK_INTERVAL> : k_anneal_ref<GK_EQ64>;
+    void (*const fn)(AnnealParams) = ref_kernel(L.gk, L.prop, L.random_order);
     const bool stream = A.seed_mode == QA_SEED_STREAM;
     // launch geometry: persistent grid, one warp per resident read
     int wpb = QA_TPB_MAX / 32;

@@ -327,21 +327,11 @@ int build_replay_tables(qa_model *M) {
     return QA_OK;
 }
 
-template <int SLOTS, bool KWAY>
-static const void *replay_instance(GroupKind gk) {
-    switch (gk) {
-    case GK_NONE: return (const void *)k_anneal_replay<GK_NONE, SLOTS, KWAY>;
-    case GK_EQ32: return (const void *)k_anneal_replay<GK_EQ32, SLOTS, KWAY>;
-    case GK_EQ64: return (const void *)k_anneal_replay<GK_EQ64, SLOTS, KWAY>;
-    default: return (const void *)k_anneal_replay<GK_INTERVAL, SLOTS, KWAY>;
-    }
-}
-
-// the instance for the model's group kind and slot count; models with k-way blocks run the one with the k-way batch phase
-static const void *replay_kernel(const qa_model *M, GroupKind gk) {
-    const bool kway = M->rp_kway_blocks > 0;
-    if (M->rp_slots == 32) return kway ? replay_instance<32, true>(gk) : replay_instance<32, false>(gk);
-    return kway ? replay_instance<64, true>(gk) : replay_instance<64, false>(gk);
+// the instance for the acceptance rule, the model's group kind and slot count; models with k-way blocks run the one with the
+// k-way batch phase.  The Gibbs instances live in their own translation unit (anneal_replay_gibbs.cu): this one's module
+// holds exactly the Metropolis instances, and the two compile in parallel.
+static const void *replay_kernel(const qa_model *M, GroupKind gk, Proposal prop) {
+    return prop == PROP_GIBBS ? replay_gibbs_kernel(M, gk) : replay_instance<PROP_METROPOLIS>(M, gk);
 }
 
 int launch_replay(Launch &L) {
@@ -367,7 +357,7 @@ int launch_replay(Launch &L) {
     const int64_t gpp = (tpp + nw - 1) / nw;
     const int64_t total_items = (int64_t)P * gpp;
     size_t smem = rp_smem_bytes(nw, mg, ctx->rp_smem_base, M->rp_slots, L.gk);
-    const void *fn = replay_kernel(M, L.gk);
+    const void *fn = replay_kernel(M, L.gk, L.prop);
     QA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int bps = 0;
     QA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessorWithFlags(&bps, fn, nw * 32, smem, cudaOccupancyDefault));

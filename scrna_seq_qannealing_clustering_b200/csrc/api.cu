@@ -27,10 +27,13 @@ int check_schedule(int32_t num_betas, const double *betas, int32_t sweeps_per_be
 
 // The annealing kernel of a call.  The rules, in order; the first that applies decides:
 //   1. DENSE          QA_MODE_THROUGHPUT on a model with the dense k-way form: one problem, per-read seeds, no interrupt
-//                     callback (the tensor-core kernel, tolerance parity).  Every other model runs a reference-order kernel:
+//                     callback, sequential order and Metropolis acceptance (the tensor-core kernel, tolerance parity; it has
+//                     neither dwave-samplers option).  Every other call runs a reference-order kernel:
 //                     for sparse models the exact replay kernel is faster than any recompute or graph-coloured update
 //                     (DESIGN.md 4.4), and bit-exact results meet the statistical bar trivially.
-//   2. WARP_PER_READ  stream seeding (one xorshift128+ stream across reads), and batched models with rank-1 groups
+//   2. WARP_PER_READ  random variable order, whatever kernel was requested: the lockstep and replay kernels walk all 32 reads
+//                     of a warp through the same variable, and random order has no order the reads share.
+//      WARP_PER_READ  stream seeding (one xorshift128+ stream across reads), and batched models with rank-1 groups
 //                     (qa_model_concat): the lockstep and replay kernels keep one copy of lambda / kappa per CTA, the
 //                     warp-per-read kernel reads them per problem.
 //   3. REPLAY         (deferred exact updates) when requested, or under AUTO from 32 reads per problem and 6144 reads in all
@@ -43,16 +46,18 @@ int check_schedule(int32_t num_betas, const double *betas, int32_t sweeps_per_be
 //   5. LOCKSTEP       when requested, or under AUTO from 32 reads per problem and 3.5 tiles of 32 reads per SM, without an
 //                     interrupt callback: the lockstep kernel has no stopping point.
 //   6. WARP_PER_READ  otherwise: any read count; with an interrupt callback it runs in read waves and polls between them.
+// Sequential Gibbs acceptance follows rules 2-6 unchanged: every reference-order kernel has both acceptance rules.
 int pick_kernel(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int64_t total_reads, int32_t seed_mode, int32_t mode,
-                bool interrupt, int *kernel) {
+                bool interrupt, int32_t var_order, int32_t proposal, int *kernel) {
     const int P = M->num_problems;
     const bool auto_ok = ctx->kernel == QA_KERNEL_AUTO && reads_per_problem >= 32;
-    if (mode == QA_MODE_THROUGHPUT && M->dn_ok && P == 1 && !interrupt && seed_mode == QA_SEED_PER_READ) {
+    if (mode == QA_MODE_THROUGHPUT && M->dn_ok && P == 1 && !interrupt && seed_mode == QA_SEED_PER_READ &&
+        var_order == QA_ORDER_SEQUENTIAL && proposal == QA_PROPOSAL_METROPOLIS) {
         *kernel = QA_KERNEL_DENSE;
         return QA_OK;
     }
     *kernel = QA_KERNEL_WARP_PER_READ;
-    if (seed_mode != QA_SEED_PER_READ || (P > 1 && M->ngroups > 0)) return QA_OK;
+    if (var_order == QA_ORDER_RANDOM || seed_mode != QA_SEED_PER_READ || (P > 1 && M->ngroups > 0)) return QA_OK;
     if ((ctx->kernel == QA_KERNEL_REPLAY || (auto_ok && total_reads >= 6144)) && (!interrupt || P == 1)) {
         const int rc = build_replay_tables(M);
         if (rc) return rc;
@@ -74,7 +79,8 @@ int pick_kernel(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int64_t tot
 // core: anneal all reads of all problems of a model; states/energies already on the device
 int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_states, double *d_energies,
                int32_t num_betas, const double *d_betas, int32_t sweeps_per_beta, const unsigned long long *d_seeds,
-               int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *iuser, qa_stats *st, int64_t *completed) {
+               int32_t seed_mode, int32_t mode, int32_t var_order, int32_t proposal, qa_interrupt_fn interrupt, void *iuser,
+               qa_stats *st, int64_t *completed) {
     const int P = M->num_problems;
     const int64_t total_reads = (int64_t)P * reads_per_problem;
     const int32_t rpad = (reads_per_problem + 31) & ~31;
@@ -105,7 +111,7 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
     }
 
     int kernel = 0;
-    rc = pick_kernel(ctx, M, reads_per_problem, total_reads, seed_mode, mode, interrupt != nullptr, &kernel);
+    rc = pick_kernel(ctx, M, reads_per_problem, total_reads, seed_mode, mode, interrupt != nullptr, var_order, proposal, &kernel);
     if (rc) return rc;
     ctx->last_kernel = kernel;
     QA_CUDA(cudaMemsetAsync(ctx->d_stats, 0, (QA_NSTAT + 1 + QA_NDEBUG) * sizeof(unsigned long long), ctx->stream));
@@ -132,6 +138,8 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
     L.M = M;
     L.A = A;
     L.gk = M->ngroups == 0 ? GK_NONE : M->gbounds ? GK_INTERVAL : M->groups_i32 ? GK_EQ32 : GK_EQ64;
+    L.prop = proposal == QA_PROPOSAL_GIBBS ? PROP_GIBBS : PROP_METROPOLIS;
+    L.random_order = var_order == QA_ORDER_RANDOM;
     L.interrupt = interrupt;
     L.iuser = iuser;
     L.st = st;
@@ -183,8 +191,11 @@ int run_anneal(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *d_st
 // stage caller buffers (host or device), run, and return results
 int sample_common(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *states_inout, double *energies_out,
                   int32_t num_betas, const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
-                  int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *iuser, qa_stats *stats_out) {
+                  int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *iuser, qa_stats *stats_out,
+                  int32_t var_order, int32_t proposal) {
     if (!ctx || !M) return fail(QA_ERR_ARG, "null context or model");
+    if (var_order != QA_ORDER_SEQUENTIAL && var_order != QA_ORDER_RANDOM) return fail(QA_ERR_ARG, "unknown var_order");
+    if (proposal != QA_PROPOSAL_METROPOLIS && proposal != QA_PROPOSAL_GIBBS) return fail(QA_ERR_ARG, "unknown proposal");
     if (M->ctx != ctx) return fail(QA_ERR_ARG, "model belongs to another context");
     if (reads_per_problem < 0) return fail(QA_ERR_ARG, "negative num_reads");
     if (mode != QA_MODE_REFERENCE && mode != QA_MODE_THROUGHPUT) return fail(QA_ERR_ARG, "unknown mode");
@@ -240,7 +251,7 @@ int sample_common(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *s
 
     int64_t completed = 0;
     rc = run_anneal(ctx, M, reads_per_problem, d_states, d_energies, num_betas, d_betas, sweeps_per_beta, d_seeds, seed_mode,
-                    mode, interrupt, iuser, &st, &completed);
+                    mode, var_order, proposal, interrupt, iuser, &st, &completed);
     if (rc) return rc;
 
     QA_CUDA(cudaEventRecord(ctx->ev[4], ctx->stream));
@@ -352,18 +363,37 @@ int qa_ctx_resident_reads(qa_ctx *ctx) {
     return rc ? rc : reads;
 }
 
+int qa_sa_sample_model_ex(qa_ctx *ctx, qa_model *model, int32_t num_reads, int8_t *states_inout, double *energies_out,
+                          int32_t num_betas, const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
+                          int32_t seed_mode, int32_t mode, int32_t var_order, int32_t proposal, qa_interrupt_fn interrupt,
+                          void *interrupt_user, qa_stats *stats_out) {
+    if (model && model->num_problems != 1) return fail(QA_ERR_ARG, "use qa_sa_sample_ising_batch for batched models");
+    return sample_common(ctx, model, num_reads, states_inout, energies_out, num_betas, beta_schedule, sweeps_per_beta, seeds,
+                         seed_mode, mode, interrupt, interrupt_user, stats_out, var_order, proposal);
+}
+
 int qa_sa_sample_model(qa_ctx *ctx, qa_model *model, int32_t num_reads, int8_t *states_inout, double *energies_out,
                        int32_t num_betas, const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
                        int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *interrupt_user, qa_stats *stats_out) {
-    if (model && model->num_problems != 1) return fail(QA_ERR_ARG, "use qa_sa_sample_ising_batch for batched models");
-    return sample_common(ctx, model, num_reads, states_inout, energies_out, num_betas, beta_schedule, sweeps_per_beta, seeds,
-                         seed_mode, mode, interrupt, interrupt_user, stats_out);
+    return qa_sa_sample_model_ex(ctx, model, num_reads, states_inout, energies_out, num_betas, beta_schedule, sweeps_per_beta,
+                                 seeds, seed_mode, mode, QA_ORDER_SEQUENTIAL, QA_PROPOSAL_METROPOLIS, interrupt, interrupt_user,
+                                 stats_out);
 }
 
 int qa_sa_sample_ising(qa_ctx *ctx, int32_t n, const double *h, int64_t m, const int32_t *starts, const int32_t *ends,
                        const double *weights, int32_t num_reads, int8_t *states_inout, double *energies_out, int32_t num_betas,
                        const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds, int32_t seed_mode,
                        int32_t mode, qa_interrupt_fn interrupt, void *interrupt_user, qa_stats *stats_out) {
+    return qa_sa_sample_ising_ex(ctx, n, h, m, starts, ends, weights, num_reads, states_inout, energies_out, num_betas,
+                                 beta_schedule, sweeps_per_beta, seeds, seed_mode, mode, QA_ORDER_SEQUENTIAL,
+                                 QA_PROPOSAL_METROPOLIS, interrupt, interrupt_user, stats_out);
+}
+
+int qa_sa_sample_ising_ex(qa_ctx *ctx, int32_t n, const double *h, int64_t m, const int32_t *starts, const int32_t *ends,
+                          const double *weights, int32_t num_reads, int8_t *states_inout, double *energies_out,
+                          int32_t num_betas, const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
+                          int32_t seed_mode, int32_t mode, int32_t var_order, int32_t proposal, qa_interrupt_fn interrupt,
+                          void *interrupt_user, qa_stats *stats_out) {
     if (!ctx) return fail(QA_ERR_ARG, "null context");
     cudaEvent_t b0 = nullptr, b1 = nullptr;
     QA_CUDA(cudaSetDevice(ctx->device));
@@ -376,7 +406,7 @@ int qa_sa_sample_ising(qa_ctx *ctx, int32_t n, const double *h, int64_t m, const
     cudaEventRecord(b1, ctx->stream);
     if (rc == QA_OK) {
         rc = sample_common(ctx, M, num_reads, states_inout, energies_out, num_betas, beta_schedule, sweeps_per_beta, seeds,
-                           seed_mode, mode, interrupt, interrupt_user, stats_out);
+                           seed_mode, mode, interrupt, interrupt_user, stats_out, var_order, proposal);
         if (rc >= 0 && stats_out) {
             cudaEventSynchronize(b1);
             stats_out->ms_build = elapsed(b0, b1);

@@ -5,6 +5,7 @@
 //   anneal_ref.cu       k_anneal_ref       one warp per read
 //   anneal_lockstep.cu  k_anneal_lockstep  32 reads per warp, eager updates
 //   anneal_replay.cu    k_anneal_replay    32 reads per warp, deferred exact updates (replay.cuh), slab packer
+//   anneal_replay_gibbs.cu                 its Gibbs-acceptance instances
 //   anneal_dense.cu     k_anneal_dense     dense k-way models on the fp64 tensor cores (dense.cuh)
 //   energy.cu           k_energy, k_pack_states
 //   builders.cu         qa_build_*          model builders on the device
@@ -285,6 +286,9 @@ __host__ __device__ __forceinline__ double interval_flip_cost(double lam, long l
 // annealing kernel.  EQ32: equality groups whose terms the host proved to fit 32-bit integers (qa_model::groups_i32).
 enum GroupKind { GK_NONE = 0, GK_EQ32 = 1, GK_EQ64 = 2, GK_INTERVAL = 3 };
 
+// Acceptance rule of a sampling call (QA_PROPOSAL_*), the PROP template argument of every annealing kernel but the dense one
+enum Proposal { PROP_METROPOLIS = QA_PROPOSAL_METROPOLIS, PROP_GIBBS = QA_PROPOSAL_GIBBS };
+
 // 64-bit words of kappa staged per group in shared memory: {kappa, lo, hi} for interval groups, kappa otherwise
 __host__ __device__ constexpr int kappa_words(GroupKind gk) { return gk == GK_INTERVAL ? 3 : 1; }
 
@@ -325,7 +329,8 @@ int model_create(qa_ctx *ctx, int32_t P, const int64_t *var_off, const int64_t *
 // api.cu
 int sample_common(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem, int8_t *states_inout, double *energies_out,
                   int32_t num_betas, const double *beta_schedule, int32_t sweeps_per_beta, const uint64_t *seeds,
-                  int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *iuser, qa_stats *stats_out);
+                  int32_t seed_mode, int32_t mode, qa_interrupt_fn interrupt, void *iuser, qa_stats *stats_out,
+                  int32_t var_order = QA_ORDER_SEQUENTIAL, int32_t proposal = QA_PROPOSAL_METROPOLIS);
 
 // one annealing launch: what run_anneal (api.cu) hands to the kernel's own translation unit
 struct Launch {
@@ -333,6 +338,8 @@ struct Launch {
     qa_model *M;
     AnnealParams A;        // also the launch's shape: reads_per_problem, total_reads, seed_mode
     GroupKind gk;
+    Proposal prop;         // acceptance rule
+    bool random_order;     // QA_ORDER_RANDOM (warp-per-read kernel only)
     qa_interrupt_fn interrupt;
     void *iuser;
     qa_stats *st;
@@ -343,6 +350,7 @@ int launch_ref(Launch &L);        // anneal_ref.cu
 int ref_resident_reads(qa_ctx *ctx, int *out);
 int launch_lockstep(Launch &L);   // anneal_lockstep.cu
 int launch_replay(Launch &L);     // anneal_replay.cu
+const void *replay_gibbs_kernel(const qa_model *M, GroupKind gk);   // anneal_replay_gibbs.cu
 int build_replay_tables(qa_model *M);
 int launch_dense(Launch &L);      // anneal_dense.cu
 int launch_energy(qa_ctx *ctx, qa_model *M, int32_t reads_per_problem);            // energy.cu: k_energy on the packed spins

@@ -89,6 +89,30 @@ __device__ __forceinline__ bool ls_accept(double dE, bool cand, double beta, uns
     return acc;
 }
 
+// Gibbs (heat-bath) counterpart of ls_accept, dwave-samplers >= 1.0 (SURVEY.md C.8): a candidate (dE < thr) is accepted
+// without a draw if dE <= -thr, else iff 2^64 > (double)rand * (1 + exp(dE*beta)).  No single-precision screen: every draw
+// takes the fp64 path, so the result is neal's arithmetic by construction.  Near ties: |2^64 - rand (1 + exp)| <= 2^-48 2^64.
+__device__ __forceinline__ bool gibbs_accept(double dE, bool cand, double beta, double thr, unsigned long long &s0,
+                                             unsigned long long &s1, LaneStats &st) {
+    bool acc = cand;
+    if (cand && !(dE <= -thr)) {
+        const unsigned long long rnd = rng_next(s0, s1);
+        st.draws++;
+        const double q = __ull2double_rn(rnd) * (1.0 + exp(dE * beta));
+        acc = QA_TWO64 > q;
+        if (fabs(QA_TWO64 - q) <= QA_TWO64 * 3.5527136788005009e-15) st.ties++;
+    }
+    return acc;
+}
+
+// the accept test of the lockstep and replay kernels for the call's acceptance rule
+template <Proposal PROP>
+__device__ __forceinline__ bool accept_test(double dE, bool cand, double beta, double thr, unsigned long long &s0,
+                                            unsigned long long &s1, LaneStats &st) {
+    if (PROP == PROP_GIBBS) return gibbs_accept(dE, cand, beta, thr, s0, s1, st);
+    return ls_accept(dE, cand, beta, s0, s1, st);
+}
+
 // lambda / kappa of every group into shared memory, kappa_words(GK) words of kappa per group ({kappa, lo, hi} for interval
 // groups).  Groups exist only on single-problem models, so the lockstep and replay kernels keep one copy per block.
 template <GroupKind GK>

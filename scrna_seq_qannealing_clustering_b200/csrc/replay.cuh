@@ -21,6 +21,10 @@
 // neighbours of accepted flips), so once the CTA-wide acceptance of a sweep drops below P.switch_permille the tile runs one
 // catch-up pass (pending u > v updates only) and finishes the schedule pushing, as neal does.  Both forms are exact, so
 // the hand-over point does not influence the result.
+// The derivation does not depend on the acceptance rule, so it holds for dwave-samplers' Gibbs rule (PROP_GIBBS) as well: each
+// variable is still visited once per sweep, so a neighbour still cannot flip twice between two visits; a field of +-0 is still
+// unobservable, because Gibbs compares dE with +-thr (never with the sign of zero) and exp(+-0) = 1; and the hand-over reads
+// acceptance counts only.
 //
 // Blocks.  The host packs consecutive variables greedily into blocks (at most RP_D = 16 variables inside ONE 16-variable
 // half-word, RP_MAXBW foreign half-words, RP_CAP entry slots) and builds one contiguous slab {RpHdr, RpEntry[]} per block.
@@ -366,8 +370,8 @@ __device__ __forceinline__ double rp_group_flip_cost(const RpCtx &c, int g, int 
 // for models whose adjacency lists are ascending (then adjacency order = pre entries u < v0, seq entries, later entries).
 // GROUPS: the group term (GK_INTERVAL: c.kap holds {kappa, lo, hi} per group).  KWAY: the slabs carry k-way sections
 // (rp_kway_batch); false compiles the replay sweep without the section test, so models without k-way blocks run exactly the
-// generic kernel.
-template <int MODE, GroupKind GROUPS, int SLOTS, bool KWAY = false>
+// generic kernel.  PROP: the acceptance rule of the decisions (modes 0 and 2).
+template <int MODE, GroupKind GROUPS, int SLOTS, bool KWAY = false, Proposal PROP = PROP_METROPOLIS>
 __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
     const int lane = threadIdx.x & 31;
     const double thr = 44.36142 / beta;
@@ -540,7 +544,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 bool acc = false;
                 if (__any_sync(FULL_MASK, cand)) {
                     if (cand) c.st.cand++;
-                    acc = ls_accept(dE, cand, beta, c.s0, c.s1, c.st);
+                    acc = accept_test<PROP>(dE, cand, beta, thr, c.s0, c.s1, c.st);
                 }
                 // F[v] := accepted (also when nothing was accepted: the flag of the previous visit must be cleared)
                 W = acc ? ((W | fb) ^ db) : (W & ~fb);
@@ -646,7 +650,7 @@ __device__ void rp_pass(RpCtx &c, double beta, bool has_next_pass) {
                 bool acc = false;
                 if (__any_sync(FULL_MASK, cand)) {
                     if (cand) c.st.cand++;
-                    acc = ls_accept(dE, cand, beta, c.s0, c.s1, c.st);
+                    acc = accept_test<PROP>(dE, cand, beta, thr, c.s0, c.s1, c.st);
                 }
                 if (__ballot_sync(FULL_MASK, acc) == 0u) continue;
                 const int sgn = up ? (int)0x80000000u : 0;   // f[j] += -2 s_v J
@@ -742,7 +746,7 @@ __host__ __device__ inline size_t rp_smem_bytes(int nw, int max_groups, unsigned
     return fixed + pad + (size_t)nw * (sf + RP_PS_BYTES);
 }
 
-template <GroupKind GROUPS, int SLOTS, bool KWAY>
+template <GroupKind GROUPS, Proposal PROP, int SLOTS, bool KWAY>
 __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_replay(AnnealParams P) {
     constexpr uint32_t RP_SF_BYTES = (uint32_t)rp_sf_bytes(SLOTS);
     extern __shared__ __align__(16) unsigned char rp_raw[];
@@ -915,11 +919,11 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
 #endif
                 RP_CLK(t_pass);
                 if (push) {
-                    rp_pass<2, GROUPS, SLOTS>(c, beta, more);
+                    rp_pass<2, GROUPS, SLOTS, false, PROP>(c, beta, more);
                     RP_PROF(7, clock64() - t_pass);
                 } else {
                     const unsigned acc0 = c.st.acc;
-                    rp_pass<0, GROUPS, SLOTS, KWAY>(c, beta, more);
+                    rp_pass<0, GROUPS, SLOTS, KWAY, PROP>(c, beta, more);
                     RP_PROF(6, clock64() - t_pass);
                     if (more) {  // CTA-uniform hand-over decision
                         unsigned wacc = c.st.acc - acc0;
@@ -977,4 +981,22 @@ __global__ void __launch_bounds__(RP_MAX_WARPS * 32, RP_MIN_CTAS) k_anneal_repla
     if (lane == 0)
         for (int k = 0; k < QA_NDEBUG; ++k) atomicAdd(P.stats + QA_NSTAT + 1 + k, (unsigned long long)c.prof[k]);
 #endif
+}
+
+// the kernel instance for the acceptance rule, group kind, slot count and k-way form of a model
+template <Proposal PROP, int SLOTS, bool KWAY>
+static const void *replay_instance(GroupKind gk) {
+    switch (gk) {
+    case GK_NONE: return (const void *)k_anneal_replay<GK_NONE, PROP, SLOTS, KWAY>;
+    case GK_EQ32: return (const void *)k_anneal_replay<GK_EQ32, PROP, SLOTS, KWAY>;
+    case GK_EQ64: return (const void *)k_anneal_replay<GK_EQ64, PROP, SLOTS, KWAY>;
+    default: return (const void *)k_anneal_replay<GK_INTERVAL, PROP, SLOTS, KWAY>;
+    }
+}
+
+template <Proposal PROP>
+static const void *replay_instance(const qa_model *M, GroupKind gk) {
+    const bool kway = M->rp_kway_blocks > 0;
+    if (M->rp_slots == 32) return kway ? replay_instance<PROP, 32, true>(gk) : replay_instance<PROP, 32, false>(gk);
+    return kway ? replay_instance<PROP, 64, true>(gk) : replay_instance<PROP, 64, false>(gk);
 }

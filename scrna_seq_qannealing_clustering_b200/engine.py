@@ -485,8 +485,10 @@ class IsingModel:
         return h, s, e, w
 
     def sample(self, states, beta_schedule, sweeps_per_beta, seeds, seed_mode=_lib.QA_SEED_PER_READ,
-               mode=_lib.QA_MODE_REFERENCE, energies=None, interrupt_function=None):
-        """Anneal ``states`` ([R][n] int8 +-1, in/out).  Returns (energies, QAStats, reads_completed)."""
+               mode=_lib.QA_MODE_REFERENCE, energies=None, interrupt_function=None, var_order=_lib.QA_ORDER_SEQUENTIAL,
+               proposal=_lib.QA_PROPOSAL_METROPOLIS):
+        """Anneal ``states`` ([R][n] int8 +-1, in/out).  Returns (energies, QAStats, reads_completed).  ``var_order`` /
+        ``proposal``: dwave-samplers' random variable order and Gibbs acceptance (QA_ORDER_*, QA_PROPOSAL_*)."""
         beta_schedule = _as(beta_schedule, np.float64, "beta_schedule")
         seeds = _as(seeds, np.uint64, "seeds")
         num_reads = int(states.shape[0])
@@ -497,9 +499,9 @@ class IsingModel:
         if interrupt_function is not None:
             cb = _lib.INTERRUPT_FN(lambda _u: 1 if interrupt_function() else 0)
         st = QAStats()
-        done = check(_lib.load().qa_sa_sample_model(
+        done = check(_lib.load().qa_sa_sample_model_ex(
             self.ctx._h, self._h, num_reads, ptr(states), ptr(energies), int(beta_schedule.shape[0]), ptr(beta_schedule),
-            int(sweeps_per_beta), ptr(seeds), int(seed_mode), int(mode),
+            int(sweeps_per_beta), ptr(seeds), int(seed_mode), int(mode), int(var_order), int(proposal),
             C.cast(cb, C.c_void_p) if cb is not None else None, None, C.byref(st)))
         return energies, st, done
 

@@ -9,6 +9,9 @@ dwave-neal's ``SimulatedAnnealingSampler.sample`` (SURVEY.md row a12):
            beta_schedule_type='geometric', seed=None, interrupt_function=None, beta_schedule=None,
            initial_states=None, initial_states_generator='random', **kwargs) -> SampleSet
 
+and dwave-samplers >= 1.0's two further options, with its names and defaults: ``randomize_order=False`` and
+``proposal_acceptance_criteria='Metropolis'`` (or ``'Gibbs'``).
+
 All annealing, energy evaluation and argmin run in the CUDA library; this file only parses arguments,
 lowers models to vectors and wraps results.  There is no CPU path: without the library or a GPU it raises.
 """
@@ -66,6 +69,8 @@ class B200SimulatedAnnealingSampler:
             "beta_range": [], "num_reads": [], "num_sweeps": [], "num_sweeps_per_beta": [],
             "beta_schedule_type": ["beta_schedule_options"], "seed": [], "interrupt_function": [], "beta_schedule": [],
             "initial_states": [], "initial_states_generator": [],
+            # dwave-samplers >= 1.0
+            "randomize_order": [], "proposal_acceptance_criteria": [],
             # extensions
             "mode": [], "seed_mode": [], "sorted": [], "aggregate": [], "return_samples": [], "num_best": [],
         }
@@ -96,13 +101,21 @@ class B200SimulatedAnnealingSampler:
     def sample(self, bqm, beta_range=None, num_reads=None, num_sweeps=None, num_sweeps_per_beta=1,
                beta_schedule_type="geometric", seed=None, interrupt_function=None, beta_schedule=None,
                initial_states=None, initial_states_generator="random", mode="reference", seed_mode="per_read",
-               sorted=False, aggregate=False, return_samples="all", num_best=16, **kwargs) -> SampleSet:
+               sorted=False, aggregate=False, return_samples="all", num_best=16, randomize_order=False,
+               proposal_acceptance_criteria="Metropolis", **kwargs) -> SampleSet:
         """Anneal a ``BinaryQuadraticModel`` (ours or dimod's), a ``LoweredModel`` or a ``DeviceModel``.
 
         Extensions to neal's signature: ``sorted`` / ``aggregate`` (QPU-like energy-sorted, duplicate-merged record);
         ``return_samples='best_k'`` with ``num_best=k``: the state matrix lives on the device from creation to ranking and only
         the k lowest-energy samples plus all R energies (``info['energies']``) come back -- with
-        ``initial_states_generator='counter'`` nothing of size R x n ever crosses PCIe (SURVEY.md hard part 7)."""
+        ``initial_states_generator='counter'`` nothing of size R x n ever crosses PCIe (SURVEY.md hard part 7).
+
+        dwave-samplers' options: ``randomize_order=True`` visits a random variable at each of the n attempts of a sweep
+        (runs on the warp-per-read kernel); ``proposal_acceptance_criteria='Gibbs'`` accepts a flip with probability
+        1 / (1 + exp(beta dE)) instead of Metropolis' min(1, exp(-beta dE)).  Both are bit-exact against the CPU oracle."""
+        if proposal_acceptance_criteria not in ("Metropolis", "Gibbs"):
+            raise ValueError("proposal_acceptance_criteria must be 'Metropolis' or 'Gibbs'")
+        self._options = (bool(randomize_order), proposal_acceptance_criteria)
         schedule.warn_unknown_kwargs(type(self).__name__, kwargs)
         t0 = time.perf_counter_ns()
         if return_samples not in ("all", "best_k"):
@@ -211,6 +224,7 @@ class B200SimulatedAnnealingSampler:
         if interrupt_function is not None and not callable(interrupt_function):
             raise TypeError("'interrupt_function' should be a callable")
         return_samples, num_best = getattr(self, "_return", ("all", 16))
+        randomize_order, criteria = getattr(self, "_options", (False, "Metropolis"))
         rank, world = _dist_rank_world()
         seed = schedule.resolve_seed(seed)
         if world > 1:
@@ -277,7 +291,10 @@ class B200SimulatedAnnealingSampler:
             energies, st, done = gm.sample(local_states, betas, spb, seeds,
                                            seed_mode=_lib.QA_SEED_STREAM if seed_mode == "stream" else _lib.QA_SEED_PER_READ,
                                            mode=_lib.QA_MODE_THROUGHPUT if mode == "throughput" else _lib.QA_MODE_REFERENCE,
-                                           interrupt_function=interrupt_function)
+                                           interrupt_function=interrupt_function,
+                                           var_order=_lib.QA_ORDER_RANDOM if randomize_order else _lib.QA_ORDER_SEQUENTIAL,
+                                           proposal=_lib.QA_PROPOSAL_GIBBS if criteria == "Gibbs" else _lib.QA_PROPOSAL_METROPOLIS)
+            kernel = ctx.last_kernel
             t2 = time.perf_counter_ns()
             self.last_stats = st.as_dict()
             energies = energies[:done]
@@ -305,6 +322,7 @@ class B200SimulatedAnnealingSampler:
         samples = local_states if vartype is SPIN else ((local_states + 1) // 2).astype(np.int8)
         info["timing"] = {"preprocessing_ns": t1 - t0, "sampling_ns": t2 - t1, "postprocessing_ns": 0}
         info["b200"] = {"mode": mode, "seed_mode": seed_mode, "world_size": world, "return_samples": return_samples,
+                        "randomize_order": randomize_order, "proposal_acceptance_criteria": criteria, "kernel": kernel,
                         **{k: self.last_stats[k] for k in
                            ("attempts", "accepted", "draws", "candidates", "nbr_updates", "near_ties", "ms_anneal")}}
         ss = SampleSet.from_samples((samples, labels), energy=energies, vartype=vartype, info=info, **extra)
